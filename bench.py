@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (our arm)
     python bench.py --impl reference --gpus N --steps K --warmup W   (reference CPU arm)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs bench_outputs  (also the last step's outputs)
 
 Headline metric (BASELINE.json configs[1]): RoIAlign crop_and_resize fwd+bwd ROIs/s on
 256-channel FPN P2-P5, batch 8 per GPU, 1000 ROIs/img, 7x7 and 14x14, fp32.  A "step" is one
@@ -29,6 +30,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the tree may be read-only: the benchmark writes nothing into it
 if "reference" in sys.argv:
     # the reference arm uses every host core; torchrun exports OMP_NUM_THREADS=1 to its workers, and the OpenMP runtime
     # reads the variable when it is first loaded (with torch, below), so it has to be overridden here
@@ -82,6 +84,29 @@ def make_workload(seed_shift=0):
     level = synth.fpn_level(boxes) - 2
     box_ind = np.repeat(np.arange(IMAGES_PER_GPU, dtype=np.int32), ROIS_PER_IMAGE)
     return boxes, box_ind, level.astype(np.int32)
+
+
+DUMP_SEED = 20241020
+DUMP_CROP_SAMPLES = 1 << 21       # per pool: 8 MB of the 100 MB (7x7) / 401 MB (14x14) of crops
+DUMP_GRAD_SAMPLES = 1 << 20       # per pool and level: 4 MB; 48 MB in all
+
+
+def dump_outputs(out_dir, outs):
+    """Writes what one step returned to its caller -- per pool the crops [N, C, p, p] and the four gradient maps
+    [B, C, H_l, W_l] -- as float32 .npy files.  Each array is a fixed, seeded sample of its elements (flat indices in
+    NCHW order, ascending), so two builds run with the same arguments can be compared element for element."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = []
+    for p in POOLS:
+        crops, gmaps = outs[p]
+        arrays.append(("crops_%dx%d" % (p, p), crops, DUMP_CROP_SAMPLES))
+        arrays += [("grad_p%d_%dx%d" % (l + 2, p, p), gm, DUMP_GRAD_SAMPLES) for l, gm in enumerate(gmaps)]
+    for k, (name, t, n) in enumerate(arrays):
+        rng = np.random.default_rng([DUMP_SEED, k])
+        idx = np.sort(rng.choice(t.numel(), min(n, t.numel()), replace=False))
+        sample = torch.take(t, torch.from_numpy(idx).to(t.device))    # logical (NCHW) order whatever the strides
+        np.save(os.path.join(out_dir, name + ".npy"), sample.cpu().numpy().astype(np.float32))
 
 
 # --------------------------------------------------------------------------------------
@@ -221,10 +246,12 @@ def run_ours(args):
     def step():
         # what the autograd operator does (pyramid._PyramidCrop): the backward's ROI lists are planned on a side stream
         # beside the forward kernel (they depend on the boxes only); the plan launches are inside the timed region
+        outs = {}
         for p in POOLS:
             plan = ops.pyramid_crop_backward_plan(boxes, box_ind, level, sizes, CHANNELS, p, p) if plan_ahead else None
-            ops.pyramid_crop_forward(maps, boxes, box_ind, level, p, p, 0.0)
-            ops.pyramid_crop_backward(grads[p], boxes, box_ind, level, sizes, plan=plan)
+            crops = ops.pyramid_crop_forward(maps, boxes, box_ind, level, p, p, 0.0)
+            outs[p] = (crops, ops.pyramid_crop_backward(grads[p], boxes, box_ind, level, sizes, plan=plan))
+        return outs
 
     def barrier():
         if world > 1:
@@ -241,7 +268,10 @@ def run_ours(args):
         t_start = time.perf_counter()
         e0.record()
         for _ in range(args.steps):
-            step()
+            # the previous step's outputs go back to the allocator first: every timed step then allocates exactly like the
+            # warmup steps, from blocks the allocator already holds (no cudaMalloc inside the timed region)
+            last = None
+            last = step()
         e1.record()
         barrier()
         t_end = time.perf_counter()
@@ -253,6 +283,9 @@ def run_ours(args):
             step()
         torch.cuda.synchronize()
     clocks_summary = clocks.summary(t_start, t_end)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     launches = launches_timed
     ms_total = sdist.max_over_ranks(e0.elapsed_time(e1))
     ms_per_step = ms_total / args.steps
@@ -1235,8 +1268,6 @@ def _cpu_pass(oracle, use_ref, maps_np, boxes, level, grads):
 def cpu_reference_sample(boxes_np, ind_np, level_np, maps=None, steps=1, warmup=1):
     from oracle import oracle
     use_ref = oracle.ref_available()
-    if not use_ref:
-        oracle.build()
     cores = os.cpu_count() or 1
     # torchrun exports OMP_NUM_THREADS=1 to its workers; the reference arm is meant to use every host core it can
     os.environ["OMP_NUM_THREADS"] = str(cores)
@@ -1294,7 +1325,13 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of what the last timed step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -142,18 +142,6 @@ def main():
     print("input scale", scale, "distinct fg scores", np.unique(fg).size, "ties among the top 6001:", 6001 - np.unique(top).size,
           "| score[5999], score[6000]:", top[5999], top[6000], "(a clean cut makes the top-6000 SET unique)")
 
-    import hashlib
-    blobs = {}
-
-    def intern(a):
-        """big arrays that occur at several boundaries (the same FPN map feeds several calls) are stored once"""
-        a = np.ascontiguousarray(a)
-        if a.nbytes < 65536:
-            return a
-        h = "blob_" + hashlib.sha1(a.tobytes()).hexdigest()[:16]
-        blobs.setdefault(h, a)
-        return np.array(h)
-
     save = {"use_nms": bool(cfg.USE_NMS), "ch256": CH256, "ch183": CH183,
             "final_detections": detections.detach().numpy(), "final_mask_shape": np.asarray(mrcnn_mask.shape)}
     for name, calls in rec.items():
@@ -181,12 +169,93 @@ def main():
     for i, (r, p, d, w, det, k, un) in enumerate(rec["refine"]):
         save.update({"refine%d_rois" % i: r, "refine%d_probs" % i: p, "refine%d_deltas" % i: d, "refine%d_window" % i: w,
                      "refine%d_det" % i: det, "refine%d_keep" % i: k, "refine%d_use_nms" % i: un})
-    save = {k: intern(v) if isinstance(v, np.ndarray) else v for k, v in save.items()}
-    save.update(blobs)
-    path = os.path.join(HERE, "predict_trace.npz")
-    np.savez_compressed(path, **save)
+    path = write_fixture(save, os.path.join(HERE, "predict_trace.npz"))
     print("recorded:", {k: len(v) for k, v in rec.items()}, "detections", tuple(detections.shape), "mask", tuple(mrcnn_mask.shape),
-          "->", path, "%.1f MB" % (os.path.getsize(path) / 1e6))
+          "->", path, "%.2f MB" % (os.path.getsize(path) / 1e6))
+
+
+# rows kept per recorded crop / pyramid call, by crop size; the same seed for calls of the same length, so that calls that
+# computed the same crops (crop3 / pyramid1, crop2 / pyrimg0) keep the same rows and still share one stored array
+SAMPLE_ROWS = {7: 48, 16: 16}
+TOP_ANCHORS = 6001                # the top-6000 SET plus the first anchor below the cut
+
+
+def _rows(n, size):
+    return np.sort(np.random.default_rng(n).choice(n, min(SAMPLE_ROWS[size], n), replace=False))
+
+
+def _footprint(boxes, H, W, mask):
+    """marks every pixel crop_and_resize.c can read for these boxes: rows floor(min(y1,y2)*(H-1)) .. ceil(max(y1,y2)*(H-1))
+    and the same for columns, one pixel of margin for the fp32 rounding of the sample positions"""
+    for y1, x1, y2, x2 in np.asarray(boxes, np.float64).reshape(-1, 4):
+        r0, r1 = int(np.floor(min(y1, y2) * (H - 1))) - 1, int(np.ceil(max(y1, y2) * (H - 1))) + 2
+        c0, c1 = int(np.floor(min(x1, x2) * (W - 1))) - 1, int(np.ceil(max(x1, x2) * (W - 1))) + 2
+        mask[max(r0, 0):max(r1, 0), max(c0, 0):max(c1, 0)] = True
+
+
+def shrink(save):
+    """Keeps the fixture small (tests/golden holds no file over 1 MB) without changing what a replay checks:
+      * proposal_layer inputs: only the TOP_ANCHORS best-scoring anchors are stored (index, foreground score, deltas);
+        test_predict_trace.Trace gives every other anchor a seeded score below the cut and zero deltas.  The reference's
+        result depends on the top 6000 only (Functions.py:144-153), so the replayed call computes the recorded one;
+      * crop / pyramid calls: a seeded sample of rows (boxes, box indices, outputs) -- each crop depends on its own box
+        only -- and the FPN maps zeroed outside the pixels the kept boxes read.  A map that no kept box reads (boxes given
+        in pixels instead of normalised, all outside the map: the recorded crops are the extrapolation value) is kept as
+        recorded, so that a replay still tells extrapolation from reading the nearest edge pixels."""
+    from oracle import oracle
+    out = dict(save)
+    for i in range(int(save["n_proposal"])):
+        p, d = save["proposal%d_probs" % i][0], save["proposal%d_deltas" % i][0]
+        top = np.sort(np.argsort(-p[:, 1].astype(np.float64), kind="stable")[:TOP_ANCHORS]).astype(np.int32)
+        del out["proposal%d_probs" % i], out["proposal%d_deltas" % i]
+        out.update({"proposal%d_n_anchors" % i: p.shape[0], "proposal%d_top" % i: top,
+                    "proposal%d_top_fg" % i: p[top, 1], "proposal%d_top_deltas" % i: d[top]})
+    masks = {}                                                  # map contents -> pixels read from that map
+
+    def use(key, boxes):
+        m = save[key]
+        mask = masks.setdefault(m.tobytes(), np.zeros(m.shape[2:], bool))
+        _footprint(boxes, m.shape[2], m.shape[3], mask)
+        return key
+    used = []
+    for i in range(int(save["n_crop"])):
+        r = _rows(save["crop%d_boxes" % i].shape[0], int(save["crop%d_size" % i][0]))
+        for k in ("boxes", "ind", "out"):
+            out["crop%d_%s" % (i, k)] = save["crop%d_%s" % (i, k)][r]
+        used.append(use("crop%d_image" % i, out["crop%d_boxes" % i]))
+    for i in range(int(save["n_pyramid"])):
+        r = _rows(save["pyramid%d_rois" % i].shape[1], int(save["pyramid%d_pool" % i]))
+        out["pyramid%d_rois" % i], out["pyramid%d_out" % i] = save["pyramid%d_rois" % i][:, r], save["pyramid%d_out" % i][r]
+        lv = oracle.roi_levels(out["pyramid%d_rois" % i][0], tuple(int(v) for v in save["pyramid%d_shape" % i][:2]))
+        for l in range(int(save["pyramid%d_nmaps" % i])):
+            used.append(use("pyramid%d_map%d" % (i, l), out["pyramid%d_rois" % i][0][lv == l + 2]))
+    for i in range(int(save["n_pyramid_image"])):
+        r = _rows(save["pyrimg%d_rois" % i].shape[1], int(save["pyrimg%d_pool" % i]))
+        out["pyrimg%d_rois" % i], out["pyrimg%d_out" % i] = save["pyrimg%d_rois" % i][:, r], save["pyrimg%d_out" % i][r]
+        used.append(use("pyrimg%d_map" % i, out["pyrimg%d_rois" % i][0]))
+    for k in used:                                              # masks are complete only now: maps are shared by calls
+        mask = masks[save[k].tobytes()]
+        if mask.any():
+            out[k] = np.where(mask[None, None], save[k], np.float32(0)).astype(np.float32)
+    return out
+
+
+def write_fixture(save, path):
+    """shrink(), then store every large array once (the same FPN map feeds several calls) under a content-named key"""
+    import hashlib
+    blobs = {}
+
+    def intern(a):
+        a = np.ascontiguousarray(a)
+        if a.nbytes < 4096:
+            return a
+        h = "blob_" + hashlib.sha1(repr((a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()[:16]
+        blobs.setdefault(h, a)
+        return np.array(h)
+    save = {k: intern(v) if isinstance(v, np.ndarray) else v for k, v in shrink(save).items()}
+    save.update(blobs)
+    np.savez_compressed(path, **save)
+    return path
 
 
 if __name__ == "__main__":

@@ -4,7 +4,9 @@ The fixture (tests/golden/make_golden_predict.py) was recorded from the referenc
 MaskRCNN.predict(mode='inference') (model.py:516-706, built as amodal_test.py:27-38 builds it; CPU, random init, one
 synthetic 1024x1024 image): every call across the boundaries of the hot path with its arguments and its result --
 nms, CropAndResizeFunction, proposal_layer, pyramid_roi_align, pyramid_roi_align_image, refine_detections.  Here the
-same arguments go through (a) the oracle (CPU) and (b) the drop-in operators on the GPU.
+same arguments go through (a) the oracle (CPU) and (b) the drop-in operators on the GPU.  The crop and pyramid calls
+are stored as a seeded sample of their rows, the RPN outputs as the anchors that decide proposal_layer's result
+(make_golden_predict.shrink).
 """
 import os
 import sys
@@ -27,10 +29,26 @@ class Trace:
         self.g = np.load(os.path.join(HERE, "golden", "predict_trace.npz"))
 
     def __getitem__(self, k):
+        call, _, what = k.partition("_")
+        if call.startswith("proposal") and what in ("probs", "deltas"):
+            return self.rpn_outputs(call)[what == "deltas"]
         a = self.g[k]
         if a.dtype.kind == "U" and a.shape == () and str(a).startswith("blob_"):
             return self.g[str(a)]
         return a
+
+    def rpn_outputs(self, call):
+        """The recorded RPN outputs [1, A, 2] / [1, A, 4] of a proposal_layer call, rebuilt from the stored top anchors
+        (make_golden_predict.shrink): every other anchor scores below all of them (seeded) and has zero deltas.  The
+        background column is 1 - foreground: proposal_layer reads the foreground column only."""
+        top, fg = self[call + "_top"], self[call + "_top_fg"]
+        n = int(self[call + "_n_anchors"])
+        below = np.nextafter(fg.min(), np.float32(0))
+        scores = (np.random.default_rng(0).random(n) * float(below)).astype(np.float32)
+        scores[top] = fg
+        deltas = np.zeros((n, 4), np.float32)
+        deltas[top] = self[call + "_top_deltas"]
+        return np.stack([np.float32(1) - scores, scores], 1)[None], deltas[None]
 
     def n(self, what):
         return int(self.g["n_" + what])
