@@ -1433,7 +1433,10 @@ extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, 
     }
     dim3 grid(N, cdiv(C, c_chunk));
     SLN_REQUIRE(grid.y <= 65535, SLN_ERR_ARG, "too many channel chunks");
+    // tap tables: 64 KB at 4096 x 4096, so crops with ph + pw > 6144 need more than the 48 KB granted without opting in
     const size_t smem = sizeof(Tap) * (size_t)(ph + pw);
+    if (smem > 48 * 1024)
+        SLN_CUDA_OK(cudaFuncSetAttribute(crop_fwd_nchw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     crop_fwd_nchw_kernel<<<grid, 256, smem, st>>>(image, B, C, H, W, boxes, box_ind, ph, pw, ext, c_chunk, crops);
     SLN_LAUNCH_OK("crop_fwd_nchw_kernel");
     return SLN_OK;

@@ -44,6 +44,23 @@ def _workspace(nbytes, device):
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
 
 
+def _check_rois(N, box_ind, level=None):
+    """The kernels read box_ind[i] (and level[i]) for every one of the N boxes: a shorter array is read out of bounds."""
+    if box_ind.shape[0] != N:
+        raise _lib.SlnError(f"box_ind has {box_ind.shape[0]} entries for {N} boxes")
+    if level is not None and level.shape[0] != N:
+        raise _lib.SlnError(f"level has {level.shape[0]} entries for {N} boxes")
+
+
+def _check_map_sizes(map_sizes, channels):
+    """map_sizes of the pyramid backward: (B, C, H, W) per level, one B for all, C == channels.  Returns B."""
+    B = int(map_sizes[0][0])
+    for sz in map_sizes:
+        if int(sz[0]) != B or int(sz[1]) != int(channels):
+            raise _lib.SlnError(f"map size {tuple(sz)} disagrees with batch {B} / channels {int(channels)}")
+    return B
+
+
 _AUX_STREAMS = {}
 
 
@@ -60,11 +77,13 @@ def _aux_stream(device):
 # layout converters
 # ---------------------------------------------------------------------------
 def to_channels_last(x):
-    """NCHW-contiguous f32 -> same logical tensor in channels_last memory (our transpose kernel)."""
+    """Any 4-D tensor -> the same logical tensor as f32 in channels_last memory (our transpose kernel)."""
     _require_cuda(x, "x")
+    if x.dtype != torch.float32:
+        x = x.detach().float()                # keeps the memory format: a channels_last input stays channels_last
     if is_channels_last(x):
         return x
-    x = _f32c(x)
+    x = x.detach().contiguous()
     B, Cc, H, W = x.shape
     out = torch.empty((B, Cc, H, W), dtype=torch.float32, device=x.device, memory_format=torch.channels_last)
     if out.numel():
@@ -75,8 +94,10 @@ def to_channels_last(x):
 
 
 def to_contiguous_nchw(x):
-    """channels_last f32 -> NCHW-contiguous (our transpose kernel)."""
+    """Any 4-D tensor -> the same logical tensor as f32, NCHW-contiguous (channels_last input: our transpose kernel)."""
     _require_cuda(x, "x")
+    if x.dtype != torch.float32:
+        x = x.detach().float()
     if x.is_contiguous():
         return x
     if not is_channels_last(x):
@@ -188,6 +209,7 @@ def crop_and_resize_backward(grads, boxes, box_ind, image_size, channels_last_ou
     N, Cg, ph, pw = grads.shape
     if Cg != Cc or boxes.shape[0] != N:
         raise _lib.SlnError("grads / boxes / image_size disagree")
+    _check_rois(N, box_ind)
     g, g_cl = _prep_grads(grads)
     if channels_last_out is None:
         channels_last_out = g_cl
@@ -232,8 +254,9 @@ def pyramid_crop_backward_plan(boxes, box_ind, level, map_sizes, channels, crop_
     box_ind = _i32c(box_ind).view(-1)
     level = _i32c(level).view(-1)
     N = boxes.shape[0]
+    _check_rois(N, box_ind, level)
     nl = len(map_sizes)
-    B = int(map_sizes[0][0])
+    B = _check_map_sizes(map_sizes, channels)
     dev = boxes.device
     cur = torch.cuda.current_stream(dev)
     side = stream if stream is not None else _aux_stream(dev)
@@ -269,8 +292,11 @@ def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last
     box_ind = _i32c(box_ind).view(-1)
     level = _i32c(level).view(-1)
     N, Cc, ph, pw = grads.shape
+    if boxes.shape[0] != N:
+        raise _lib.SlnError(f"grads hold {N} crops for {boxes.shape[0]} boxes")
+    _check_rois(N, box_ind, level)
     nl = len(map_sizes)
-    B = int(map_sizes[0][0])
+    B = _check_map_sizes(map_sizes, Cc)
     g, _ = _prep_grads(grads)
     outs = [torch.empty(tuple(int(v) for v in sz), dtype=torch.float32, device=grads.device,
                         memory_format=torch.channels_last) for sz in map_sizes]
@@ -296,24 +322,28 @@ def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last
 def pyramid_crop_forward(feature_maps, boxes, box_ind, level, crop_height, crop_width, extrapolation_value=0.0):
     """One launch for all FPN levels: feature_maps = list of channels_last [B,C,H_l,W_l] tensors,
     level[i] in [0, len(feature_maps)) names the source map of ROI i.  Output channels_last
-    [N,C,ph,pw] in the original ROI order."""
-    maps = []
+    [N,C,ph,pw] in the original ROI order.  Maps of another dtype are cropped from their f32 values."""
     for m in feature_maps:
         _require_cuda(m, "feature map")
-        if is_channels_last(m) and m.dtype == torch.float32:
-            maps.append(m.detach())
-        elif m.dtype == torch.float32 and m.dim() == 4:
-            maps.append(_nhwc_cached(m))                 # NCHW map: transposed once, remembered while the tensor lives
-        else:
-            maps.append(to_channels_last(m))
+        if m.dim() != 4:
+            raise _lib.SlnError("feature maps must be [B,C,H_l,W_l]")
     boxes = _f32c(boxes).view(-1, 4)
     box_ind = _i32c(box_ind).view(-1)
     level = _i32c(level).view(-1)
     N = boxes.shape[0]
-    B, Cc = maps[0].shape[0], maps[0].shape[1]
-    for m in maps:
+    _check_rois(N, box_ind, level)
+    B, Cc = feature_maps[0].shape[0], feature_maps[0].shape[1]
+    for m in feature_maps:
         if m.shape[0] != B or m.shape[1] != Cc:
             raise _lib.SlnError("feature maps disagree on batch / channels")
+    maps = []
+    for m in feature_maps:
+        if is_channels_last(m) and m.dtype == torch.float32:
+            maps.append(m.detach())
+        elif m.dtype == torch.float32:
+            maps.append(_nhwc_cached(m))                 # NCHW map: transposed once, remembered while the tensor lives
+        else:
+            maps.append(to_channels_last(m))
     nl = len(maps)
     out = torch.empty((N, Cc, crop_height, crop_width), dtype=torch.float32, device=boxes.device,
                       memory_format=torch.channels_last)
@@ -464,6 +494,8 @@ def mask_targets_device(gt_masks, assignment, boxes, mh, mw):
     boxes = _f32c(boxes).view(-1, 4)
     assignment = _i32c(assignment).view(-1)
     P = boxes.shape[0]
+    if assignment.shape[0] != P:
+        raise _lib.SlnError(f"assignment has {assignment.shape[0]} entries for {P} boxes")
     out = torch.empty((P, L, int(mh), int(mw)), dtype=torch.float32, device=gt_masks.device)
     if out.numel():
         with torch.cuda.device(gt_masks.device):
