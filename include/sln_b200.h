@@ -52,6 +52,10 @@ extern "C" {
 #define SLN_LAYOUT_NCHW 0        /* [B,C,H,W] contiguous                              */
 #define SLN_LAYOUT_NHWC 1        /* [B,H,W,C] contiguous (torch channels_last)        */
 
+#define SLN_DTYPE_F32  0         /* element type of the *_ex crop entry points: float  */
+#define SLN_DTYPE_BF16 1         /* bfloat16                                          */
+#define SLN_DTYPE_F16  2         /* IEEE half                                         */
+
 /* ---- library ---------------------------------------------------------- */
 SLN_API int         sln_version(void);                 /* 10000*major + 100*minor + patch   */
 SLN_API const char *sln_last_error_string(void);       /* thread-local, never NULL          */
@@ -121,9 +125,38 @@ SLN_API int sln_pyramid_crop_bwd(const float *grads, const float *boxes, const i
  * boxes f32 [N,4] normalised (y1,x1,y2,x2), 16-byte aligned; level_out i32 [N] in 0..3 (P2..P5).               */
 SLN_API int sln_roi_levels(const float *boxes, int N, int image_h, int image_w, int *level_out, void *stream);
 
-/* Layout converters (f32).  src and dst must not alias.                            */
+/* ---- RoIAlign on 2-byte maps (bf16 / fp16, e.g. under mixed precision) ------- *
+ * The four crop entry points above with an element type: `dtype` (SLN_DTYPE_*) names the type of the maps, crops,
+ * grads and grad maps of the call (one type for all of them); boxes stay f32 and indices i32.  SLN_DTYPE_F32 is
+ * exactly the call without the suffix.  For a 2-byte type the kernels widen every element to f32 (exact), run the
+ * f32 operation sequence with f32 accumulators, and round each result once to nearest even: a crop or gradient map
+ * is bit-identical to the f32 call on the widened inputs, rounded to the type (NaN payloads aside).  The
+ * extrapolation value is rounded the same way.
+ *   forward : NHWC only (any C; 16-byte vectors when C % 8 == 0 and the pointers allow).  SLN_ERR_LAYOUT for NCHW:
+ *             convert with sln_nchw_to_nhwc_b16, or widen and use the f32 NCHW kernel.
+ *   backward: the bulk-async kernel only -- C % 8 == 0, ph and pw <= 32, grads and grad maps 16-byte aligned;
+ *             SLN_ERR_LAYOUT otherwise (widen, run the f32 call and round: same bits).  SLN_BWD_PLAN_ONLY /
+ *             SLN_BWD_PLANNED work as for f32, and a plan does not depend on the dtype: a PLAN_ONLY call of any
+ *             dtype serves PLANNED calls of every dtype with the same boxes and sizes.                            */
+SLN_API int sln_crop_and_resize_fwd_ex(int dtype, const void *image, int B, int C, int H, int W, int layout,
+                               const float *boxes, const int *box_ind, int N, int ph, int pw,
+                               float extrapolation_value, void *crops, void *stream);
+SLN_API int sln_crop_and_resize_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind, int N,
+                               int C, int ph, int pw, void *grad_image, int B, int H, int W, int layout, int flags,
+                               void *workspace, size_t workspace_bytes, void *stream);
+SLN_API int sln_pyramid_crop_fwd_ex(int dtype, const void *const *maps_host, const int *H_host, const int *W_host,
+                            int n_levels, int B, int C, const float *boxes, const int *box_ind, const int *level,
+                            int N, int ph, int pw, float extrapolation_value, void *crops, void *stream);
+SLN_API int sln_pyramid_crop_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind,
+                            const int *level, int N, int C, int ph, int pw, void *const *grad_maps_host,
+                            const int *H_host, const int *W_host, int n_levels, int B, int flags,
+                            void *workspace, size_t workspace_bytes, void *stream);
+
+/* Layout converters (f32; the _b16 forms move any 2-byte type).  src and dst must not alias.                    */
 SLN_API int sln_nchw_to_nhwc(const float *src, float *dst, int B, int C, int H, int W, void *stream);
 SLN_API int sln_nhwc_to_nchw(const float *src, float *dst, int B, int C, int H, int W, void *stream);
+SLN_API int sln_nchw_to_nhwc_b16(const uint16_t *src, uint16_t *dst, int B, int C, int H, int W, void *stream);
+SLN_API int sln_nhwc_to_nchw_b16(const uint16_t *src, uint16_t *dst, int B, int C, int H, int W, void *stream);
 
 /* ---- NMS --------------------------------------------------------------- *
  * Replaces cpu_nms (nms/src/nms.c:4-69) + the pth_nms front end (nms/pth_nms.py:5-24)

@@ -17,6 +17,9 @@ LAYOUT_NHWC = 1
 BWD_EXACT = 1
 BWD_PLAN_ONLY = 2        # sln_pyramid_crop_bwd: build the ROI lists only
 BWD_PLANNED = 4          # ... the workspace already holds them
+DTYPE_F32 = 0            # element type of the *_ex crop entry points
+DTYPE_BF16 = 1
+DTYPE_F16 = 2
 
 _vp, _i, _f, _sz = C.c_void_p, C.c_int, C.c_float, C.c_size_t
 
@@ -33,9 +36,17 @@ PROTOTYPES = {
     "sln_pyramid_crop_bwd_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "sln_pyramid_crop_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, C.POINTER(_vp), C.POINTER(_i), C.POINTER(_i), _i, _i,
                                   _i, _vp, _sz, _vp]),
+    "sln_crop_and_resize_fwd_ex": (_i, [_i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _f, _vp, _vp]),
+    "sln_crop_and_resize_bwd_ex": (_i, [_i, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _vp, _sz, _vp]),
+    "sln_pyramid_crop_fwd_ex": (_i, [_i, C.POINTER(_vp), C.POINTER(_i), C.POINTER(_i), _i, _i, _i, _vp, _vp, _vp, _i,
+                                     _i, _i, _f, _vp, _vp]),
+    "sln_pyramid_crop_bwd_ex": (_i, [_i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, C.POINTER(_vp), C.POINTER(_i), C.POINTER(_i),
+                                     _i, _i, _i, _vp, _sz, _vp]),
     "sln_roi_levels": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "sln_nchw_to_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     "sln_nhwc_to_nchw": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
+    "sln_nchw_to_nhwc_b16": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
+    "sln_nhwc_to_nchw_b16": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     "sln_nms_workspace_bytes": (_sz, [_i]),
     "sln_nms": (_i, [_vp, _vp, _i, _f, _i, _vp, _vp, _vp, _sz, _vp]),
     "sln_nms_ex": (_i, [_vp, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),

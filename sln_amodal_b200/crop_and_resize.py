@@ -19,12 +19,23 @@ from torch import nn
 from . import ops
 
 
+def keeps_dtype(*maps):
+    """Inside an enabled CUDA autocast region, bf16 / fp16 maps (all of one dtype) are cropped in their own dtype, like
+    torchvision's roi_align, and their gradient is written in it; the values are today's f32 results rounded once, which
+    is what autocast's cast hands a low-precision consumer anyway.  Outside autocast, crops are f32."""
+    dt = maps[0].dtype
+    return torch.is_autocast_enabled("cuda") and dt in ops.LOWP_DTYPES and all(m.dtype == dt for m in maps)
+
+
 class _CropAndResize(torch.autograd.Function):
     @staticmethod
     def forward(ctx, image, boxes, box_ind, crop_height, crop_width, extrapolation_value):
-        crops = ops.crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extrapolation_value)
+        lowp = keeps_dtype(image)
+        crops = ops.crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extrapolation_value,
+                                            keep_dtype=lowp)
         ctx.im_size = tuple(image.shape)                       # crop_and_resize.py:30-31
         ctx.im_channels_last = ops.is_channels_last(image)
+        ctx.grad_dtype = image.dtype if lowp else torch.float32
         ctx.save_for_backward(boxes, box_ind)
         return crops
 
@@ -32,14 +43,15 @@ class _CropAndResize(torch.autograd.Function):
     def backward(ctx, grad_outputs):
         boxes, box_ind = ctx.saved_tensors
         grad_image = ops.crop_and_resize_backward(grad_outputs, boxes, box_ind, ctx.im_size,
-                                                  channels_last_out=ctx.im_channels_last)
+                                                  channels_last_out=ctx.im_channels_last, out_dtype=ctx.grad_dtype)
         return grad_image, None, None, None, None, None       # crop_and_resize.py:50
 
 
 class CropAndResizeFunction(object):
     """CropAndResizeFunction(ch, cw, ext)(image, boxes, box_ind) -> crops [N,C,ch,cw].
 
-    image   f32 [B,C,H,W] (CUDA); NCHW or channels_last memory, the result follows it
+    image   f32 [B,C,H,W] (CUDA); NCHW or channels_last memory, the result follows it.  bf16 / fp16 images
+            give crops of their dtype inside torch.autocast (see keeps_dtype), f32 crops outside it
     boxes   f32 [N,4] (y1,x1,y2,x2) normalised to [0,1] over (H-1, W-1)
     box_ind i32 [N] image index of each box"""
 

@@ -1,6 +1,8 @@
 // common.cuh -- shared helpers for libsln_b200 (sm_100a only).
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -199,5 +201,123 @@ __device__ __forceinline__ float4 lerp2v(float4 tl, float4 tr, float4 bl, float4
     unpk2(r1, r.z, r.w);
     return r;
 }
+
+// ---------------------------------------------------------------------------
+// 2-byte elements (bf16 / fp16 maps under autocast).  Widening to fp32 is exact, so a kernel that widens its inputs,
+// runs the fp32 operation sequence and rounds its result once (to nearest even) gives the bits of the fp32 kernel run
+// on the widened tensor, rounded.  Elements travel as raw 16-bit words.
+// ---------------------------------------------------------------------------
+template <typename T> struct Elem16;
+template <> struct Elem16<__nv_bfloat16> {
+    static __device__ __forceinline__ float widen(unsigned short h) { return __uint_as_float((unsigned)h << 16); }
+    static __device__ __forceinline__ void widen2(unsigned w, float &lo, float &hi)
+    {
+        lo = __uint_as_float(w << 16);
+        hi = __uint_as_float(w & 0xffff0000u);
+    }
+    static __device__ __forceinline__ unsigned short narrow(float f) { return __bfloat16_as_ushort(__float2bfloat16_rn(f)); }
+    static __device__ __forceinline__ unsigned narrow2(float lo, float hi)
+    {
+        const __nv_bfloat162 r = __floats2bfloat162_rn(lo, hi);
+        return *reinterpret_cast<const unsigned *>(&r);
+    }
+};
+template <> struct Elem16<__half> {
+    static __device__ __forceinline__ float widen(unsigned short h) { return __half2float(__ushort_as_half(h)); }
+    static __device__ __forceinline__ void widen2(unsigned w, float &lo, float &hi)
+    {
+        const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&w));
+        lo = f.x;
+        hi = f.y;
+    }
+    static __device__ __forceinline__ unsigned short narrow(float f) { return __half_as_ushort(__float2half_rn(f)); }
+    static __device__ __forceinline__ unsigned narrow2(float lo, float hi)
+    {
+        const __half2 r = __floats2half2_rn(lo, hi);
+        return *reinterpret_cast<const unsigned *>(&r);
+    }
+};
+
+// 16 bytes of a 2-byte type (8 elements) <-> two float4 (elements 0..3, 4..7)
+template <typename T>
+__device__ __forceinline__ void widen8(uint4 v, float4 &a, float4 &b)
+{
+    Elem16<T>::widen2(v.x, a.x, a.y);
+    Elem16<T>::widen2(v.y, a.z, a.w);
+    Elem16<T>::widen2(v.z, b.x, b.y);
+    Elem16<T>::widen2(v.w, b.z, b.w);
+}
+template <typename T>
+__device__ __forceinline__ uint4 narrow8(float4 a, float4 b)
+{
+    return make_uint4(Elem16<T>::narrow2(a.x, a.y), Elem16<T>::narrow2(a.z, a.w), Elem16<T>::narrow2(b.x, b.y),
+                      Elem16<T>::narrow2(b.z, b.w));
+}
+
+// Vector I/O of the forward gather: VEC elements per load / store.  fp32: float / float4 as before.  2-byte types:
+// 8 / 4 / 2 / 1 elements (16 / 8 / 4 / 2 bytes), widened on load, the lerp run on packed fp32 pairs (same bits as
+// lerp2() per element), rounded once on store.
+template <typename T, int VEC> struct CropIO {
+    using V = typename VecT<VEC>::type;
+    static __device__ __forceinline__ V ld(const V *p) { return ldg_vec(p); }
+    static __device__ __forceinline__ V splat(float v) { return make_splat(v, (V *)nullptr); }
+    static __device__ __forceinline__ V lerp(V tl, V tr, V bl, V br, float xl, float yl) { return lerp2v(tl, tr, bl, br, xl, yl); }
+};
+
+template <int VEC> struct Vec16;
+template <> struct Vec16<8> { using type = uint4; };
+template <> struct Vec16<4> { using type = uint2; };
+template <> struct Vec16<2> { using type = unsigned; };
+template <> struct Vec16<1> { using type = unsigned short; };
+
+template <typename T, int VEC> struct CropIO16 {
+    using V = typename Vec16<VEC>::type;
+    static constexpr int NW = VEC >= 2 ? VEC / 2 : 1;     // 32-bit words per vector
+    static __device__ __forceinline__ V ld(const V *p) { return __ldg(p); }
+    static __device__ __forceinline__ V splat(float v)
+    {
+        if constexpr (VEC == 1) {
+            return Elem16<T>::narrow(v);
+        } else {
+            unsigned w[NW];
+            const unsigned h = Elem16<T>::narrow2(v, v);
+#pragma unroll
+            for (int i = 0; i < NW; ++i) w[i] = h;
+            V r;
+            __builtin_memcpy(&r, w, sizeof(V));
+            return r;
+        }
+    }
+    static __device__ __forceinline__ V lerp(V tl, V tr, V bl, V br, float xl, float yl)
+    {
+        using E = Elem16<T>;
+        if constexpr (VEC == 1) {
+            return E::narrow(lerp2(E::widen(tl), E::widen(tr), E::widen(bl), E::widen(br), xl, yl));
+        } else {
+            unsigned a[NW], b[NW], c[NW], d[NW], r[NW];
+            __builtin_memcpy(a, &tl, sizeof(V));
+            __builtin_memcpy(b, &tr, sizeof(V));
+            __builtin_memcpy(c, &bl, sizeof(V));
+            __builtin_memcpy(d, &br, sizeof(V));
+#pragma unroll
+            for (int i = 0; i < NW; ++i) {
+                float a0, a1, b0, b1, c0, c1, d0, d1;
+                E::widen2(a[i], a0, a1);
+                E::widen2(b[i], b0, b1);
+                E::widen2(c[i], c0, c1);
+                E::widen2(d[i], d0, d1);
+                const f32x2_t top = lerp_pair(pk2(a0, a1), pk2(b0, b1), xl), bot = lerp_pair(pk2(c0, c1), pk2(d0, d1), xl);
+                float r0, r1;
+                unpk2(lerp_pair(top, bot, yl), r0, r1);
+                r[i] = E::narrow2(r0, r1);
+            }
+            V out;
+            __builtin_memcpy(&out, r, sizeof(V));
+            return out;
+        }
+    }
+};
+template <int VEC> struct CropIO<__nv_bfloat16, VEC> : CropIO16<__nv_bfloat16, VEC> {};
+template <int VEC> struct CropIO<__half, VEC> : CropIO16<__half, VEC> {};
 
 }  // namespace sln

@@ -30,7 +30,7 @@ namespace sln {
 // forward, NHWC
 // ===========================================================================
 struct PyramidMaps {
-    const float *map[8];
+    const void *map[8];       // elements of the kernel's type T
     int H[8];
     int W[8];
 };
@@ -42,15 +42,16 @@ struct SampleRec {
     float xl, yl;
 };
 
-// img/out addressed in units of VEC floats.  LEVELS: take the source map from
-// `pm` by level[r]; otherwise use pm.map[0].
-template <int VEC, bool LEVELS>
+// img/out addressed in units of VEC elements of T (float, or a 2-byte type: see CropIO).  LEVELS: take the source map
+// from `pm` by level[r]; otherwise use pm.map[0].
+template <typename T, int VEC, bool LEVELS>
 __global__ void __launch_bounds__(256)
 crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ boxes,
                      const int *__restrict__ box_ind, const int *__restrict__ level, int n_levels,
-                     int ph, int pw, int band, float ext, float *__restrict__ out)
+                     int ph, int pw, int band, float ext, T *__restrict__ out)
 {
-    using V = typename VecT<VEC>::type;
+    using IO = CropIO<T, VEC>;
+    using V = typename IO::V;
     extern __shared__ __align__(16) unsigned char s_fwd_raw[];
     SampleRec *rec = reinterpret_cast<SampleRec *>(s_fwd_raw);      // [band]: samples [s_lo, s_hi) of the crop
 
@@ -64,7 +65,7 @@ crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ box
     // select the level with static indices (dynamic indexing would spill the
     // by-value parameter struct to local memory)
     int H = pm.H[0], W = pm.W[0];
-    const float *mp = pm.map[0];
+    const void *mp = pm.map[0];
     if (LEVELS && ok) {
 #pragma unroll
         for (int l = 1; l < 8; ++l)
@@ -76,7 +77,7 @@ crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ box
     const size_t out_base = ((size_t)r * ph * pw + s_lo) * CV;
 
     if (!ok) {   // reference GPU kernel skips such boxes (kernel.cu:34-38): rows stay zero
-        V z = make_splat(0.f, (V *)nullptr);
+        const V z = IO::splat(0.f);
         for (int i = tid; i < S * CV; i += nthr) o[out_base + i] = z;
         return;
     }
@@ -99,8 +100,8 @@ crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ box
     }
     __syncthreads();
 
-    const V vext = make_splat(ext, (V *)nullptr);
-    const V *__restrict__ img = reinterpret_cast<const V *>(mp) + (size_t)b * H * W * CV;
+    const V vext = IO::splat(ext);
+    const V *__restrict__ img = static_cast<const V *>(mp) + (size_t)b * H * W * CV;
     const int sstep = blockDim.y;
 
     for (int cv = threadIdx.x; cv < CV; cv += blockDim.x) {
@@ -112,15 +113,15 @@ crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ box
             const SampleRec qa = rec[s], qb = rec[s + sstep];
             V a0, a1, a2, a3, b0, b1, b2, b3;
             if (qa.o00 >= 0) {
-                a0 = ldg_vec(imc + qa.o00); a1 = ldg_vec(imc + qa.o01);
-                a2 = ldg_vec(imc + qa.o10); a3 = ldg_vec(imc + qa.o11);
+                a0 = IO::ld(imc + qa.o00); a1 = IO::ld(imc + qa.o01);
+                a2 = IO::ld(imc + qa.o10); a3 = IO::ld(imc + qa.o11);
             }
             if (qb.o00 >= 0) {
-                b0 = ldg_vec(imc + qb.o00); b1 = ldg_vec(imc + qb.o01);
-                b2 = ldg_vec(imc + qb.o10); b3 = ldg_vec(imc + qb.o11);
+                b0 = IO::ld(imc + qb.o00); b1 = IO::ld(imc + qb.o01);
+                b2 = IO::ld(imc + qb.o10); b3 = IO::ld(imc + qb.o11);
             }
-            const V ra = qa.o00 >= 0 ? lerp2v(a0, a1, a2, a3, qa.xl, qa.yl) : vext;
-            const V rb = qb.o00 >= 0 ? lerp2v(b0, b1, b2, b3, qb.xl, qb.yl) : vext;
+            const V ra = qa.o00 >= 0 ? IO::lerp(a0, a1, a2, a3, qa.xl, qa.yl) : vext;
+            const V rb = qb.o00 >= 0 ? IO::lerp(b0, b1, b2, b3, qb.xl, qb.yl) : vext;
             __stcs(oc + (size_t)s * CV, ra);
             __stcs(oc + (size_t)(s + sstep) * CV, rb);
         }
@@ -128,7 +129,7 @@ crop_fwd_nhwc_kernel(PyramidMaps pm, int B, int C, const float *__restrict__ box
             const SampleRec q = rec[s];
             V res = vext;
             if (q.o00 >= 0)
-                res = lerp2v(ldg_vec(imc + q.o00), ldg_vec(imc + q.o01), ldg_vec(imc + q.o10), ldg_vec(imc + q.o11), q.xl, q.yl);
+                res = IO::lerp(IO::ld(imc + q.o00), IO::ld(imc + q.o01), IO::ld(imc + q.o10), IO::ld(imc + q.o11), q.xl, q.yl);
             __stcs(oc + (size_t)s * CV, res);
         }
     }
@@ -1002,13 +1003,13 @@ crop_bwd_tile_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
 // ===========================================================================
 // layout converters: per image, [C][HW] <-> [HW][C]
 // ===========================================================================
-static bool aligned16_ptr(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
+// T: float, or unsigned short for every 2-byte type (the transposes move bits)
+template <typename T>
 __global__ void __launch_bounds__(256)
-transpose_kernel(const float *__restrict__ src, float *__restrict__ dst, int rows, int cols)
+transpose_kernel(const T *__restrict__ src, T *__restrict__ dst, int rows, int cols)
 {
     // src [batch][rows][cols] -> dst [batch][cols][rows]
-    __shared__ float tile[32][33];
+    __shared__ T tile[32][33];
     const size_t boff = (size_t)blockIdx.z * rows * cols;
     const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -1027,10 +1028,17 @@ transpose_kernel(const float *__restrict__ src, float *__restrict__ dst, int row
 // tile per CTA, 16-byte loads along the source rows, 16-byte stores along the destination rows.  The tile is stored
 // transposed with a 65-word pitch, so the four scalar writes of a loaded vector hit four different rows (banks 4 apart
 // plus the lane's own offset: conflict-free per quarter warp) and the 16-byte reads along a row are contiguous.
+// 2-byte elements move as 8-byte vectors of four (ushort4), with the same tile and thread mapping.
+template <typename T> struct Vec4T;
+template <> struct Vec4T<float> { using type = float4; };
+template <> struct Vec4T<unsigned short> { using type = ushort4; };
+
+template <typename T>
 __global__ void __launch_bounds__(256)
-transpose_v4_kernel(const float *__restrict__ src, float *__restrict__ dst, int rows, int cols)
+transpose_v4_kernel(const T *__restrict__ src, T *__restrict__ dst, int rows, int cols)
 {
-    __shared__ float tile[64][65];                              // tile[c][r] = src[r0 + r][c0 + c]
+    using V4 = typename Vec4T<T>::type;
+    __shared__ T tile[64][65];                                  // tile[c][r] = src[r0 + r][c0 + c]
     const size_t boff = (size_t)blockIdx.z * rows * cols;
     const int c0 = blockIdx.x * 64, r0 = blockIdx.y * 64;
     const int q = threadIdx.x & 15, j0 = threadIdx.x >> 4;      // 16 vectors per 64-float row, 16 rows per pass
@@ -1038,7 +1046,7 @@ transpose_v4_kernel(const float *__restrict__ src, float *__restrict__ dst, int 
     for (int k = 0; k < 4; ++k) {
         const int r = r0 + j0 + 16 * k, c = c0 + 4 * q;
         if (r < rows && c < cols) {
-            const float4 v = __ldcs(reinterpret_cast<const float4 *>(src + boff + (size_t)r * cols + c));
+            const V4 v = __ldcs(reinterpret_cast<const V4 *>(src + boff + (size_t)r * cols + c));
             tile[4 * q + 0][j0 + 16 * k] = v.x;
             tile[4 * q + 1][j0 + 16 * k] = v.y;
             tile[4 * q + 2][j0 + 16 * k] = v.z;
@@ -1050,25 +1058,30 @@ transpose_v4_kernel(const float *__restrict__ src, float *__restrict__ dst, int 
     for (int k = 0; k < 4; ++k) {
         const int c = c0 + j0 + 16 * k, r = r0 + 4 * q;          // destination row c, columns r .. r + 3
         if (c < cols && r < rows) {
-            const float *t = &tile[j0 + 16 * k][4 * q];
-            __stcs(reinterpret_cast<float4 *>(dst + boff + (size_t)c * rows + r), make_float4(t[0], t[1], t[2], t[3]));
+            const T *t = &tile[j0 + 16 * k][4 * q];
+            V4 o;
+            o.x = t[0]; o.y = t[1]; o.z = t[2]; o.w = t[3];
+            __stcs(reinterpret_cast<V4 *>(dst + boff + (size_t)c * rows + r), o);
         }
     }
 }
 
-static int launch_transpose(const float *src, float *dst, int batch, int rows, int cols, cudaStream_t st)
+template <typename T>
+static int launch_transpose(const T *src, T *dst, int batch, int rows, int cols, cudaStream_t st)
 {
+    constexpr uintptr_t a = 4 * sizeof(T) - 1;
+    const bool al = ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & a) == 0;
     if (batch == 0 || rows == 0 || cols == 0) return SLN_OK;
-    if (rows % 4 == 0 && cols % 4 == 0 && aligned16_ptr(src) && aligned16_ptr(dst) && batch <= 65535 && cdiv(rows, 64) <= 65535) {
+    if (rows % 4 == 0 && cols % 4 == 0 && al && batch <= 65535 && cdiv(rows, 64) <= 65535) {
         dim3 grid(cdiv(cols, 64), cdiv(rows, 64), batch);
-        transpose_v4_kernel<<<grid, 256, 0, st>>>(src, dst, rows, cols);
+        transpose_v4_kernel<T><<<grid, 256, 0, st>>>(src, dst, rows, cols);
         SLN_LAUNCH_OK("transpose_v4_kernel");
         return SLN_OK;
     }
     SLN_REQUIRE(cdiv(rows, 32) <= 65535 && batch <= 65535, SLN_ERR_ARG,
                 "transpose: rows/batch too large (%d, %d)", rows, batch);
     dim3 grid(cdiv(cols, 32), cdiv(rows, 32), batch);
-    transpose_kernel<<<grid, 256, 0, st>>>(src, dst, rows, cols);
+    transpose_kernel<T><<<grid, 256, 0, st>>>(src, dst, rows, cols);
     SLN_LAUNCH_OK("transpose_kernel");
     return SLN_OK;
 }
@@ -1102,13 +1115,37 @@ static void fwd_block_shape(int CV, dim3 &block)
     block = dim3(bx, by, 1);
 }
 
+// widest vector of VEC elements that C and every pointer allow: 16 bytes (float4 / 8 x 2-byte) down to one element
+template <typename T, int VEC>
+static bool fwd_vec_ok(const PyramidMaps &pm, int n_levels, int C, const void *out)
+{
+    constexpr uintptr_t a = sizeof(T) * VEC - 1;
+    bool ok = C % VEC == 0 && (reinterpret_cast<uintptr_t>(out) & a) == 0;
+    for (int l = 0; l < n_levels; ++l) ok = ok && (reinterpret_cast<uintptr_t>(pm.map[l]) & a) == 0;
+    return ok;
+}
+
+template <typename T, int VEC>
+static void launch_fwd_nhwc(dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool levels, const PyramidMaps &pm, int n_levels,
+                            int B, int C, const float *boxes, const int *box_ind, const int *level, int ph, int pw, int band,
+                            float ext, T *out)
+{
+    if (levels) crop_fwd_nhwc_kernel<T, VEC, true><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
+    else crop_fwd_nhwc_kernel<T, VEC, false><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
+}
+
+template <typename T>
 static int crop_fwd_nhwc(const PyramidMaps &pm, int n_levels, bool levels, int B, int C,
                          const float *boxes, const int *box_ind, const int *level, int N, int ph, int pw,
-                         float ext, float *out, cudaStream_t st)
+                         float ext, T *out, cudaStream_t st)
 {
-    bool vec4 = (C % 4 == 0) && aligned16(out);
-    for (int l = 0; l < n_levels; ++l) vec4 = vec4 && aligned16(pm.map[l]);
-    const int CV = vec4 ? C / 4 : C;
+    constexpr bool F32 = sizeof(T) == 4;
+    constexpr int VMAX = 16 / sizeof(T);                     // elements per 16-byte vector
+    int vec = 1;
+    if (fwd_vec_ok<T, VMAX>(pm, n_levels, C, out)) vec = VMAX;
+    else if (!F32 && fwd_vec_ok<T, 4>(pm, n_levels, C, out)) vec = 4;
+    else if (!F32 && fwd_vec_ok<T, 2>(pm, n_levels, C, out)) vec = 2;
+    const int CV = C / vec;
     dim3 block;
     fwd_block_shape(CV, block);
     const int band = ph * pw < 2048 ? ph * pw : 2048;        // samples per CTA (48 KB of records at most)
@@ -1118,15 +1155,33 @@ static int crop_fwd_nhwc(const PyramidMaps &pm, int n_levels, bool levels, int B
     SLN_REQUIRE(plane_max * (size_t)CV < (1ull << 31), SLN_ERR_ARG, "feature map too large for 32-bit tap offsets");
     dim3 grid(N, cdiv(ph * pw, band));
     SLN_REQUIRE(grid.y <= 65535, SLN_ERR_ARG, "crop too large");
-    if (vec4) {
-        if (levels) crop_fwd_nhwc_kernel<4, true><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
-        else crop_fwd_nhwc_kernel<4, false><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
+    if constexpr (F32) {
+        if (vec == 4) launch_fwd_nhwc<T, 4>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
+        else launch_fwd_nhwc<T, 1>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
     } else {
-        if (levels) crop_fwd_nhwc_kernel<1, true><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
-        else crop_fwd_nhwc_kernel<1, false><<<grid, block, smem, st>>>(pm, B, C, boxes, box_ind, level, n_levels, ph, pw, band, ext, out);
+        if (vec == 8) launch_fwd_nhwc<T, 8>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
+        else if (vec == 4) launch_fwd_nhwc<T, 4>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
+        else if (vec == 2) launch_fwd_nhwc<T, 2>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
+        else launch_fwd_nhwc<T, 1>(grid, block, smem, st, levels, pm, n_levels, B, C, boxes, box_ind, level, ph, pw, band, ext, out);
     }
     SLN_LAUNCH_OK("crop_fwd_nhwc_kernel");
     return SLN_OK;
+}
+
+// the forward of a call whose element type is named by an SLN_DTYPE_* code
+static int crop_fwd_nhwc_dt(int dtype, const PyramidMaps &pm, int n_levels, bool levels, int B, int C, const float *boxes,
+                            const int *box_ind, const int *level, int N, int ph, int pw, float ext, void *out, cudaStream_t st)
+{
+    switch (dtype) {
+    case SLN_DTYPE_F32:
+        return crop_fwd_nhwc(pm, n_levels, levels, B, C, boxes, box_ind, level, N, ph, pw, ext, static_cast<float *>(out), st);
+    case SLN_DTYPE_BF16:
+        return crop_fwd_nhwc(pm, n_levels, levels, B, C, boxes, box_ind, level, N, ph, pw, ext, static_cast<__nv_bfloat16 *>(out), st);
+    case SLN_DTYPE_F16:
+        return crop_fwd_nhwc(pm, n_levels, levels, B, C, boxes, box_ind, level, N, ph, pw, ext, static_cast<__half *>(out), st);
+    }
+    SLN_REQUIRE(false, SLN_ERR_ARG, "unknown dtype %d", dtype);
+    return SLN_ERR_ARG;
 }
 
 struct BwdWs {
@@ -1191,16 +1246,24 @@ static unsigned bwd_tma_grid(long long n_work)
     return (unsigned)(n_work < resident ? n_work : resident);
 }
 
-// One configuration of the bulk-async kernel (stage size, ring depth; see crop_bwd_tma.cuh).
-template <bool EXACT, int STG_S, int NST>
-static int launch_bwd_tma_cfg(const float *grads, const BwdWs &ws, const BwdTileBases &TB, long long n_work, int chunks, int C,
+// One configuration of the bulk-async kernel (stage size, ring depth; see crop_bwd_tma.cuh).  2-byte element types keep
+// the fp32 stage geometry (samples per stage, ring depth); their stages take half the bytes.
+template <typename T, bool EXACT, int STG_S, int NST>
+static int launch_bwd_tma_cfg(const T *grads, const BwdWs &ws, const BwdTileBases &TB, long long n_work, int chunks, int C,
                               int ph, int pw, cudaStream_t st)
 {
-    const size_t smem = bwdtma::smem_bytes<STG_S, NST>();
-    auto kern = C % 256 == 0  ? bwdtma::crop_bwd_tma_kernel<2, EXACT, true, STG_S, NST>
-                : C == 128    ? bwdtma::crop_bwd_tma_kernel<1, EXACT, true, STG_S, NST>
-                : C > 128     ? bwdtma::crop_bwd_tma_kernel<2, EXACT, false, STG_S, NST>
-                              : bwdtma::crop_bwd_tma_kernel<1, EXACT, false, STG_S, NST>;
+    const size_t smem = bwdtma::smem_bytes<STG_S, NST, sizeof(T)>();
+    void (*kern)(const T *, const ListEntryA *, const int *, const int *, const BwdLevel *, BwdTileBases, int, int, int, int,
+                 int, int *);
+    if constexpr (sizeof(T) == 4) {
+        kern = C % 256 == 0  ? bwdtma::crop_bwd_tma_kernel<2, EXACT, true, STG_S, NST>
+               : C == 128    ? bwdtma::crop_bwd_tma_kernel<1, EXACT, true, STG_S, NST>
+               : C > 128     ? bwdtma::crop_bwd_tma_kernel<2, EXACT, false, STG_S, NST>
+                             : bwdtma::crop_bwd_tma_kernel<1, EXACT, false, STG_S, NST>;
+    } else {
+        kern = C % 256 == 0 ? bwdtma::crop_bwd_tma_b16_kernel<T, EXACT, true, STG_S, NST>
+                            : bwdtma::crop_bwd_tma_b16_kernel<T, EXACT, false, STG_S, NST>;
+    }
     SLN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // work-item tickets: tickets below `grid` are the CTAs' first items (the counter starts there, set by the windows kernel)
     const unsigned grid = bwd_tma_grid(n_work);
@@ -1213,8 +1276,8 @@ static int launch_bwd_tma_cfg(const float *grads, const BwdWs &ws, const BwdTile
     return SLN_OK;
 }
 
-template <bool EXACT>
-static int launch_bwd_tma(const float *grads, const BwdWs &ws, const BwdParams &P, long long tiles, int C, int ph, int pw,
+template <typename T, bool EXACT>
+static int launch_bwd_tma(const T *grads, const BwdWs &ws, const BwdParams &P, long long tiles, int C, int ph, int pw,
                           cudaStream_t st)
 {
     const int chunks = cdiv(C, bwdtma::CH_MAX);
@@ -1228,8 +1291,31 @@ static int launch_bwd_tma(const float *grads, const BwdWs &ws, const BwdParams &
     // SLN_BWD_CFG=0/1 in the environment forces one for A/B runs.
     const char *e = getenv("SLN_BWD_CFG");
     const bool small = (e && (e[0] == '0' || e[0] == '1')) ? e[0] == '1' : ph * pw <= 64;
-    if (small) return launch_bwd_tma_cfg<EXACT, 16, 6>(grads, ws, TB, n_work, chunks, C, ph, pw, st);
-    return launch_bwd_tma_cfg<EXACT, 32, 3>(grads, ws, TB, n_work, chunks, C, ph, pw, st);
+    if (small) return launch_bwd_tma_cfg<T, EXACT, 16, 6>(grads, ws, TB, n_work, chunks, C, ph, pw, st);
+    return launch_bwd_tma_cfg<T, EXACT, 32, 3>(grads, ws, TB, n_work, chunks, C, ph, pw, st);
+}
+
+// the bulk-async kernel for the element type named by an SLN_DTYPE_* code
+static int launch_bwd_tma_dt(int dtype, const void *grads, bool exact, const BwdWs &ws, const BwdParams &P, long long tiles,
+                             int C, int ph, int pw, cudaStream_t st)
+{
+    switch (dtype) {
+    case SLN_DTYPE_BF16: {
+        const __nv_bfloat16 *g = static_cast<const __nv_bfloat16 *>(grads);
+        return exact ? launch_bwd_tma<__nv_bfloat16, true>(g, ws, P, tiles, C, ph, pw, st)
+                     : launch_bwd_tma<__nv_bfloat16, false>(g, ws, P, tiles, C, ph, pw, st);
+    }
+    case SLN_DTYPE_F16: {
+        const __half *g = static_cast<const __half *>(grads);
+        return exact ? launch_bwd_tma<__half, true>(g, ws, P, tiles, C, ph, pw, st)
+                     : launch_bwd_tma<__half, false>(g, ws, P, tiles, C, ph, pw, st);
+    }
+    default: {
+        const float *g = static_cast<const float *>(grads);
+        return exact ? launch_bwd_tma<float, true>(g, ws, P, tiles, C, ph, pw, st)
+                     : launch_bwd_tma<float, false>(g, ws, P, tiles, C, ph, pw, st);
+    }
+    }
 }
 
 template <int VEC, int NV, bool EXACT>
@@ -1289,10 +1375,14 @@ static int dispatch_bwd(const float *grads, const BwdWs &ws, const BwdParams &P,
 // plausible addresses); 2 (SLN_BWD_PLANNED): the workspace holds the lists of a mode-1 call with the same boxes, box_ind,
 // level, N, C, ph, pw, B and map sizes -- skip the three prep launches.  Only the bulk-async form plans ahead; the other
 // forms ignore mode 1 and treat mode 2 as mode 0.
-static int crop_bwd_nhwc(const float *grads, const float *boxes, const int *box_ind, const int *level, int N, int C,
+// dtype: element type of grads and maps (SLN_DTYPE_*).  2-byte types run the bulk-async kernel only (C % 8 == 0, crops
+// of at most 32 per side, 16-byte aligned pointers); other shapes are refused.  A plan does not depend on the dtype: the
+// prep kernels see boxes and sizes only, and the tile grid (8 x 8) and channel chunks (256) are the same for every type.
+static int crop_bwd_nhwc(int dtype, const void *grads, const float *boxes, const int *box_ind, const int *level, int N, int C,
                          int ph, int pw, float *const *maps, const int *Hs, const int *Ws, int n_levels, int B,
                          bool exact, void *wsp, size_t ws_bytes, cudaStream_t st, int mode = 0)
 {
+    SLN_REQUIRE(dtype == SLN_DTYPE_F32 || dtype == SLN_DTYPE_BF16 || dtype == SLN_DTYPE_F16, SLN_ERR_ARG, "unknown dtype %d", dtype);
     if (B == 0 || C == 0) return SLN_OK;
     SLN_REQUIRE(ws_bytes >= bwd_ws_bytes(N, B, n_levels, ph, pw), SLN_ERR_WORKSPACE,
                 "crop bwd workspace: need %zu bytes, got %zu", bwd_ws_bytes(N, B, n_levels, ph, pw), ws_bytes);
@@ -1303,7 +1393,15 @@ static int crop_bwd_nhwc(const float *grads, const float *boxes, const int *box_
     long long tiles = 0;
     bool vec4 = (C % 4 == 0) && (mode == 1 || aligned16(grads));
     for (int l = 0; l < n_levels; ++l) vec4 = vec4 && (mode == 1 || aligned16(maps[l]));
-    const bool use_tma = bwd_use_tma(ph, pw, vec4);
+    bool use_tma = bwd_use_tma(ph, pw, vec4);
+    if (dtype != SLN_DTYPE_F32 && mode != 1) {
+        bool ok = C % 8 == 0 && ph <= bwdtma::MAX_POOL && pw <= bwdtma::MAX_POOL && aligned16(grads);
+        for (int l = 0; l < n_levels; ++l) ok = ok && aligned16(maps[l]);
+        SLN_REQUIRE(ok, SLN_ERR_LAYOUT, "2-byte crop backward needs C %% 8 == 0 (C = %d), crops of at most 32 per side "
+                    "(%dx%d) and 16-byte aligned grads and grad maps", C, ph, pw);
+        if (mode == 2 && !use_tma) mode = 0;    // SLN_BWD_IMPL chose another form for fp32: no plan was built
+        use_tma = true;
+    }
     if (!use_tma) {
         if (mode == 1) return SLN_OK;
         mode = 0;
@@ -1369,8 +1467,7 @@ static int crop_bwd_nhwc(const float *grads, const float *boxes, const int *box_
         SLN_CUDA_OK(launch_chain(crop_bwd_republish_kernel, dim3(1), dim3(32), 0, st, true, P, ws.lv_table, ws.queue,
                                  (int)bwd_tma_grid(tiles * cdiv(C, bwdtma::CH_MAX))));
         SLN_LAUNCH_OK("crop_bwd_republish_kernel");
-        if (exact) return launch_bwd_tma<true>(grads, ws, P, tiles, C, ph, pw, st);
-        return launch_bwd_tma<false>(grads, ws, P, tiles, C, ph, pw, st);
+        return launch_bwd_tma_dt(dtype, grads, exact, ws, P, tiles, C, ph, pw, st);
     }
     SLN_CUDA_OK(cudaMemsetAsync(ws.st_count, 0, sizeof(int) * (size_t)(n_st + 1), st));
     // the windows kernel also publishes the level table, so it always runs (>= 1 CTA)
@@ -1390,16 +1487,14 @@ static int crop_bwd_nhwc(const float *grads, const float *boxes, const int *box_
         SLN_LAUNCH_OK("crop_bwd_fill_kernel");
     }
     if (mode == 1) return SLN_OK;
-    if (use_tma) {
-        if (exact) return launch_bwd_tma<true>(grads, ws, P, tiles, C, ph, pw, st);
-        return launch_bwd_tma<false>(grads, ws, P, tiles, C, ph, pw, st);
-    }
+    if (use_tma) return launch_bwd_tma_dt(dtype, grads, exact, ws, P, tiles, C, ph, pw, st);
+    const float *g32 = static_cast<const float *>(grads);
     if (vec4) {
-        if (exact) return dispatch_bwd<4, true>(grads, ws, P, tiles, C, ph, pw, st);
-        return dispatch_bwd<4, false>(grads, ws, P, tiles, C, ph, pw, st);
+        if (exact) return dispatch_bwd<4, true>(g32, ws, P, tiles, C, ph, pw, st);
+        return dispatch_bwd<4, false>(g32, ws, P, tiles, C, ph, pw, st);
     }
-    if (exact) return dispatch_bwd<1, true>(grads, ws, P, tiles, C, ph, pw, st);
-    return dispatch_bwd<1, false>(grads, ws, P, tiles, C, ph, pw, st);
+    if (exact) return dispatch_bwd<1, true>(g32, ws, P, tiles, C, ph, pw, st);
+    return dispatch_bwd<1, false>(g32, ws, P, tiles, C, ph, pw, st);
 }
 
 }  // namespace sln
@@ -1409,10 +1504,11 @@ static int crop_bwd_nhwc(const float *grads, const float *boxes, const int *box_
 // ===========================================================================
 using namespace sln;
 
-extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, int W, int layout,
-                                       const float *boxes, const int *box_ind, int N, int ph, int pw,
-                                       float ext, float *crops, void *stream)
+extern "C" int sln_crop_and_resize_fwd_ex(int dtype, const void *image, int B, int C, int H, int W, int layout,
+                                          const float *boxes, const int *box_ind, int N, int ph, int pw,
+                                          float ext, void *crops, void *stream)
 {
+    SLN_REQUIRE(dtype == SLN_DTYPE_F32 || dtype == SLN_DTYPE_BF16 || dtype == SLN_DTYPE_F16, SLN_ERR_ARG, "unknown dtype %d", dtype);
     int rc = check_crop_args(image, boxes, box_ind, crops, B, C, H, W, N, ph, pw, 4096);
     if (rc != SLN_OK) return rc;
     if (N == 0 || C == 0) return SLN_OK;
@@ -1420,9 +1516,10 @@ extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, 
     if (layout == SLN_LAYOUT_NHWC) {
         PyramidMaps pm{};
         pm.map[0] = image; pm.H[0] = H; pm.W[0] = W;
-        return crop_fwd_nhwc(pm, 1, false, B, C, boxes, box_ind, nullptr, N, ph, pw, ext, crops, st);
+        return crop_fwd_nhwc_dt(dtype, pm, 1, false, B, C, boxes, box_ind, nullptr, N, ph, pw, ext, crops, st);
     }
     SLN_REQUIRE(layout == SLN_LAYOUT_NCHW, SLN_ERR_LAYOUT, "unknown layout %d", layout);
+    SLN_REQUIRE(dtype == SLN_DTYPE_F32, SLN_ERR_LAYOUT, "2-byte crop forward is NHWC-only; convert with sln_nchw_to_nhwc_b16");
     // channel chunks so that small-N calls still fill the machine
     int c_chunk = C;
     const int want_ctas = 4 * sm_count();
@@ -1437,9 +1534,17 @@ extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, 
     const size_t smem = sizeof(Tap) * (size_t)(ph + pw);
     if (smem > 48 * 1024)
         SLN_CUDA_OK(cudaFuncSetAttribute(crop_fwd_nchw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    crop_fwd_nchw_kernel<<<grid, 256, smem, st>>>(image, B, C, H, W, boxes, box_ind, ph, pw, ext, c_chunk, crops);
+    crop_fwd_nchw_kernel<<<grid, 256, smem, st>>>(static_cast<const float *>(image), B, C, H, W, boxes, box_ind, ph, pw, ext,
+                                                  c_chunk, static_cast<float *>(crops));
     SLN_LAUNCH_OK("crop_fwd_nchw_kernel");
     return SLN_OK;
+}
+
+extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, int W, int layout,
+                                       const float *boxes, const int *box_ind, int N, int ph, int pw,
+                                       float ext, float *crops, void *stream)
+{
+    return sln_crop_and_resize_fwd_ex(SLN_DTYPE_F32, image, B, C, H, W, layout, boxes, box_ind, N, ph, pw, ext, crops, stream);
 }
 
 extern "C" size_t sln_crop_and_resize_bwd_workspace_bytes(int N, int B, int ph, int pw)
@@ -1448,9 +1553,9 @@ extern "C" size_t sln_crop_and_resize_bwd_workspace_bytes(int N, int B, int ph, 
     return bwd_ws_bytes(N, B, 1, ph, pw);
 }
 
-extern "C" int sln_crop_and_resize_bwd(const float *grads, const float *boxes, const int *box_ind, int N,
-                                       int C, int ph, int pw, float *grad_image, int B, int H, int W,
-                                       int layout, int flags, void *workspace, size_t workspace_bytes, void *stream)
+extern "C" int sln_crop_and_resize_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind, int N,
+                                          int C, int ph, int pw, void *grad_image, int B, int H, int W,
+                                          int layout, int flags, void *workspace, size_t workspace_bytes, void *stream)
 {
     SLN_REQUIRE(layout == SLN_LAYOUT_NHWC, SLN_ERR_LAYOUT,
                 "crop backward is NHWC-only; convert with sln_nchw_to_nhwc / sln_nhwc_to_nchw");
@@ -1458,15 +1563,23 @@ extern "C" int sln_crop_and_resize_bwd(const float *grads, const float *boxes, c
     if (rc != SLN_OK) return rc;
     SLN_REQUIRE(N == 0 || C == 0 || grads, SLN_ERR_ARG, "null grads");
     if (H == 0 || W == 0) return SLN_OK;
-    float *maps[1] = {grad_image};
-    return crop_bwd_nhwc(grads, boxes, box_ind, nullptr, N, C, ph, pw, maps, &H, &W, 1, B,
+    float *maps[1] = {static_cast<float *>(grad_image)};
+    return crop_bwd_nhwc(dtype, grads, boxes, box_ind, nullptr, N, C, ph, pw, maps, &H, &W, 1, B,
                          (flags & SLN_BWD_EXACT) != 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int sln_pyramid_crop_fwd(const float *const *maps_host, const int *H_host, const int *W_host,
-                                    int n_levels, int B, int C, const float *boxes, const int *box_ind,
-                                    const int *level, int N, int ph, int pw, float ext, float *crops,
-                                    void *stream)
+extern "C" int sln_crop_and_resize_bwd(const float *grads, const float *boxes, const int *box_ind, int N,
+                                       int C, int ph, int pw, float *grad_image, int B, int H, int W,
+                                       int layout, int flags, void *workspace, size_t workspace_bytes, void *stream)
+{
+    return sln_crop_and_resize_bwd_ex(SLN_DTYPE_F32, grads, boxes, box_ind, N, C, ph, pw, grad_image, B, H, W, layout, flags,
+                                      workspace, workspace_bytes, stream);
+}
+
+extern "C" int sln_pyramid_crop_fwd_ex(int dtype, const void *const *maps_host, const int *H_host, const int *W_host,
+                                       int n_levels, int B, int C, const float *boxes, const int *box_ind,
+                                       const int *level, int N, int ph, int pw, float ext, void *crops,
+                                       void *stream)
 {
     SLN_REQUIRE(n_levels >= 1 && n_levels <= 8, SLN_ERR_ARG, "n_levels %d outside [1,8]", n_levels);
     SLN_REQUIRE(maps_host && H_host && W_host && level, SLN_ERR_ARG, "null pointer");
@@ -1477,8 +1590,17 @@ extern "C" int sln_pyramid_crop_fwd(const float *const *maps_host, const int *H_
         pm.map[l] = maps_host[l]; pm.H[l] = H_host[l]; pm.W[l] = W_host[l];
     }
     if (N == 0 || C == 0) return SLN_OK;
-    return crop_fwd_nhwc(pm, n_levels, true, B, C, boxes, box_ind, level, N, ph, pw, ext, crops,
-                         static_cast<cudaStream_t>(stream));
+    return crop_fwd_nhwc_dt(dtype, pm, n_levels, true, B, C, boxes, box_ind, level, N, ph, pw, ext, crops,
+                            static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sln_pyramid_crop_fwd(const float *const *maps_host, const int *H_host, const int *W_host,
+                                    int n_levels, int B, int C, const float *boxes, const int *box_ind,
+                                    const int *level, int N, int ph, int pw, float ext, float *crops,
+                                    void *stream)
+{
+    return sln_pyramid_crop_fwd_ex(SLN_DTYPE_F32, reinterpret_cast<const void *const *>(maps_host), H_host, W_host, n_levels, B, C,
+                                   boxes, box_ind, level, N, ph, pw, ext, crops, stream);
 }
 
 extern "C" size_t sln_pyramid_crop_bwd_workspace_bytes(int N, int B, int n_levels, int ph, int pw)
@@ -1487,10 +1609,10 @@ extern "C" size_t sln_pyramid_crop_bwd_workspace_bytes(int N, int B, int n_level
     return bwd_ws_bytes(N, B, n_levels, ph, pw);
 }
 
-extern "C" int sln_pyramid_crop_bwd(const float *grads, const float *boxes, const int *box_ind, const int *level,
-                                    int N, int C, int ph, int pw, float *const *grad_maps_host, const int *H_host,
-                                    const int *W_host, int n_levels, int B, int flags, void *workspace,
-                                    size_t workspace_bytes, void *stream)
+extern "C" int sln_pyramid_crop_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind, const int *level,
+                                       int N, int C, int ph, int pw, void *const *grad_maps_host, const int *H_host,
+                                       const int *W_host, int n_levels, int B, int flags, void *workspace,
+                                       size_t workspace_bytes, void *stream)
 {
     SLN_REQUIRE(n_levels >= 1 && n_levels <= BWD_MAX_LEVELS, SLN_ERR_ARG, "n_levels %d outside [1,8]", n_levels);
     SLN_REQUIRE(grad_maps_host && H_host && W_host, SLN_ERR_ARG, "null pointer");
@@ -1501,8 +1623,19 @@ extern "C" int sln_pyramid_crop_bwd(const float *grads, const float *boxes, cons
     }
     const int mode = (flags & SLN_BWD_PLAN_ONLY) ? 1 : ((flags & SLN_BWD_PLANNED) ? 2 : 0);
     SLN_REQUIRE(N == 0 || C == 0 || grads || mode == 1, SLN_ERR_ARG, "null grads");
-    return crop_bwd_nhwc(grads, boxes, box_ind, level, N, C, ph, pw, grad_maps_host, H_host, W_host, n_levels, B,
-                         (flags & SLN_BWD_EXACT) != 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), mode);
+    return crop_bwd_nhwc(dtype, grads, boxes, box_ind, level, N, C, ph, pw, reinterpret_cast<float *const *>(grad_maps_host),
+                         H_host, W_host, n_levels, B, (flags & SLN_BWD_EXACT) != 0, workspace, workspace_bytes,
+                         static_cast<cudaStream_t>(stream), mode);
+}
+
+extern "C" int sln_pyramid_crop_bwd(const float *grads, const float *boxes, const int *box_ind, const int *level,
+                                    int N, int C, int ph, int pw, float *const *grad_maps_host, const int *H_host,
+                                    const int *W_host, int n_levels, int B, int flags, void *workspace,
+                                    size_t workspace_bytes, void *stream)
+{
+    return sln_pyramid_crop_bwd_ex(SLN_DTYPE_F32, grads, boxes, box_ind, level, N, C, ph, pw,
+                                   reinterpret_cast<void *const *>(grad_maps_host), H_host, W_host, n_levels, B, flags,
+                                   workspace, workspace_bytes, stream);
 }
 
 // FPN level of every ROI, modal/modals.py:53-64, with the exact fp32 operation sequence the reference's torch
@@ -1540,7 +1673,8 @@ extern "C" int sln_roi_levels(const float *boxes, int N, int image_h, int image_
     return SLN_OK;
 }
 
-extern "C" int sln_nchw_to_nhwc(const float *src, float *dst, int B, int C, int H, int W, void *stream)
+template <typename T>
+static int nchw_to_nhwc(const T *src, T *dst, int B, int C, int H, int W, void *stream)
 {
     SLN_REQUIRE(B >= 0 && C >= 0 && H >= 0 && W >= 0, SLN_ERR_ARG, "negative size");
     SLN_REQUIRE((size_t)H * W < (1ull << 31), SLN_ERR_ARG, "plane too large");
@@ -1549,11 +1683,32 @@ extern "C" int sln_nchw_to_nhwc(const float *src, float *dst, int B, int C, int 
     return launch_transpose(src, dst, B, C, H * W, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int sln_nhwc_to_nchw(const float *src, float *dst, int B, int C, int H, int W, void *stream)
+template <typename T>
+static int nhwc_to_nchw(const T *src, T *dst, int B, int C, int H, int W, void *stream)
 {
     SLN_REQUIRE(B >= 0 && C >= 0 && H >= 0 && W >= 0, SLN_ERR_ARG, "negative size");
     SLN_REQUIRE((size_t)H * W < (1ull << 31), SLN_ERR_ARG, "plane too large");
     if ((size_t)B * C * H * W == 0) return SLN_OK;
     SLN_REQUIRE(src && dst && src != dst, SLN_ERR_ARG, "null or aliased pointers");
     return launch_transpose(src, dst, B, H * W, C, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sln_nchw_to_nhwc(const float *src, float *dst, int B, int C, int H, int W, void *stream)
+{
+    return nchw_to_nhwc(src, dst, B, C, H, W, stream);
+}
+
+extern "C" int sln_nhwc_to_nchw(const float *src, float *dst, int B, int C, int H, int W, void *stream)
+{
+    return nhwc_to_nchw(src, dst, B, C, H, W, stream);
+}
+
+extern "C" int sln_nchw_to_nhwc_b16(const uint16_t *src, uint16_t *dst, int B, int C, int H, int W, void *stream)
+{
+    return nchw_to_nhwc(src, dst, B, C, H, W, stream);
+}
+
+extern "C" int sln_nhwc_to_nchw_b16(const uint16_t *src, uint16_t *dst, int B, int C, int H, int W, void *stream)
+{
+    return nhwc_to_nchw(src, dst, B, C, H, W, stream);
 }

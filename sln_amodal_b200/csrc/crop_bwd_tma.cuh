@@ -12,7 +12,7 @@
 //     samples reach the tile -- into STAGES of up to STG_S samples (whole sample rows).  A stage is a descriptor
 //     (per tile row the range of stage rows that reach it; per stage row its top tile row and lerp; per sample column
 //     the tile column of its left tap and its lerp) plus the gradient vectors themselves, fetched by cp.async.bulk
-//     (one per sample row: n * C * 4 contiguous bytes; SASS UBLKCP) into a ring of shared-memory stages.  An mbarrier
+//     (one per sample row: n * C * sizeof(T) contiguous bytes; SASS UBLKCP) into a ring of shared-memory stages.  An mbarrier
 //     per stage counts the bytes in (complete_tx); a second one counts the eight consumers out.  The producer runs
 //     ahead of the consumers by the depth of the ring, across tile boundaries: the list heads of the next two tiles and
 //     the tap tables of the next ROI are in flight while the current ROI is planned.
@@ -57,9 +57,9 @@ struct StageDesc {
     XEnt x[STG_S];      // per sample column of the stage
 };
 struct TileOut {     // overlays StageDesc::rows for ST_TILE_END
-    unsigned long long out;   // float4* of pixel (b, y0, x0), channel c0
-    int row_stride;           // float4 per map row
-    int pix_stride;           // float4 per pixel
+    unsigned long long out;   // address of pixel (b, y0, x0), channel c0
+    int row_stride;           // 16-byte vectors per map row
+    int pix_stride;           // 16-byte vectors per pixel
     int ny, nx;               // valid rows / columns of the tile
 };
 
@@ -119,7 +119,7 @@ __device__ __forceinline__ float4 term(float4 a, float4 g, float w, float wy, fl
 #define SLN_TMA_ADD(K, W, WY, WX)                                                  \
     {                                                                              \
         acc[K][0] = term<EXACT>(acc[K][0], g0, W, WY, WX);                         \
-        if (NV == 2) acc[K][1] = term<EXACT>(acc[K][1], g1, W, WY, WX);            \
+        if (NACC == 2) acc[K][1] = term<EXACT>(acc[K][1], g1, W, WY, WX);          \
     }
 
 // The run [k0, k0 + n) of sample indices k in [0, crop) whose position pos(k) = base + k * scale (rounded exactly like
@@ -212,18 +212,26 @@ __device__ __forceinline__ TileGeom tile_geom(int w, int chunks, const BwdTileBa
     return g;
 }
 
-// FULL: the CTA's channel chunk fills every lane's vectors (CH == 128 * NV), so no lane predicates
-template <int NV, bool EXACT, bool FULL, int STG_S, int NST>
-__global__ void __launch_bounds__(THREADS, 2)
-crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restrict__ entries, const int *__restrict__ st_off,
-                    const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
-                    BwdTileBases TB, int C, int ph, int pw, int n_work, int chunks, int *__restrict__ queue)
+// T: element type of grads and grad maps -- float, or a 2-byte type (__nv_bfloat16 / __half) that the consumers widen on
+// the shared-memory read and round once on the write; the accumulators and their arithmetic are fp32 either way.
+// NV: 16-byte vectors per consumer lane (fp32: 1 or 2, i.e. 4 or 8 channels; 2-byte types: 1, i.e. 8 channels).
+// FULL: the CTA's channel chunk fills every lane's vectors (CH == 32 * NV * 16 / sizeof(T)), so no lane predicates.
+// The kernels are the two __global__ wrappers below: crop_bwd_tma_kernel (f32) and crop_bwd_tma_b16_kernel (2-byte types).
+template <typename T, int NV, bool EXACT, bool FULL, int STG_S, int NST>
+__device__ __forceinline__ void
+crop_bwd_tma_body(const T *__restrict__ grads, const ListEntryA *__restrict__ entries, const int *__restrict__ st_off,
+                  const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
+                  BwdTileBases TB, int C, int ph, int pw, int n_work, int chunks, int *__restrict__ queue)
 {
     extern __shared__ __align__(128) unsigned char s_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
     static_assert(STG_S >= 8 && STG_S <= 32, "a consumer finds its sample columns with one 32-lane ballot");
-    constexpr int STAGE_BYTES = STG_S * CH_MAX * 4;
+    constexpr int ESZ = sizeof(T);
+    constexpr int VPV = 16 / ESZ;                         // elements per 16-byte vector
+    constexpr int NACC = ESZ == 4 ? NV : 2;               // float4 accumulators per pixel and lane
+    static_assert(ESZ == 4 || NV == 1, "2-byte elements: one 16-byte vector (8 channels) per lane");
+    constexpr int STAGE_BYTES = STG_S * CH_MAX * ESZ;
     using Desc = StageDesc<STG_S>;
     // ---- shared memory carve-up
     unsigned char *stages = s_raw;                                                    // [NST][STAGE_BYTES]
@@ -307,7 +315,7 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
             const BwdLevel &L = lv[gC.l];
             const int y0 = gC.y0, x0 = gC.x0, y1 = gC.y1, x1 = gC.x1, c0 = gC.c0;
             const int CH = min(C - c0, CH_MAX);
-            const int chb = CH * 4;
+            const int chb = CH * ESZ;
             const float em1y = (float)(L.H - 1), em1x = (float)(L.W - 1);
             const int n_list = cntC;
             const ListEntryA *__restrict__ list = entries + offC;
@@ -344,7 +352,7 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
                     XEnt my_col;
                     my_col.pl = tx.lo - x0;
                     my_col.xl = tx.lerp;
-                    const float *gr = grads + go;
+                    const T *gr = grads + go;
                     // stages: whole sample rows, as many as fit; a row longer than a stage takes several stages
                     const int n_s_full = pk2 >> 8;
                     const int rows_per = pk2 & 0xff;
@@ -364,7 +372,7 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
                             // pending arrival), so bytes landing ahead of the expect_tx only drive the count negative for a while
                             if (row_mine) {                  // lane ra + i fetches stage row i
                                 const uint32_t dst = smem_u32(stages + (size_t)s * STAGE_BYTES) + rrow * n_s * chb;
-                                const float *src = gr + ((size_t)lane * pw + sb) * C;
+                                const T *src = gr + ((size_t)lane * pw + sb) * C;
                                 if (CH == C) {
                                     bulk_g2s(dst, src, (uint32_t)(n_s * chb), bar);
                                 } else {                     // channel chunk of a wider map: one copy per sample
@@ -386,9 +394,9 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
                     d->flags = ST_TILE_END;
                     d->n_s = CH;
                     TileOut o;
-                    o.out = (unsigned long long)(L.out + (((size_t)gC.b * L.H + y0) * L.W + x0) * C + c0);
-                    o.row_stride = L.W * (C / 4);
-                    o.pix_stride = C / 4;
+                    o.out = (unsigned long long)(reinterpret_cast<T *>(L.out) + (((size_t)gC.b * L.H + y0) * L.W + x0) * C + c0);
+                    o.row_stride = L.W * (C / VPV);
+                    o.pix_stride = C / VPV;
                     o.ny = y1 - y0 + 1;
                     o.nx = x1 - x0 + 1;
                     *reinterpret_cast<TileOut *>(d->rows) = o;
@@ -413,11 +421,11 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
     // rows but, with its ~8-16 samples, every column of the tile: column ownership keeps all eight warps busy on every
     // stage row (row ownership, the first version of this kernel, had two of eight at work and was latency-bound).
     const int c = warp;                                     // tile column
-    float4 acc[TH][NV];
+    float4 acc[TH][NACC];
 #pragma unroll
     for (int k = 0; k < TH; ++k)
 #pragma unroll
-        for (int v = 0; v < NV; ++v) acc[k][v] = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int v = 0; v < NACC; ++v) acc[k][v] = make_float4(0.f, 0.f, 0.f, 0.f);
 
     for (unsigned s = 0, fpar = 0;; fpar ^= (++s == NST), s = s == NST ? 0u : s) {
         mbar_wait(full0 + 8 * s, fpar);
@@ -428,21 +436,28 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
             // ---- end of tile: write the column exactly once (zeros included), clear the accumulators
             const TileOut o = *reinterpret_cast<const TileOut *>(d->rows);
             const int CH = hdr.y;
-            const bool ok0 = FULL || lane * 4 < CH, ok1 = NV == 2 && (FULL || lane * 4 + 128 < CH);
+            const bool ok0 = FULL || lane * VPV < CH, ok1 = NV == 2 && (FULL || lane * 4 + 128 < CH);
             if (c < o.nx) {
-                float4 *__restrict__ op = reinterpret_cast<float4 *>(o.out) + (size_t)c * o.pix_stride + lane;
+                if constexpr (ESZ == 4) {
+                    float4 *__restrict__ op = reinterpret_cast<float4 *>(o.out) + (size_t)c * o.pix_stride + lane;
 #pragma unroll
-                for (int k = 0; k < TH; ++k) {
-                    if (k < o.ny) {
-                        if (ok0) __stcs(op + (size_t)k * o.row_stride, acc[k][0]);
-                        if (ok1) __stcs(op + (size_t)k * o.row_stride + 32, acc[k][1]);
+                    for (int k = 0; k < TH; ++k) {
+                        if (k < o.ny) {
+                            if (ok0) __stcs(op + (size_t)k * o.row_stride, acc[k][0]);
+                            if (ok1) __stcs(op + (size_t)k * o.row_stride + 32, acc[k][1]);
+                        }
                     }
+                } else {        // 8 channels per lane, rounded once: 16 bytes per pixel
+                    uint4 *__restrict__ op = reinterpret_cast<uint4 *>(o.out) + (size_t)c * o.pix_stride + lane;
+#pragma unroll
+                    for (int k = 0; k < TH; ++k)
+                        if (k < o.ny && ok0) __stcs(op + (size_t)k * o.row_stride, narrow8<T>(acc[k][0], acc[k][1]));
                 }
             }
 #pragma unroll
             for (int k = 0; k < TH; ++k)
 #pragma unroll
-                for (int v = 0; v < NV; ++v) acc[k][v] = make_float4(0.f, 0.f, 0.f, 0.f);
+                for (int v = 0; v < NACC; ++v) acc[k][v] = make_float4(0.f, 0.f, 0.f, 0.f);
             __syncwarp();
             if (lane == 0) mbar_arrive(empty0 + 8 * s);
             continue;
@@ -477,7 +492,11 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
                 for (int k = ns; k > 0; --k, rowp += chb, ++xe) {
                     const XEnt e = *xe;
                     float4 g0, g1;
-                    if (FULL) {
+                    if constexpr (ESZ != 4) {       // widen the lane's 8 staged channels
+                        uint4 raw = make_uint4(0u, 0u, 0u, 0u);
+                        if (FULL || ok0) raw = *reinterpret_cast<const uint4 *>(rowp);
+                        widen8<T>(raw, g0, g1);
+                    } else if (FULL) {
                         g0 = *reinterpret_cast<const float4 *>(rowp);
                         if (NV == 2) g1 = *reinterpret_cast<const float4 *>(rowp + 512);
                     } else {
@@ -540,10 +559,30 @@ crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restric
 }
 #undef SLN_TMA_ADD
 
-template <int STG_S, int NST>
+template <int NV, bool EXACT, bool FULL, int STG_S, int NST>
+__global__ void __launch_bounds__(THREADS, 2)
+crop_bwd_tma_kernel(const float *__restrict__ grads, const ListEntryA *__restrict__ entries, const int *__restrict__ st_off,
+                    const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
+                    BwdTileBases TB, int C, int ph, int pw, int n_work, int chunks, int *__restrict__ queue)
+{
+    crop_bwd_tma_body<float, NV, EXACT, FULL, STG_S, NST>(grads, entries, st_off, st_count, lv_table, TB, C, ph, pw, n_work, chunks,
+                                                          queue);
+}
+
+// T = __nv_bfloat16 / __half: 8 channels (one 16-byte vector) per consumer lane
+template <typename T, bool EXACT, bool FULL, int STG_S, int NST>
+__global__ void __launch_bounds__(THREADS, 2)
+crop_bwd_tma_b16_kernel(const T *__restrict__ grads, const ListEntryA *__restrict__ entries, const int *__restrict__ st_off,
+                        const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
+                        BwdTileBases TB, int C, int ph, int pw, int n_work, int chunks, int *__restrict__ queue)
+{
+    crop_bwd_tma_body<T, 1, EXACT, FULL, STG_S, NST>(grads, entries, st_off, st_count, lv_table, TB, C, ph, pw, n_work, chunks, queue);
+}
+
+template <int STG_S, int NST, int ESZ = 4>
 static size_t smem_bytes()
 {
-    return (size_t)NST * STG_S * CH_MAX * 4 + sizeof(StageDesc<STG_S>) * NST + sizeof(BwdLevel) * BWD_MAX_LEVELS +
+    return (size_t)NST * STG_S * CH_MAX * ESZ + sizeof(StageDesc<STG_S>) * NST + sizeof(BwdLevel) * BWD_MAX_LEVELS +
            sizeof(uint64_t) * 2 * NST + 128;
 }
 

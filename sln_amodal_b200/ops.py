@@ -111,6 +111,45 @@ def to_contiguous_nchw(x):
     return out
 
 
+# 2-byte element types the crop kernels run natively (SLN_DTYPE_* codes of the *_ex entry points).  The caller asks for
+# it (keep_dtype= / out_dtype=); the autograd functions do so inside an enabled CUDA autocast region only.
+LOWP_DTYPES = {torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}
+
+
+def _b16_transpose(x, to_nhwc):
+    """A 2-byte [B,C,H,W] tensor -> the same tensor, same dtype, in channels_last (to_nhwc) or NCHW-contiguous memory
+    (sln_nchw_to_nhwc_b16 / sln_nhwc_to_nchw_b16: the bits move, nothing is converted)."""
+    x = x.detach()
+    if to_nhwc and is_channels_last(x):
+        return x
+    if not to_nhwc and x.is_contiguous():
+        return x
+    src = x.contiguous() if to_nhwc else x
+    if not to_nhwc and not is_channels_last(src):
+        return src.contiguous()
+    B, Cc, H, W = x.shape
+    out = torch.empty((B, Cc, H, W), dtype=x.dtype, device=x.device,
+                      memory_format=torch.channels_last if to_nhwc else torch.contiguous_format)
+    if out.numel():
+        fn = lib().sln_nchw_to_nhwc_b16 if to_nhwc else lib().sln_nhwc_to_nchw_b16
+        with torch.cuda.device(x.device):
+            check(fn(ptr(src), ptr(out), B, Cc, H, W, stream_ptr()), "sln_nchw_to_nhwc_b16" if to_nhwc else "sln_nhwc_to_nchw_b16")
+        _lib.count_launches(1)
+    return out
+
+
+def _aligned16(t):
+    return t.data_ptr() % 16 == 0
+
+
+def _bwd_native_lowp(grads, out_dtype, Cc, ph, pw):
+    """True when the 2-byte backward runs natively (bulk-async kernel): grads already in out_dtype, C % 8 == 0, crops of
+    at most 32 per side, and channels_last grads 16-byte aligned (other layouts are transposed into a fresh buffer)."""
+    if grads.dtype != out_dtype or Cc % 8 or ph > 32 or pw > 32:
+        return False
+    return not is_channels_last(grads) or _aligned16(grads)
+
+
 # NCHW callers (the unmodified reference: cuDNN hands out NCHW tensors unless the model was converted) on the fast path:
 # the NHWC gather kernel is ~3x faster than the NCHW one at C = 256, and the same FPN map is cropped several times per
 # step (classifier 7x7, mask head 14x14 / 16x16, every level call of the reference's pyramid_roi_align).  So a wide NCHW
@@ -123,10 +162,12 @@ _nhwc_cache = {}          # key -> (weakref to the owning tensor, channels_last 
 _NHWC_CACHE_MAX = 16
 
 
-def _nhwc_cached(image):
+def _nhwc_cached(image, keep_dtype=False):
+    """keep_dtype: a 2-byte map is remembered in its own dtype (sln_nchw_to_nhwc_b16) instead of as an f32 copy."""
     import weakref
     owner = image._base if image._base is not None else image
-    key = (id(owner), owner._version, image.storage_offset(), tuple(image.shape), tuple(image.stride()), image.device.index)
+    key = (id(owner), owner._version, image.storage_offset(), tuple(image.shape), tuple(image.stride()), image.device.index,
+           bool(keep_dtype))
     hit = _nhwc_cache.get(key)
     if hit is not None and hit[0]() is owner:
         return hit[1]
@@ -134,7 +175,7 @@ def _nhwc_cached(image):
         del _nhwc_cache[k]
     while len(_nhwc_cache) >= _NHWC_CACHE_MAX:
         del _nhwc_cache[next(iter(_nhwc_cache))]
-    cl = to_channels_last(image)
+    cl = _b16_transpose(image, True) if keep_dtype else to_channels_last(image)
     _nhwc_cache[key] = (weakref.ref(owner), cl)
     return cl
 
@@ -142,13 +183,14 @@ def _nhwc_cached(image):
 # ---------------------------------------------------------------------------
 # crop_and_resize
 # ---------------------------------------------------------------------------
-def crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extrapolation_value=0.0):
+def crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extrapolation_value=0.0, keep_dtype=False):
     """crops[N,C,ph,pw] = crop_and_resize(image[B,C,H,W], boxes[N,4], box_ind[N]).
 
     channels_last images go through the NHWC gather kernel and give channels_last crops.  NCHW images with at least
     NHWC_CACHE_MIN_CHANNELS channels (a multiple of 4) do too, through a remembered channels_last copy (see above); narrow
     NCHW images (mask targets C = 1, image crops C = 3) take the NCHW kernel and give NCHW crops.  Values are identical
-    either way."""
+    either way.  Crops are f32 whatever the image dtype, unless keep_dtype is set and the image is bf16 / fp16: then the
+    crops come in the image's dtype, bit-identical to the f32 crops of image.float() rounded to it (_crop_forward_lowp)."""
     _require_cuda(image, "image")
     _require_cuda(boxes, "boxes")
     _require_cuda(box_ind, "box_ind")
@@ -160,6 +202,8 @@ def crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extr
     if box_ind.shape[0] != N:
         raise _lib.SlnError("box_ind and boxes disagree on N")
     B, Cc, H, W = image.shape
+    if keep_dtype and image.dtype in LOWP_DTYPES:
+        return _crop_forward_lowp(image, boxes, box_ind, crop_height, crop_width, extrapolation_value)
     nhwc = is_channels_last(image) and image.dtype == torch.float32
     if (not nhwc and image.dtype == torch.float32 and Cc >= NHWC_CACHE_MIN_CHANNELS and Cc % 4 == 0 and N and H * W > 1):
         image = _nhwc_cached(image)
@@ -183,6 +227,30 @@ def crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extr
     return out
 
 
+def _crop_forward_lowp(image, boxes, box_ind, crop_height, crop_width, extrapolation_value):
+    """bf16 / fp16 image -> crops of its dtype.  channels_last images and wide NCHW ones (through a remembered 2-byte
+    channels_last copy) take the 2-byte NHWC gather kernel; narrow NCHW images take the f32 NCHW kernel on the widened
+    image and are rounded once, which gives the same bits."""
+    B, Cc, H, W = image.shape
+    N = boxes.shape[0]
+    img = None
+    if is_channels_last(image):
+        img = image.detach()
+    elif Cc >= NHWC_CACHE_MIN_CHANNELS and Cc % 4 == 0 and N and H * W > 1:
+        img = _nhwc_cached(image, keep_dtype=True)
+    out = torch.empty((N, Cc, crop_height, crop_width), dtype=image.dtype, device=image.device,
+                      memory_format=torch.channels_last)
+    if img is None or (N and Cc and not is_channels_last(out)):
+        return crop_and_resize_forward(image, boxes, box_ind, crop_height, crop_width, extrapolation_value).to(image.dtype)
+    with torch.cuda.device(image.device):
+        check(lib().sln_crop_and_resize_fwd_ex(LOWP_DTYPES[image.dtype], ptr(img), B, Cc, H, W, LAYOUT_NHWC, ptr(boxes),
+                                               ptr(box_ind), N, int(crop_height), int(crop_width), float(extrapolation_value),
+                                               ptr(out), stream_ptr()), "sln_crop_and_resize_fwd_ex")
+    if N and Cc:
+        _lib.count_launches(1)
+    return out
+
+
 def _prep_grads(grads):
     g = grads.detach()
     if g.dtype != torch.float32:
@@ -193,12 +261,15 @@ def _prep_grads(grads):
     return g, cl
 
 
-def crop_and_resize_backward(grads, boxes, box_ind, image_size, channels_last_out=None, exact=None):
+def crop_and_resize_backward(grads, boxes, box_ind, image_size, channels_last_out=None, exact=None, out_dtype=torch.float32):
     """grad_image[B,C,H,W] of crop_and_resize w.r.t. the image (deterministic gather kernel).
 
     channels_last_out: memory format of the returned gradient (default: follow `grads`).
     exact: True -> round every term like crop_and_resize.c (bit-identical to the reference CPU
-    backward); False -> fused multiply-add per term (default; see EXACT_BACKWARD)."""
+    backward); False -> fused multiply-add per term (default; see EXACT_BACKWARD).
+    out_dtype: f32 (default), or bf16 / fp16: the gradient in that dtype, bit-identical to the f32 gradient of
+    grads.float() rounded to it.  bf16 / fp16 grads of that dtype are read natively (C % 8 == 0, crops of at most 32
+    per side, 16-byte aligned); other shapes run the f32 kernels and round."""
     _require_cuda(grads, "grads")
     if exact is None:
         exact = EXACT_BACKWARD
@@ -210,19 +281,32 @@ def crop_and_resize_backward(grads, boxes, box_ind, image_size, channels_last_ou
     if Cg != Cc or boxes.shape[0] != N:
         raise _lib.SlnError("grads / boxes / image_size disagree")
     _check_rois(N, box_ind)
-    g, g_cl = _prep_grads(grads)
+    lowp = out_dtype in LOWP_DTYPES
+    if lowp and not _bwd_native_lowp(grads, out_dtype, Cc, ph, pw):
+        return crop_and_resize_backward(grads, boxes, box_ind, image_size, channels_last_out, exact).to(out_dtype)
+    if lowp:
+        g_cl = is_channels_last(grads)
+        g = _b16_transpose(grads, True)
+    else:
+        g, g_cl = _prep_grads(grads)
     if channels_last_out is None:
         channels_last_out = g_cl
-    out = torch.empty((B, Cc, H, W), dtype=torch.float32, device=grads.device, memory_format=torch.channels_last)
+    out = torch.empty((B, Cc, H, W), dtype=out_dtype if lowp else torch.float32, device=grads.device,
+                      memory_format=torch.channels_last)
     with torch.cuda.device(grads.device):
         ws = _workspace(lib().sln_crop_and_resize_bwd_workspace_bytes(N, B, ph, pw), grads.device)
-        check(lib().sln_crop_and_resize_bwd(ptr(g), ptr(boxes), ptr(box_ind), N, Cc, ph, pw, ptr(out), B, H, W,
-                                            LAYOUT_NHWC, flags, ptr(ws), ws.numel(), stream_ptr()),
-              "sln_crop_and_resize_bwd")
+        if lowp:
+            check(lib().sln_crop_and_resize_bwd_ex(LOWP_DTYPES[out_dtype], ptr(g), ptr(boxes), ptr(box_ind), N, Cc, ph, pw,
+                                                   ptr(out), B, H, W, LAYOUT_NHWC, flags, ptr(ws), ws.numel(), stream_ptr()),
+                  "sln_crop_and_resize_bwd_ex")
+        else:
+            check(lib().sln_crop_and_resize_bwd(ptr(g), ptr(boxes), ptr(box_ind), N, Cc, ph, pw, ptr(out), B, H, W,
+                                                LAYOUT_NHWC, flags, ptr(ws), ws.numel(), stream_ptr()),
+                  "sln_crop_and_resize_bwd")
     if out.numel():
         _lib.count_launches(4 if N else 1)
     if not channels_last_out:
-        out = to_contiguous_nchw(out)
+        out = _b16_transpose(out, False) if lowp else to_contiguous_nchw(out)
     return out
 
 
@@ -279,10 +363,12 @@ def pyramid_crop_backward_plan(boxes, box_ind, level, map_sizes, channels, crop_
     return BackwardPlan(ws, ev, key)
 
 
-def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last_out=None, exact=None, plan=None):
+def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last_out=None, exact=None, plan=None,
+                          out_dtype=torch.float32):
     """Backward of pyramid_crop_forward for all levels in one call.  map_sizes: list of (B,C,H_l,W_l).
     Returns the list of grad maps (channels_last unless channels_last_out[l] is False).
-    plan: a BackwardPlan from pyramid_crop_backward_plan for the same ROIs (ignored when it does not match)."""
+    plan: a BackwardPlan from pyramid_crop_backward_plan for the same ROIs (ignored when it does not match); a plan does
+    not depend on the dtype.  out_dtype: as in crop_and_resize_backward."""
     _require_cuda(grads, "grads")
     if exact is None:
         exact = EXACT_BACKWARD
@@ -297,8 +383,11 @@ def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last
     _check_rois(N, box_ind, level)
     nl = len(map_sizes)
     B = _check_map_sizes(map_sizes, Cc)
-    g, _ = _prep_grads(grads)
-    outs = [torch.empty(tuple(int(v) for v in sz), dtype=torch.float32, device=grads.device,
+    lowp = out_dtype in LOWP_DTYPES
+    if lowp and not _bwd_native_lowp(grads, out_dtype, Cc, ph, pw):
+        return [o.to(out_dtype) for o in pyramid_crop_backward(grads, *key_src, map_sizes, channels_last_out, exact, plan)]
+    g = _b16_transpose(grads, True) if lowp else _prep_grads(grads)[0]
+    outs = [torch.empty(tuple(int(v) for v in sz), dtype=out_dtype if lowp else torch.float32, device=grads.device,
                         memory_format=torch.channels_last) for sz in map_sizes]
     mp = (C.c_void_p * nl)(*[o.data_ptr() for o in outs])
     hs = (C.c_int * nl)(*[int(sz[2]) for sz in map_sizes])
@@ -311,18 +400,27 @@ def pyramid_crop_backward(grads, boxes, box_ind, level, map_sizes, channels_last
             flags |= _lib.BWD_PLANNED
         else:
             ws = _workspace(lib().sln_pyramid_crop_bwd_workspace_bytes(N, B, nl, ph, pw), grads.device)
-        check(lib().sln_pyramid_crop_bwd(ptr(g), ptr(boxes), ptr(box_ind), ptr(level), N, Cc, ph, pw, mp, hs, ws_, nl, B,
-                                         flags, ptr(ws), ws.numel(), stream_ptr()), "sln_pyramid_crop_bwd")
+        if lowp:
+            check(lib().sln_pyramid_crop_bwd_ex(LOWP_DTYPES[out_dtype], ptr(g), ptr(boxes), ptr(box_ind), ptr(level), N, Cc,
+                                                ph, pw, mp, hs, ws_, nl, B, flags, ptr(ws), ws.numel(), stream_ptr()),
+                  "sln_pyramid_crop_bwd_ex")
+        else:
+            check(lib().sln_pyramid_crop_bwd(ptr(g), ptr(boxes), ptr(box_ind), ptr(level), N, Cc, ph, pw, mp, hs, ws_, nl, B,
+                                             flags, ptr(ws), ws.numel(), stream_ptr()), "sln_pyramid_crop_bwd")
     _lib.count_launches((2 if planned else 4) if N else 1)
     if channels_last_out is not None:
-        outs = [o if cl else to_contiguous_nchw(o) for o, cl in zip(outs, channels_last_out)]
+        outs = [o if cl else (_b16_transpose(o, False) if lowp else to_contiguous_nchw(o))
+                for o, cl in zip(outs, channels_last_out)]
     return outs
 
 
-def pyramid_crop_forward(feature_maps, boxes, box_ind, level, crop_height, crop_width, extrapolation_value=0.0):
+def pyramid_crop_forward(feature_maps, boxes, box_ind, level, crop_height, crop_width, extrapolation_value=0.0,
+                         keep_dtype=False):
     """One launch for all FPN levels: feature_maps = list of channels_last [B,C,H_l,W_l] tensors,
     level[i] in [0, len(feature_maps)) names the source map of ROI i.  Output channels_last
-    [N,C,ph,pw] in the original ROI order.  Maps of another dtype are cropped from their f32 values."""
+    [N,C,ph,pw] in the original ROI order.  Maps of another dtype are cropped from their f32 values, into f32 crops --
+    unless keep_dtype is set and every map is bf16, or every map fp16: then the 2-byte kernel writes crops of that dtype,
+    bit-identical to the f32 crops rounded to it (NCHW maps are transposed once and remembered, in their dtype)."""
     for m in feature_maps:
         _require_cuda(m, "feature map")
         if m.dim() != 4:
@@ -336,24 +434,33 @@ def pyramid_crop_forward(feature_maps, boxes, box_ind, level, crop_height, crop_
     for m in feature_maps:
         if m.shape[0] != B or m.shape[1] != Cc:
             raise _lib.SlnError("feature maps disagree on batch / channels")
+    dt = feature_maps[0].dtype
+    lowp = keep_dtype and dt in LOWP_DTYPES and all(m.dtype == dt for m in feature_maps)
     maps = []
     for m in feature_maps:
-        if is_channels_last(m) and m.dtype == torch.float32:
+        if lowp:
+            maps.append(m.detach() if is_channels_last(m) else _nhwc_cached(m, keep_dtype=True))
+        elif is_channels_last(m) and m.dtype == torch.float32:
             maps.append(m.detach())
         elif m.dtype == torch.float32:
             maps.append(_nhwc_cached(m))                 # NCHW map: transposed once, remembered while the tensor lives
         else:
             maps.append(to_channels_last(m))
     nl = len(maps)
-    out = torch.empty((N, Cc, crop_height, crop_width), dtype=torch.float32, device=boxes.device,
+    out = torch.empty((N, Cc, crop_height, crop_width), dtype=dt if lowp else torch.float32, device=boxes.device,
                       memory_format=torch.channels_last)
     mp = (C.c_void_p * nl)(*[m.data_ptr() for m in maps])
     hs = (C.c_int * nl)(*[m.shape[2] for m in maps])
     ws_ = (C.c_int * nl)(*[m.shape[3] for m in maps])
     with torch.cuda.device(boxes.device):
-        check(lib().sln_pyramid_crop_fwd(mp, hs, ws_, nl, B, Cc, ptr(boxes), ptr(box_ind), ptr(level), N,
-                                         int(crop_height), int(crop_width), float(extrapolation_value), ptr(out),
-                                         stream_ptr()), "sln_pyramid_crop_fwd")
+        if lowp:
+            check(lib().sln_pyramid_crop_fwd_ex(LOWP_DTYPES[dt], mp, hs, ws_, nl, B, Cc, ptr(boxes), ptr(box_ind), ptr(level),
+                                                N, int(crop_height), int(crop_width), float(extrapolation_value), ptr(out),
+                                                stream_ptr()), "sln_pyramid_crop_fwd_ex")
+        else:
+            check(lib().sln_pyramid_crop_fwd(mp, hs, ws_, nl, B, Cc, ptr(boxes), ptr(box_ind), ptr(level), N,
+                                             int(crop_height), int(crop_width), float(extrapolation_value), ptr(out),
+                                             stream_ptr()), "sln_pyramid_crop_fwd")
     if N and Cc:
         _lib.count_launches(1)
     return out

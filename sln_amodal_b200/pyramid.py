@@ -10,7 +10,7 @@ from __future__ import annotations
 import torch
 
 from . import ops
-from .crop_and_resize import CropAndResizeFunction
+from .crop_and_resize import CropAndResizeFunction, keeps_dtype
 
 
 # Training: plan the backward (its three ROI-list launches) beside the forward kernel; False restores plan-in-backward.
@@ -43,17 +43,20 @@ class _PyramidCrop(torch.autograd.Function):
         ctx.cl = [ops.is_channels_last(m) for m in maps]
         ctx.needs = [m.requires_grad for m in maps]
         ctx.plan = None
+        lowp = keeps_dtype(*maps)
+        ctx.grad_dtype = maps[0].dtype if lowp else torch.float32
         if PLAN_BACKWARD_IN_FORWARD and any(ctx.needs) and boxes.shape[0] and not torch.cuda.is_current_stream_capturing():
             # the backward's ROI lists only depend on the boxes: build them on a side stream while the forward kernel runs
             ctx.plan = ops.pyramid_crop_backward_plan(boxes, box_ind, level, ctx.sizes, maps[0].shape[1], pool, pool)
-        out = ops.pyramid_crop_forward(list(maps), boxes, box_ind, level, pool, pool, 0.0)
+        out = ops.pyramid_crop_forward(list(maps), boxes, box_ind, level, pool, pool, 0.0, keep_dtype=lowp)
         ctx.save_for_backward(boxes, box_ind, level)
         return out
 
     @staticmethod
     def backward(ctx, grad):
         boxes, box_ind, level = ctx.saved_tensors
-        outs = ops.pyramid_crop_backward(grad, boxes, box_ind, level, ctx.sizes, channels_last_out=ctx.cl, plan=ctx.plan)
+        outs = ops.pyramid_crop_backward(grad, boxes, box_ind, level, ctx.sizes, channels_last_out=ctx.cl, plan=ctx.plan,
+                                         out_dtype=ctx.grad_dtype)
         grads = [o if need else None for o, need in zip(outs, ctx.needs)]
         return (None, None, None, None) + tuple(grads)
 
