@@ -91,7 +91,8 @@ SLN_API int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, int
  *                       non-NULL (nothing is read or written through them).
  *   SLN_BWD_PLANNED   : `workspace` holds the lists of a PLAN_ONLY call with the same boxes, box_ind, level, N, C, ph, pw,
  *                       B and map sizes (a plan can be used any number of times): the three prep launches are skipped.
- * Shapes that do not take the bulk-async kernel ignore PLAN_ONLY and treat PLANNED as a plain call.                  */
+ * The lists do not depend on the gradients' alignment, so this works for every shape: the PLANNED call picks the
+ * gather kernel from its own pointers.                                                                              */
 #define SLN_BWD_PLAN_ONLY 2
 #define SLN_BWD_PLANNED 4
 SLN_API size_t sln_crop_and_resize_bwd_workspace_bytes(int N, int B, int ph, int pw);
@@ -136,8 +137,9 @@ SLN_API int sln_roi_levels(const float *boxes, int N, int image_h, int image_w, 
  *             convert with sln_nchw_to_nhwc_b16, or widen and use the f32 NCHW kernel.
  *   backward: the bulk-async kernel only -- C % 8 == 0, ph and pw <= 32, grads and grad maps 16-byte aligned;
  *             SLN_ERR_LAYOUT otherwise (widen, run the f32 call and round: same bits).  SLN_BWD_PLAN_ONLY /
- *             SLN_BWD_PLANNED work as for f32, and a plan does not depend on the dtype: a PLAN_ONLY call of any
- *             dtype serves PLANNED calls of every dtype with the same boxes and sizes.                            */
+ *             SLN_BWD_PLANNED work as for f32, and a plan depends neither on the dtype nor on the shape's gather
+ *             kernel: a PLAN_ONLY call of any dtype serves PLANNED calls of every dtype with the same boxes and
+ *             sizes, including the f32 call of that widening fallback.                                            */
 SLN_API int sln_crop_and_resize_fwd_ex(int dtype, const void *image, int B, int C, int H, int W, int layout,
                                const float *boxes, const int *box_ind, int N, int ph, int pw,
                                float extrapolation_value, void *crops, void *stream);

@@ -258,19 +258,14 @@ struct BwdTileBases {  // passed by value to the main kernel: static-index compa
     int n_levels;
 };
 
-struct ListEntry {
-    RoiWin win;
-    int roi;
-};
-
 // Per-ROI sampling grid, evaluated once: pos(k) = base + k*scale on each axis, the same
 // expression (and rounding) as axis_tap / crop_and_resize.c:44-56.
 struct RoiAxes {
     float by, sy, bx, sx;
 };
 
-// list entry of the bulk-async kernel: the ROI's sampling grid rides along, so that the planner needs no second,
-// dependent load per ROI
+// supertile list entry: the ROI's sampling grid rides along, so that the gather kernels need no second, dependent load
+// per ROI
 struct __align__(16) ListEntryA {
     RoiWin win;
     int roi;
@@ -289,15 +284,8 @@ __device__ __forceinline__ void axis_base_scale(float a1, float a2, int extent, 
     }
 }
 
-__device__ __forceinline__ Tap ld_tap(const Tap *p)
-{
-    const int2 v = __ldg(reinterpret_cast<const int2 *>(p));
-    Tap t;
-    t.lo = v.x;
-    t.lerp = __int_as_float(v.y);
-    return t;
-}
-
+// tap k of an axis from its sampling grid (axis_base_scale): the same fp32 operations as axis_tap for crop > 1; for
+// crop == 1 the base plus 0 * k at k = 0, which is the base itself
 __device__ __forceinline__ Tap tap_at(float base, float scale, float em1, int k)
 {
     const float pos = __fadd_rn(base, __fmul_rn((float)k, scale));
@@ -327,8 +315,8 @@ __device__ __forceinline__ BwdLevel pick_level(const BwdParams &P, int l)
 // order-independent result); thread 0 also publishes the level table for the main kernel.
 __global__ void crop_bwd_windows_kernel(const float *__restrict__ boxes, const int *__restrict__ box_ind,
                                         const int *__restrict__ level, int N, int B, int ph, int pw,
-                                        BwdParams P, RoiWin *__restrict__ win, Tap *__restrict__ taps,
-                                        RoiAxes *__restrict__ axes, int *__restrict__ st_count,
+                                        BwdParams P, RoiWin *__restrict__ win, RoiAxes *__restrict__ axes,
+                                        int *__restrict__ st_count,
                                         BwdLevel *__restrict__ lv_table, int *__restrict__ queue, int queue_init,
                                         int *__restrict__ gid)
 {
@@ -342,21 +330,13 @@ __global__ void crop_bwd_windows_kernel(const float *__restrict__ boxes, const i
     int my_gid = -1;                                 // (image, level) group of the ROI; -1: contributes nothing
     const int b = box_ind[r];
     const int l = level ? level[r] : 0;
-    Tap *tp = taps + (size_t)r * (ph + pw);          // [ph] y taps then [pw] x taps of this ROI
     if (b >= 0 && b < B && l >= 0 && l < P.n_levels) {
         const BwdLevel L = pick_level(P, l);
         const float y1 = boxes[4 * r + 0], x1 = boxes[4 * r + 1], y2 = boxes[4 * r + 2], x2 = boxes[4 * r + 3];
-        const float sc_y = axis_scale(y1, y2, L.H, ph), sc_x = axis_scale(x1, x2, L.W, pw);
-        if (taps) {
-            for (int k = 0; k < ph; ++k) tp[k] = axis_tap(y1, y2, sc_y, L.H, ph, k);
-            for (int k = 0; k < pw; ++k) tp[ph + k] = axis_tap(x1, x2, sc_x, L.W, pw, k);
-        }
-        if (axes) {
-            RoiAxes a;
-            axis_base_scale(y1, y2, L.H, ph, a.by, a.sy);
-            axis_base_scale(x1, x2, L.W, pw, a.bx, a.sx);
-            axes[r] = a;
-        }
+        RoiAxes a;
+        axis_base_scale(y1, y2, L.H, ph, a.by, a.sy);
+        axis_base_scale(x1, x2, L.W, pw, a.bx, a.sx);
+        axes[r] = a;
         int a0, a1, c0, c1;
         axis_window(y1, y2, L.H, ph, a0, a1);
         axis_window(x1, x2, L.W, pw, c0, c1);
@@ -441,14 +421,11 @@ crop_bwd_group_kernel(const int *__restrict__ gid, int N, int *__restrict__ glis
 constexpr int FILL_THREADS = 1024;
 constexpr int FILL_PER_THREAD = 2;
 
-template <bool WITH_AXES>
 __global__ void __launch_bounds__(FILL_THREADS)
 crop_bwd_fill_kernel(const int *__restrict__ glist, const int *__restrict__ gcount,
                      const RoiWin *__restrict__ win, const RoiAxes *__restrict__ axes, int N, BwdParams P,
-                     const int *__restrict__ st_count, int *__restrict__ st_off, void *__restrict__ entries_raw)
+                     const int *__restrict__ st_count, int *__restrict__ st_off, ListEntryA *__restrict__ entries)
 {
-    ListEntry *__restrict__ entries = static_cast<ListEntry *>(entries_raw);
-    ListEntryA *__restrict__ entries_a = static_cast<ListEntryA *>(entries_raw);
     __shared__ int s_cnt[FILL_PER_THREAD][FILL_THREADS / 32];
     __shared__ int s_base;
     pdl_prologue();
@@ -522,19 +499,12 @@ crop_bwd_fill_kernel(const int *__restrict__ glist, const int *__restrict__ gcou
         for (int it = 0; it < FILL_PER_THREAD; ++it) {
             if ((masks[it] >> lane) & 1u) {
                 const int slot = base + s_cnt[it][warp] + __popc(masks[it] & ((1u << lane) - 1u));
-                if (WITH_AXES) {
-                    ListEntryA e;
-                    e.win = w[it];
-                    e.roi = roi[it];
-                    e.pad = 0;
-                    e.ax = axes[roi[it]];
-                    entries_a[slot] = e;
-                } else {
-                    ListEntry e;
-                    e.win = w[it];
-                    e.roi = roi[it];
-                    entries[slot] = e;
-                }
+                ListEntryA e;
+                e.win = w[it];
+                e.roi = roi[it];
+                e.pad = 0;
+                e.ax = axes[roi[it]];
+                entries[slot] = e;
             }
         }
         base += s_base;
@@ -574,18 +544,18 @@ __device__ __forceinline__ int fast_div(int t, int d, float rcp)
 //   warp  = one strip of 4 horizontally adjacent destination pixels of one image and level
 //   lanes = channel vectors (NV per lane), accumulators in registers
 // The warp walks its supertile's ROI list in original box order.  For every ROI whose window
-// meets the strip, lane k evaluates tap k of the y axis and of the x axis (same arithmetic
-// as the forward); ballots give the samples that touch the strip's row and columns; the
-// warp then visits those samples in (y, x) order and adds each tap's term to the pixel it
-// lands on.  Per destination pixel the summation order is (ROI, y, x, tap TL/TR/BL/BR) --
+// meets the strip, lane k evaluates tap k of the y axis and of the x axis from the entry's
+// sampling grid (tap_at: same arithmetic as the forward; the grid is read from the list at
+// each use, since holding it in registers spills); ballots give the samples that touch the
+// strip's row and columns; the warp then visits those samples in (y, x) order and adds each
+// tap's term to the pixel it lands on.  Per destination pixel the summation order is (ROI, y, x, tap TL/TR/BL/BR) --
 // the reference's serial order (crop_and_resize.c:190-250).
 // EXACT: each term is wx*(wy*g) with every operation rounded like crop_and_resize.c:241-247
 // (bit-identical to the reference CPU backward); otherwise fma(wy*wx, g, acc).
 // 4 resident CTAs per SM (<= 64 registers): measured best on B200 (A/B runs, profiles/README.md)
 template <int VEC, int NV, bool EXACT>
 __global__ void __launch_bounds__(BWD_THREADS, 4)
-crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ taps,
-                     const ListEntry *__restrict__ entries, const int *__restrict__ st_off,
+crop_bwd_nhwc_kernel(const float *__restrict__ grads, const ListEntryA *__restrict__ entries, const int *__restrict__ st_off,
                      const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
                      BwdTileBases TB, int C, int ph, int pw)
 {
@@ -606,6 +576,7 @@ crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
     const int py = ty_i * BWD_ROWS + warp;
     if (py >= H) return;
     const int tx0 = tx_i * TW, tx1 = min(tx0 + TW, W) - 1;
+    const float em1y = (float)(H - 1), em1x = (float)(W - 1);
     const int CV = C / VEC;
     const int cvbase = blockIdx.y * (32 * NV) + lane;
 
@@ -619,7 +590,7 @@ crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
 
     const int st = L.st_base + (b * L.sg.ny + (py >> L.sg_shift)) * L.sg.nx + (tx0 >> L.sg_shift);
     const int n_list = st_count[st];
-    const ListEntry *__restrict__ list = entries + (n_list ? st_off[st] : 0);
+    const ListEntryA *__restrict__ list = entries + (n_list ? st_off[st] : 0);
     const V *__restrict__ g = reinterpret_cast<const V *>(grads) + cvbase;
     const int S = ph * pw;
 
@@ -634,21 +605,21 @@ crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
         int my_roi = -1;
         bool take = false;
         if (li < n_list) {
-            const ListEntry e = list[li];
-            my_roi = e.roi;
-            take = !(e.win.y1 < py || e.win.y0 > py || e.win.x1 < tx0 || e.win.x0 > tx1);
+            const RoiWin w = list[li].win;
+            my_roi = list[li].roi;
+            take = !(w.y1 < py || w.y0 > py || w.x1 < tx0 || w.x0 > tx1);
         }
         unsigned todo = __ballot_sync(0xffffffffu, take);
         while (todo) {
             const int bit = __ffs(todo) - 1;
             todo &= todo - 1;
             const int r = __shfl_sync(0xffffffffu, my_roi, bit);
-            const Tap *__restrict__ tp = taps + (size_t)r * (ph + pw);   // precomputed by the prep kernel
+            const RoiAxes *__restrict__ ax = &list[base + bit].ax;
             const V *gr = g + (size_t)r * S * CV;
             for (int ky0 = 0; ky0 < ph; ky0 += 32) {
                 Tap ty;
                 ty.lo = INVALID_TAP; ty.lerp = 0.f;
-                if (ky0 + lane < ph) ty = ld_tap(tp + ky0 + lane);
+                if (ky0 + lane < ph) ty = tap_at(ax->by, ax->sy, em1y, ky0 + lane);
                 unsigned ym = __ballot_sync(0xffffffffu, ty.lo == py || (ty.lo + 1 == py && ty.lerp != 0.f));
                 while (ym) {
                     const int yb = __ffs(ym) - 1;
@@ -663,7 +634,7 @@ crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
                     for (int kx0 = 0; kx0 < pw; kx0 += 32) {
                         Tap tx;
                         tx.lo = INVALID_TAP; tx.lerp = 0.f;
-                        if (kx0 + lane < pw) tx = ld_tap(tp + ph + kx0 + lane);
+                        if (kx0 + lane < pw) tx = tap_at(ax->bx, ax->sx, em1x, kx0 + lane);
                         unsigned xm = __ballot_sync(0xffffffffu, tx.lo != INVALID_TAP && tx.lo <= tx1 &&
                                                                      tx.lo + (tx.lerp != 0.f) >= tx0);
                         while (xm) {
@@ -725,276 +696,6 @@ crop_bwd_nhwc_kernel(const float *__restrict__ grads, const Tap *__restrict__ ta
         if (tx0 + 1 <= tx1) __stcs(o + (size_t)CV + 32, p1b);
         if (tx0 + 2 <= tx1) __stcs(o + 2 * (size_t)CV + 32, p2b);
         if (tx0 + 3 <= tx1) __stcs(o + 3 * (size_t)CV + 32, p3b);
-    }
-}
-
-// ===========================================================================
-// backward, NHWC, tile-owner form (default)
-// ===========================================================================
-// warp  = one 4x4 pixel tile of one image and level (BWD_TILE_WARPS independent warps per CTA, no barriers)
-// lanes = channel vectors (NV per lane); the tile's accumulators live in the warp's slice of shared memory
-//         ([16 pixels][32*NV vectors]: consecutive lanes = consecutive vectors, conflict-free)
-// The warp walks its supertile's ROI list in original box order; for every ROI whose window meets the tile it
-// takes the ROI's tap tables (lane k = tap k of each axis), ballots the sample rows / columns that touch the tile,
-// and visits those samples in (y, x) order.  One visit = one coalesced load of the sample's gradient vector (all
-// loads of a sample row are issued before the first use) + up to four read-modify-writes of the warp's own shared
-// memory, in the reference's tap order TL, TR, BL, BR.  Per destination pixel the summation order is therefore
-// (ROI, y, x, tap) -- the reference's serial order (crop_and_resize.c:190-250) -- without atomics; every pixel is
-// written exactly once at the end (zeros included: no memset).
-// Versus the strip form above: the search "which samples touch me" is paid once per (ROI, 16 pixels) instead of
-// once per (ROI, 4 pixels), and a visit carries no per-pixel switch -- 2.5x fewer warp instructions per byte.
-constexpr int BWD_TILE = 4;                 // tile side in pixels
-#ifndef SLN_BWD_TILE_WARPS
-#define SLN_BWD_TILE_WARPS 2
-#endif
-#ifndef SLN_BWD_BATCH
-#define SLN_BWD_BATCH 8
-#endif
-constexpr int BWD_TILE_WARPS = SLN_BWD_TILE_WARPS;   // warps (tiles) per CTA: tiles side by side along x
-constexpr int BWD_BATCH = SLN_BWD_BATCH;             // samples whose gradient loads are issued together
-
-// one sample's contribution to the warp's tile (see the kernel comment)
-template <int VEC, int NV, bool EXACT>
-__device__ __forceinline__ void bwd_tile_visit(typename VecT<VEC>::type *acc, const typename VecT<VEC>::type (&gv)[NV],
-                                               int ylo, float yl, int xlo, float xl, int y0, int y1, int x0, int x1)
-{
-    using V = typename VecT<VEC>::type;
-    constexpr int T = BWD_TILE, ROWV = 32 * NV;
-    const int yhi = ylo + (yl != 0.f), xhi = xlo + (xl != 0.f);
-    const float wt = __fsub_rn(1.f, yl), wb = yl, wl = __fsub_rn(1.f, xl), wr = xl;
-    const bool top_in = ylo >= y0 && ylo <= y1, bot_in = yhi >= y0 && yhi <= y1;
-    const bool l_in = xlo >= x0 && xlo <= x1, r_in = xhi >= x0 && xhi <= x1;
-    const int rt = (ylo - y0) * T, rb = (yhi - y0) * T, cl = xlo - x0, cr = xhi - x0;
-    if (EXACT) {
-        // reference order TL, TR, BL, BR, one read-modify-write after the other: taps coincide when the sample
-        // position is integral on an axis, and the reference still adds their "0 * g" terms
-#define SLN_TAP(IN, POFF, WY, WX)                                                                  \
-    if (IN) {                                                                                     \
-        _Pragma("unroll") for (int j = 0; j < NV; ++j) {                                          \
-            V a_ = acc[(POFF) * ROWV + 32 * j];                                                   \
-            a_ = accum<true>(a_, gv[j], (WY), (WX), 0.f);                                          \
-            acc[(POFF) * ROWV + 32 * j] = a_;                                                     \
-        }                                                                                         \
-    }
-        SLN_TAP(top_in && l_in, rt + cl, wt, wl)
-        SLN_TAP(top_in && r_in, rt + cr, wt, wr)
-        SLN_TAP(bot_in && l_in, rb + cl, wb, wl)
-        SLN_TAP(bot_in && r_in, rb + cr, wb, wr)
-#undef SLN_TAP
-    } else {
-        // zero-weight taps are skipped, so the (up to) four destinations are distinct pixels: all loads, then all
-        // fused multiply-adds, then all stores.  A tap that is not ours reads pixel 0 of the tile (any valid address)
-        // and is simply not stored: no selects, no register zeroing.
-        const bool t0 = top_in && l_in, t1 = top_in && r_in && wr != 0.f;
-        const bool t2 = bot_in && l_in && wb != 0.f, t3 = bot_in && r_in && wb != 0.f && wr != 0.f;
-        const float w0 = __fmul_rn(wt, wl), w1 = __fmul_rn(wt, wr), w2 = __fmul_rn(wb, wl), w3 = __fmul_rn(wb, wr);
-        V *q0 = acc + (t0 ? (rt + cl) * ROWV : 0), *q1 = acc + (t1 ? (rt + cr) * ROWV : 0);
-        V *q2 = acc + (t2 ? (rb + cl) * ROWV : 0), *q3 = acc + (t3 ? (rb + cr) * ROWV : 0);
-        V a0[NV], a1[NV], a2[NV], a3[NV];
-#pragma unroll
-        for (int j = 0; j < NV; ++j) {
-            a0[j] = q0[32 * j]; a1[j] = q1[32 * j]; a2[j] = q2[32 * j]; a3[j] = q3[32 * j];
-        }
-#pragma unroll
-        for (int j = 0; j < NV; ++j) {
-            a0[j] = accum<false>(a0[j], gv[j], 0.f, 0.f, w0);
-            a1[j] = accum<false>(a1[j], gv[j], 0.f, 0.f, w1);
-            a2[j] = accum<false>(a2[j], gv[j], 0.f, 0.f, w2);
-            a3[j] = accum<false>(a3[j], gv[j], 0.f, 0.f, w3);
-        }
-#pragma unroll
-        for (int j = 0; j < NV; ++j) {
-            if (t0) q0[32 * j] = a0[j];
-            if (t1) q1[32 * j] = a1[j];
-            if (t2) q2[32 * j] = a2[j];
-            if (t3) q3[32 * j] = a3[j];
-        }
-    }
-}
-
-template <int VEC, int NV, bool EXACT, bool FULL>
-__global__ void __launch_bounds__(32 * BWD_TILE_WARPS)
-crop_bwd_tile_kernel(const float *__restrict__ grads, const Tap *__restrict__ taps,
-                     const ListEntry *__restrict__ entries, const int *__restrict__ st_off,
-                     const int *__restrict__ st_count, const BwdLevel *__restrict__ lv_table,
-                     BwdTileBases TB, int C, int ph, int pw)
-{
-    using V = typename VecT<VEC>::type;
-    extern __shared__ __align__(16) unsigned char s_bwd_raw[];
-    constexpr int T = BWD_TILE, NPX = T * T, ROWV = 32 * NV;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    V *acc = reinterpret_cast<V *>(s_bwd_raw) + (size_t)warp * NPX * ROWV + lane;   // acc[p * ROWV + 32 * j]
-
-    int l = TB.lvl[0];
-#pragma unroll
-    for (int k = 1; k < BWD_MAX_LEVELS; ++k)
-        if (k < TB.n_levels && (int)blockIdx.x >= TB.base[k]) l = TB.lvl[k];
-    const BwdLevel L = lv_table[l];
-    const int t = blockIdx.x - L.tile_base;
-    const int q1 = fast_div(t, L.tiles_x, L.rcp_tiles_x);
-    const int tx_i = t - q1 * L.tiles_x;
-    const int b = fast_div(q1, L.tiles_y, L.rcp_tiles_y);
-    const int ty_i = q1 - b * L.tiles_y;
-    const int H = L.H, W = L.W;
-    const int y0 = ty_i * T, x0 = (tx_i * BWD_TILE_WARPS + warp) * T;
-    if (y0 >= H || x0 >= W) return;            // no barriers in this kernel
-    const int y1 = min(y0 + T, H) - 1, x1 = min(x0 + T, W) - 1;
-    const int CV = C / VEC;
-    const int cvbase = blockIdx.y * ROWV + lane;
-    bool ok[NV];                               // FULL: every lane's vectors exist (CV is a multiple of 32 * NV)
-#pragma unroll
-    for (int j = 0; j < NV; ++j) ok[j] = FULL || cvbase + 32 * j < CV;
-
-    const V zero = make_splat(0.f, (V *)nullptr);
-    bool touched = false;                      // warp-uniform: accumulators initialised and in use
-
-    const int st = L.st_base + (b * L.sg.ny + (y0 >> L.sg_shift)) * L.sg.nx + (x0 >> L.sg_shift);
-    const int n_list = st_count[st];
-    const ListEntry *__restrict__ list = entries + (n_list ? st_off[st] : 0);
-    const V *__restrict__ g = reinterpret_cast<const V *>(grads) + cvbase;
-    const int S = ph * pw;
-    const bool small = ph <= 32 && pw <= 32;   // one tap per lane and axis: the pipelined path
-
-    for (int base = 0; base < n_list; base += 32) {
-        const int li = base + lane;
-        int my_roi = -1;
-        bool take = false;
-        if (li < n_list) {
-            const ListEntry e = list[li];
-            my_roi = e.roi;
-            take = !(e.win.y1 < y0 || e.win.y0 > y1 || e.win.x1 < x0 || e.win.x0 > x1);
-        }
-        unsigned todo = __ballot_sync(0xffffffffu, take);
-        if (!todo) continue;
-        if (small) {
-            // ---- taps of the next ROI are in flight while the current one is accumulated
-            Tap ty_n, tx_n;
-            auto fetch_taps = [&](int r) {
-                const Tap *__restrict__ tp = taps + (size_t)r * (ph + pw);
-                ty_n.lo = INVALID_TAP; ty_n.lerp = 0.f; tx_n.lo = INVALID_TAP; tx_n.lerp = 0.f;
-                if (lane < ph) ty_n = ld_tap(tp + lane);
-                if (lane < pw) tx_n = ld_tap(tp + ph + lane);
-            };
-            int r_n = __shfl_sync(0xffffffffu, my_roi, __ffs(todo) - 1);
-            todo &= todo - 1;
-            fetch_taps(r_n);
-            while (r_n >= 0) {
-                const int r = r_n;
-                const Tap ty = ty_n, tx = tx_n;
-                r_n = -1;
-                if (todo) {
-                    r_n = __shfl_sync(0xffffffffu, my_roi, __ffs(todo) - 1);
-                    todo &= todo - 1;
-                    fetch_taps(r_n);
-                }
-                const unsigned ym = __ballot_sync(0xffffffffu, ty.lo != INVALID_TAP && ty.lo <= y1 && ty.lo + (ty.lerp != 0.f) >= y0);
-                const unsigned xm = __ballot_sync(0xffffffffu, tx.lo != INVALID_TAP && tx.lo <= x1 && tx.lo + (tx.lerp != 0.f) >= x0);
-                if (!ym || !xm) continue;
-                if (!touched) {                // first contribution: clear the accumulators
-#pragma unroll
-                    for (int p = 0; p < NPX; ++p)
-#pragma unroll
-                        for (int j = 0; j < NV; ++j) acc[p * ROWV + 32 * j] = zero;
-                    touched = true;
-                }
-                const V *gr = g + (size_t)r * S * CV;
-                // samples in (y, x) order, BWD_BATCH at a time: every gradient load of a batch is issued before
-                // the first accumulation
-                unsigned yrem = ym, xrem = xm;
-                while (yrem) {
-                    int sb[BWD_BATCH];         // yb << 8 | xb, -1: none
-                    V gv[BWD_BATCH][NV];
-#pragma unroll
-                    for (int u = 0; u < BWD_BATCH; ++u) {
-                        sb[u] = -1;
-                        if (yrem) {
-                            const int yb = __ffs(yrem) - 1, xb = __ffs(xrem) - 1;
-                            sb[u] = (yb << 8) | xb;
-                            xrem &= xrem - 1;
-                            if (!xrem) { yrem &= yrem - 1; xrem = xm; }
-#pragma unroll
-                            for (int j = 0; j < NV; ++j) {
-                                if (!FULL) gv[u][j] = zero;
-                                if (ok[j]) gv[u][j] = ldg_vec(gr + (size_t)(yb * pw + xb) * CV + 32 * j);
-                            }
-                        }
-                    }
-#pragma unroll
-                    for (int u = 0; u < BWD_BATCH; ++u) {
-                        if (sb[u] < 0) break;  // warp-uniform
-                        const int yb = sb[u] >> 8, xb = sb[u] & 0xff;
-                        const int ylo = __shfl_sync(0xffffffffu, ty.lo, yb), xlo = __shfl_sync(0xffffffffu, tx.lo, xb);
-                        const float yl = __shfl_sync(0xffffffffu, ty.lerp, yb), xl = __shfl_sync(0xffffffffu, tx.lerp, xb);
-                        bwd_tile_visit<VEC, NV, EXACT>(acc, gv[u], ylo, yl, xlo, xl, y0, y1, x0, x1);
-                    }
-                }
-            }
-        } else {
-            // ---- crops larger than 32 samples per side: tap tables in chunks of 32, one sample at a time
-            while (todo) {
-                const int bit = __ffs(todo) - 1;
-                todo &= todo - 1;
-                const int r = __shfl_sync(0xffffffffu, my_roi, bit);
-                const Tap *__restrict__ tp = taps + (size_t)r * (ph + pw);
-                const V *gr = g + (size_t)r * S * CV;
-                for (int ky0 = 0; ky0 < ph; ky0 += 32) {
-                    Tap ty;
-                    ty.lo = INVALID_TAP; ty.lerp = 0.f;
-                    if (ky0 + lane < ph) ty = ld_tap(tp + ky0 + lane);
-                    unsigned ym = __ballot_sync(0xffffffffu, ty.lo != INVALID_TAP && ty.lo <= y1 && ty.lo + (ty.lerp != 0.f) >= y0);
-                    while (ym) {
-                        const int yb = __ffs(ym) - 1;
-                        ym &= ym - 1;
-                        const int ylo = __shfl_sync(0xffffffffu, ty.lo, yb);
-                        const float yl = __shfl_sync(0xffffffffu, ty.lerp, yb);
-                        for (int kx0 = 0; kx0 < pw; kx0 += 32) {
-                            Tap tx;
-                            tx.lo = INVALID_TAP; tx.lerp = 0.f;
-                            if (kx0 + lane < pw) tx = ld_tap(tp + ph + kx0 + lane);
-                            unsigned xm = __ballot_sync(0xffffffffu, tx.lo != INVALID_TAP && tx.lo <= x1 && tx.lo + (tx.lerp != 0.f) >= x0);
-                            if (xm && !touched) {
-#pragma unroll
-                                for (int p = 0; p < NPX; ++p)
-#pragma unroll
-                                    for (int j = 0; j < NV; ++j) acc[p * ROWV + 32 * j] = zero;
-                                touched = true;
-                            }
-                            while (xm) {
-                                const int xb = __ffs(xm) - 1;
-                                xm &= xm - 1;
-                                const int xlo = __shfl_sync(0xffffffffu, tx.lo, xb);
-                                const float xl = __shfl_sync(0xffffffffu, tx.lerp, xb);
-                                V gv[NV];
-#pragma unroll
-                                for (int j = 0; j < NV; ++j) {
-                                    gv[j] = zero;
-                                    if (ok[j]) gv[j] = ldg_vec(gr + (size_t)((ky0 + yb) * pw + kx0 + xb) * CV + 32 * j);
-                                }
-                                bwd_tile_visit<VEC, NV, EXACT>(acc, gv, ylo, yl, xlo, xl, y0, y1, x0, x1);
-                            }
-                        }
-                    }
-                }
-            }
-        }
-    }
-
-    // ---- write every pixel of the tile exactly once (zeros included)
-    V *__restrict__ o = reinterpret_cast<V *>(L.out) + (((size_t)b * H + y0) * W + x0) * CV + cvbase;
-#pragma unroll
-    for (int py = 0; py < T; ++py) {
-        if (y0 + py > y1) break;
-#pragma unroll
-        for (int px = 0; px < T; ++px) {
-            if (x0 + px > x1) break;
-#pragma unroll
-            for (int j = 0; j < NV; ++j) {
-                if (!ok[j]) continue;
-                V v = zero;
-                if (touched) v = acc[(py * T + px) * ROWV + 32 * j];
-                __stcs(o + ((size_t)py * W + px) * CV + 32 * j, v);
-            }
-        }
     }
 }
 
@@ -1187,7 +888,6 @@ static int crop_fwd_nhwc_dt(int dtype, const PyramidMaps &pm, int n_levels, bool
 struct BwdWs {
     RoiWin *win;
     RoiAxes *axes;
-    Tap *taps;
     int *st_count;
     int *st_off;
     BwdLevel *lv_table;
@@ -1195,47 +895,28 @@ struct BwdWs {
     int *gid;       // [N] (image, level) group of every ROI
     int *gcount;    // [B * n_levels]
     int *glist;     // [B * n_levels][N] ROI ids per group, in index order
-    ListEntry *entries;
+    ListEntryA *entries;
 };
 
 constexpr int BWD_MAX_ST = 64;        // supertiles per image and level (8 x 8)
 
-static size_t bwd_ws_bytes(int N, int B, int n_levels, int ph, int pw)
+static size_t bwd_ws_bytes(int N, int B, int n_levels)
 {
     // every ROI lives on one level and meets at most 64 supertiles of its image
     const size_t n_st = (size_t)B * BWD_MAX_ST * (size_t)n_levels + 1;
     return align_up(sizeof(RoiWin) * (size_t)N, 256) + align_up(sizeof(RoiAxes) * (size_t)N, 256) +
-           align_up(sizeof(Tap) * (size_t)N * (size_t)(ph + pw), 256) +
            2 * align_up(sizeof(int) * n_st, 256) + align_up(sizeof(BwdLevel) * BWD_MAX_LEVELS, 256) + 256 +
            align_up(sizeof(int) * (size_t)N, 256) + align_up(sizeof(int) * (size_t)B * n_levels, 256) +
            align_up(sizeof(int) * (size_t)B * n_levels * (size_t)N, 256) +
            align_up(sizeof(ListEntryA) * (size_t)N * BWD_MAX_ST, 256);
 }
 
-// Which gather kernel serves a call (A/B on B200, 8 x 1000 ROIs, C = 256, all four levels, ms per call incl. prep):
-//   7x7    strip 0.382   tile 0.352        14x14   strip 0.793   tile 0.874
-// A tile visit pays shared-memory read-modify-writes the strip form keeps in registers, which costs more than the
-// cheaper search saves once a tile sees ~9+ samples of a ROI (14x14 crops), so: tile form for crops of at most
-// BWD_TILE_MAX_SAMPLES samples, strip form above.  SLN_BWD_IMPL forces one of them (0 strip, 1 tile) for A/B runs.
-// Since round 2 both are the fallback for shapes the bulk-async kernel (crop_bwd_tma.cuh) does not take: channel counts
-// that are not a multiple of 4, unaligned pointers, crops larger than 32 samples per side.  SLN_BWD_IMPL in the
-// environment forces one form for A/B runs: 0 strip, 1 tile, 2 strip / tile by crop size, 3 (default) bulk-async.
-constexpr int BWD_TILE_MAX_SAMPLES = 64;
-static int bwd_impl_env()
-{
-    const char *e = getenv("SLN_BWD_IMPL");
-    return (e && e[0] >= '0' && e[0] <= '3') ? e[0] - '0' : 3;
-}
+// Which gather kernel serves an fp32 call: the bulk-async kernel (crop_bwd_tma.cuh) when C % 4 == 0, grads and grad maps
+// are 16-byte aligned and the crop is at most 32 samples per side; the strip form (crop_bwd_nhwc_kernel) for every other
+// shape.  DESIGN.md section 4.3 has the timings of both.
 static bool bwd_use_tma(int ph, int pw, bool vec4)
 {
-    return bwd_impl_env() == 3 && vec4 && ph <= bwdtma::MAX_POOL && pw <= bwdtma::MAX_POOL;
-}
-static bool bwd_use_tile(int ph, int pw)
-{
-    const int impl = bwd_impl_env();
-    if (impl == 0) return false;
-    if (impl == 1) return true;
-    return ph * pw <= BWD_TILE_MAX_SAMPLES;
+    return vec4 && ph <= bwdtma::MAX_POOL && pw <= bwdtma::MAX_POOL;
 }
 
 // persistent grid of the bulk-async kernel: two CTAs per SM; CTA i starts with work item i and then draws tickets
@@ -1270,7 +951,7 @@ static int launch_bwd_tma_cfg(const T *grads, const BwdWs &ws, const BwdTileBase
     // programmatic dependent of the prep chain: its CTAs are placed and set their barriers up while the fill kernel's last
     // wave drains, and block (griddepcontrol.wait in the kernel) before they read anything the prep wrote
     SLN_CUDA_OK(launch_chain(kern, dim3(grid), dim3(bwdtma::THREADS), smem, st, true, grads,
-                             reinterpret_cast<const ListEntryA *>(ws.entries), (const int *)ws.st_off, (const int *)ws.st_count,
+                             (const ListEntryA *)ws.entries, (const int *)ws.st_off, (const int *)ws.st_count,
                              (const BwdLevel *)ws.lv_table, TB, C, ph, pw, (int)n_work, chunks, ws.queue));
     SLN_LAUNCH_OK("crop_bwd_tma_kernel");
     return SLN_OK;
@@ -1319,26 +1000,6 @@ static int launch_bwd_tma_dt(int dtype, const void *grads, bool exact, const Bwd
 }
 
 template <int VEC, int NV, bool EXACT>
-static int launch_bwd_tile(const float *grads, const BwdWs &ws, const BwdParams &P, long long tiles, int C, int ph, int pw,
-                           cudaStream_t st)
-{
-    const int chunks = cdiv(C / VEC, 32 * NV);
-    SLN_REQUIRE(chunks <= 65535, SLN_ERR_ARG, "too many channel chunks");
-    if (tiles == 0) return SLN_OK;
-    BwdTileBases TB{};
-    TB.n_levels = P.n_levels;
-    for (int j = 0; j < P.n_levels; ++j) { TB.base[j] = P.sched_base[j]; TB.lvl[j] = P.sched_lvl[j]; }
-    dim3 grid((unsigned)tiles, chunks);
-    const size_t smem = (size_t)BWD_TILE_WARPS * BWD_TILE * BWD_TILE * 32 * NV * sizeof(float) * VEC;
-    auto kern = (C / VEC) % (32 * NV) == 0 ? crop_bwd_tile_kernel<VEC, NV, EXACT, true> : crop_bwd_tile_kernel<VEC, NV, EXACT, false>;
-    SLN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    SLN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    kern<<<grid, 32 * BWD_TILE_WARPS, smem, st>>>(grads, ws.taps, ws.entries, ws.st_off, ws.st_count, ws.lv_table, TB, C, ph, pw);
-    SLN_LAUNCH_OK("crop_bwd_tile_kernel");
-    return SLN_OK;
-}
-
-template <int VEC, int NV, bool EXACT>
 static int launch_bwd(const float *grads, const BwdWs &ws, const BwdParams &P, long long tiles, int C, int ph, int pw,
                       cudaStream_t st)
 {
@@ -1349,8 +1010,8 @@ static int launch_bwd(const float *grads, const BwdWs &ws, const BwdParams &P, l
     TB.n_levels = P.n_levels;
     for (int j = 0; j < P.n_levels; ++j) { TB.base[j] = P.sched_base[j]; TB.lvl[j] = P.sched_lvl[j]; }
     dim3 grid((unsigned)tiles, chunks);
-    crop_bwd_nhwc_kernel<VEC, NV, EXACT><<<grid, BWD_THREADS, 0, st>>>(grads, ws.taps, ws.entries, ws.st_off,
-                                                                      ws.st_count, ws.lv_table, TB, C, ph, pw);
+    crop_bwd_nhwc_kernel<VEC, NV, EXACT><<<grid, BWD_THREADS, 0, st>>>(grads, ws.entries, ws.st_off, ws.st_count, ws.lv_table,
+                                                                      TB, C, ph, pw);
     SLN_LAUNCH_OK("crop_bwd_nhwc_kernel");
     return SLN_OK;
 }
@@ -1360,10 +1021,6 @@ static int dispatch_bwd(const float *grads, const BwdWs &ws, const BwdParams &P,
                         cudaStream_t st)
 {
     const int CV = C / VEC;
-    if (bwd_use_tile(ph, pw)) {
-        if (CV > 32) return launch_bwd_tile<VEC, 2, EXACT>(grads, ws, P, tiles, C, ph, pw, st);
-        return launch_bwd_tile<VEC, 1, EXACT>(grads, ws, P, tiles, C, ph, pw, st);
-    }
     // two channel vectors per lane halve the control work per byte, but also the CTA count:
     // only use them when the maps provide enough strips to fill the machine
     if (CV > 32 && tiles >= 6LL * sm_count()) return launch_bwd<VEC, 2, EXACT>(grads, ws, P, tiles, C, ph, pw, st);
@@ -1373,8 +1030,9 @@ static int dispatch_bwd(const float *grads, const BwdWs &ws, const BwdParams &P,
 // grads [N,ph,pw,C]; one grad map per level (NHWC); level[i] selects the map of ROI i (null: level 0)
 // mode 0: plan + run; 1 (SLN_BWD_PLAN_ONLY): build the lists only (grads / maps are not touched; maps[l] only need to be
 // plausible addresses); 2 (SLN_BWD_PLANNED): the workspace holds the lists of a mode-1 call with the same boxes, box_ind,
-// level, N, C, ph, pw, B and map sizes -- skip the three prep launches.  Only the bulk-async form plans ahead; the other
-// forms ignore mode 1 and treat mode 2 as mode 0.
+// level, N, C, ph, pw, B and map sizes -- skip the three prep launches and only republish the level table (grad map
+// addresses and the tile geometry of the gather kernel that runs) and the ticket counter.  The lists do not depend on
+// which gather kernel runs, so every shape plans ahead the same way.
 // dtype: element type of grads and maps (SLN_DTYPE_*).  2-byte types run the bulk-async kernel only (C % 8 == 0, crops
 // of at most 32 per side, 16-byte aligned pointers); other shapes are refused.  A plan does not depend on the dtype: the
 // prep kernels see boxes and sizes only, and the tile grid (8 x 8) and channel chunks (256) are the same for every type.
@@ -1384,28 +1042,20 @@ static int crop_bwd_nhwc(int dtype, const void *grads, const float *boxes, const
 {
     SLN_REQUIRE(dtype == SLN_DTYPE_F32 || dtype == SLN_DTYPE_BF16 || dtype == SLN_DTYPE_F16, SLN_ERR_ARG, "unknown dtype %d", dtype);
     if (B == 0 || C == 0) return SLN_OK;
-    SLN_REQUIRE(ws_bytes >= bwd_ws_bytes(N, B, n_levels, ph, pw), SLN_ERR_WORKSPACE,
-                "crop bwd workspace: need %zu bytes, got %zu", bwd_ws_bytes(N, B, n_levels, ph, pw), ws_bytes);
+    SLN_REQUIRE(ws_bytes >= bwd_ws_bytes(N, B, n_levels), SLN_ERR_WORKSPACE,
+                "crop bwd workspace: need %zu bytes, got %zu", bwd_ws_bytes(N, B, n_levels), ws_bytes);
     SLN_REQUIRE(wsp != nullptr, SLN_ERR_WORKSPACE, "null workspace");
     BwdParams P{};
     P.n_levels = n_levels;
     int n_st = 0;
     long long tiles = 0;
-    bool vec4 = (C % 4 == 0) && (mode == 1 || aligned16(grads));
-    for (int l = 0; l < n_levels; ++l) vec4 = vec4 && (mode == 1 || aligned16(maps[l]));
-    bool use_tma = bwd_use_tma(ph, pw, vec4);
-    if (dtype != SLN_DTYPE_F32 && mode != 1) {
-        bool ok = C % 8 == 0 && ph <= bwdtma::MAX_POOL && pw <= bwdtma::MAX_POOL && aligned16(grads);
-        for (int l = 0; l < n_levels; ++l) ok = ok && aligned16(maps[l]);
-        SLN_REQUIRE(ok, SLN_ERR_LAYOUT, "2-byte crop backward needs C %% 8 == 0 (C = %d), crops of at most 32 per side "
-                    "(%dx%d) and 16-byte aligned grads and grad maps", C, ph, pw);
-        if (mode == 2 && !use_tma) mode = 0;    // SLN_BWD_IMPL chose another form for fp32: no plan was built
-        use_tma = true;
-    }
-    if (!use_tma) {
-        if (mode == 1) return SLN_OK;
-        mode = 0;
-    }
+    bool vec4 = C % 4 == 0 && aligned16(grads);
+    for (int l = 0; l < n_levels; ++l) vec4 = vec4 && aligned16(maps[l]);
+    const bool use_tma = bwd_use_tma(ph, pw, vec4);
+    // 2-byte shapes that pass this check are bulk-async shapes (C % 8 == 0 implies C % 4 == 0)
+    SLN_REQUIRE(dtype == SLN_DTYPE_F32 || mode == 1 || (C % 8 == 0 && use_tma), SLN_ERR_LAYOUT,
+                "2-byte crop backward needs C %% 8 == 0 (C = %d), crops of at most 32 per side (%dx%d) and 16-byte aligned "
+                "grads and grad maps", C, ph, pw);
     for (int l = 0; l < n_levels; ++l) {
         BwdLevel &L = P.lv[l];
         L.out = maps[l];
@@ -1416,19 +1066,10 @@ static int crop_bwd_nhwc(int dtype, const void *grads, const float *boxes, const
         while ((1 << L.sg_shift) < L.sg.side) ++L.sg_shift;
         L.st_base = n_st;
         n_st += B * L.sg.nx * L.sg.ny;
-        if (use_tma) {
-            L.tiles_x = cdiv(L.W, bwdtma::TW);
-            L.tiles_y = cdiv(L.H, bwdtma::TH);
-        } else if (bwd_use_tile(ph, pw)) {
-            L.tiles_x = cdiv(L.W, BWD_TILE_WARPS * BWD_TILE);
-            L.tiles_y = cdiv(L.H, BWD_TILE);
-        } else {
-            L.tiles_x = cdiv(L.W, BWD_TW);
-            L.tiles_y = cdiv(L.H, BWD_ROWS);
-        }
+        L.tiles_x = cdiv(L.W, use_tma ? bwdtma::TW : BWD_TW);
+        L.tiles_y = cdiv(L.H, use_tma ? bwdtma::TH : BWD_ROWS);
         L.rcp_tiles_x = L.tiles_x ? 1.0f / (float)L.tiles_x : 0.f;
         L.rcp_tiles_y = L.tiles_y ? 1.0f / (float)L.tiles_y : 0.f;
-        vec4 = vec4 && aligned16(maps[l]);
         SLN_REQUIRE((size_t)L.H * L.W == 0 || maps[l] != nullptr, SLN_ERR_ARG, "null grad map");
     }
     {   // schedule levels by ascending map area
@@ -1453,7 +1094,6 @@ static int crop_bwd_nhwc(int dtype, const void *grads, const float *boxes, const
     BwdWs ws;
     ws.win = reinterpret_cast<RoiWin *>(p);        p += align_up(sizeof(RoiWin) * (size_t)N, 256);
     ws.axes = reinterpret_cast<RoiAxes *>(p);      p += align_up(sizeof(RoiAxes) * (size_t)N, 256);
-    ws.taps = reinterpret_cast<Tap *>(p);          p += align_up(sizeof(Tap) * (size_t)N * (size_t)(ph + pw), 256);
     ws.st_count = reinterpret_cast<int *>(p);      p += align_up(sizeof(int) * n_st_cap, 256);
     ws.st_off = reinterpret_cast<int *>(p);        p += align_up(sizeof(int) * n_st_cap, 256);
     ws.lv_table = reinterpret_cast<BwdLevel *>(p); p += align_up(sizeof(BwdLevel) * BWD_MAX_LEVELS, 256);
@@ -1461,32 +1101,30 @@ static int crop_bwd_nhwc(int dtype, const void *grads, const float *boxes, const
     ws.gid = reinterpret_cast<int *>(p);           p += align_up(sizeof(int) * (size_t)N, 256);
     ws.gcount = reinterpret_cast<int *>(p);        p += align_up(sizeof(int) * (size_t)B * n_levels, 256);
     ws.glist = reinterpret_cast<int *>(p);         p += align_up(sizeof(int) * (size_t)B * n_levels * (size_t)N, 256);
-    ws.entries = reinterpret_cast<ListEntry *>(p);
+    ws.entries = reinterpret_cast<ListEntryA *>(p);
 
+    const int queue_init = (int)bwd_tma_grid(tiles * cdiv(C, bwdtma::CH_MAX));   // ticket counter of the bulk-async kernel
     if (mode == 2) {
-        SLN_CUDA_OK(launch_chain(crop_bwd_republish_kernel, dim3(1), dim3(32), 0, st, true, P, ws.lv_table, ws.queue,
-                                 (int)bwd_tma_grid(tiles * cdiv(C, bwdtma::CH_MAX))));
+        SLN_CUDA_OK(launch_chain(crop_bwd_republish_kernel, dim3(1), dim3(32), 0, st, true, P, ws.lv_table, ws.queue, queue_init));
         SLN_LAUNCH_OK("crop_bwd_republish_kernel");
-        return launch_bwd_tma_dt(dtype, grads, exact, ws, P, tiles, C, ph, pw, st);
+    } else {
+        SLN_CUDA_OK(cudaMemsetAsync(ws.st_count, 0, sizeof(int) * (size_t)(n_st + 1), st));
+        // the windows kernel also publishes the level table, so it always runs (>= 1 CTA)
+        SLN_CUDA_OK(launch_chain(crop_bwd_windows_kernel, dim3(cdiv(N > BWD_MAX_LEVELS ? N : BWD_MAX_LEVELS, 256)), dim3(256), 0, st,
+                                 true, boxes, box_ind, level, N, B, ph, pw, P, ws.win, ws.axes, ws.st_count, ws.lv_table,
+                                 ws.queue, queue_init, ws.gid));
+        SLN_LAUNCH_OK("crop_bwd_windows_kernel");
+        if (N > 0 && n_st > 0) {
+            SLN_CUDA_OK(launch_chain(crop_bwd_group_kernel, dim3(B * n_levels), dim3(GROUP_THREADS), 0, st, true, (const int *)ws.gid,
+                                     N, ws.glist, ws.gcount));
+            SLN_LAUNCH_OK("crop_bwd_group_kernel");
+            SLN_CUDA_OK(launch_chain(crop_bwd_fill_kernel, dim3(n_st), dim3(FILL_THREADS), 0, st, true, (const int *)ws.glist,
+                                     (const int *)ws.gcount, (const RoiWin *)ws.win, (const RoiAxes *)ws.axes, N, P,
+                                     (const int *)ws.st_count, ws.st_off, ws.entries));
+            SLN_LAUNCH_OK("crop_bwd_fill_kernel");
+        }
+        if (mode == 1) return SLN_OK;
     }
-    SLN_CUDA_OK(cudaMemsetAsync(ws.st_count, 0, sizeof(int) * (size_t)(n_st + 1), st));
-    // the windows kernel also publishes the level table, so it always runs (>= 1 CTA)
-    // the bulk-async kernel plans from the ROI's sampling grid (axes), the strip / tile forms from tap tables
-    SLN_CUDA_OK(launch_chain(crop_bwd_windows_kernel, dim3(cdiv(N > BWD_MAX_LEVELS ? N : BWD_MAX_LEVELS, 256)), dim3(256), 0, st, true,
-                             boxes, box_ind, level, N, B, ph, pw, P, ws.win, use_tma ? (Tap *)nullptr : ws.taps,
-                             use_tma ? ws.axes : (RoiAxes *)nullptr, ws.st_count, ws.lv_table, ws.queue,
-                             (int)bwd_tma_grid(tiles * cdiv(C, bwdtma::CH_MAX)), ws.gid));
-    SLN_LAUNCH_OK("crop_bwd_windows_kernel");
-    if (N > 0 && n_st > 0) {
-        SLN_CUDA_OK(launch_chain(crop_bwd_group_kernel, dim3(B * n_levels), dim3(GROUP_THREADS), 0, st, true, (const int *)ws.gid, N,
-                                 ws.glist, ws.gcount));
-        SLN_LAUNCH_OK("crop_bwd_group_kernel");
-        SLN_CUDA_OK(launch_chain(use_tma ? crop_bwd_fill_kernel<true> : crop_bwd_fill_kernel<false>, dim3(n_st), dim3(FILL_THREADS), 0, st,
-                                 true, (const int *)ws.glist, (const int *)ws.gcount, (const RoiWin *)ws.win, (const RoiAxes *)ws.axes, N, P,
-                                 (const int *)ws.st_count, ws.st_off, (void *)ws.entries));
-        SLN_LAUNCH_OK("crop_bwd_fill_kernel");
-    }
-    if (mode == 1) return SLN_OK;
     if (use_tma) return launch_bwd_tma_dt(dtype, grads, exact, ws, P, tiles, C, ph, pw, st);
     const float *g32 = static_cast<const float *>(grads);
     if (vec4) {
@@ -1550,7 +1188,7 @@ extern "C" int sln_crop_and_resize_fwd(const float *image, int B, int C, int H, 
 extern "C" size_t sln_crop_and_resize_bwd_workspace_bytes(int N, int B, int ph, int pw)
 {
     if (N < 0 || B < 0 || ph < 1 || pw < 1) return 0;
-    return bwd_ws_bytes(N, B, 1, ph, pw);
+    return bwd_ws_bytes(N, B, 1);
 }
 
 extern "C" int sln_crop_and_resize_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind, int N,
@@ -1606,7 +1244,7 @@ extern "C" int sln_pyramid_crop_fwd(const float *const *maps_host, const int *H_
 extern "C" size_t sln_pyramid_crop_bwd_workspace_bytes(int N, int B, int n_levels, int ph, int pw)
 {
     if (N < 0 || B < 0 || n_levels < 1 || n_levels > BWD_MAX_LEVELS || ph < 1 || pw < 1) return 0;
-    return bwd_ws_bytes(N, B, n_levels, ph, pw);
+    return bwd_ws_bytes(N, B, n_levels);
 }
 
 extern "C" int sln_pyramid_crop_bwd_ex(int dtype, const void *grads, const float *boxes, const int *box_ind, const int *level,

@@ -3,7 +3,7 @@
 // Reference semantics: roialign/roi_align/src/crop_and_resize.c:157-252 (serial scatter, order (box, y, x, tap));
 // GPU baseline being replaced: cuda/crop_and_resize_kernel.cu:84-165 (atomicAdd scatter).
 //
-// Why another form: the strip / tile-owner kernels (crop.cu) spend ~7 warp instructions on search and addressing
+// Why another form: the strip kernel (crop.cu) spends ~7 warp instructions on search and addressing
 // per useful FMA and stall on every gradient load (ncu, round 1: 389 M warp instructions for 50 M warp-FMAs at 14x14,
 // 48 % of the stall samples on the first FMA after the loads).  Here the search, the data movement and the arithmetic
 // are three decoupled agents of a persistent CTA (two CTAs per SM, each walking tiles blockIdx.x, + gridDim.x, ...):

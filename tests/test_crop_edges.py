@@ -69,8 +69,8 @@ def edge_boxes(N, seed):
 
 # --------------------------------------------------------------------------- backward dispatch matrix
 # `kernel` names the instantiation the case is meant to reach: (kernel name, template arguments) with "E" for the EXACT
-# flag.  crop_bwd_tma_kernel<NV, EXACT, FULL, STG_S, NST>, crop_bwd_nhwc_kernel<VEC, NV, EXACT> (strip form),
-# crop_bwd_tile_kernel<VEC, NV, EXACT, FULL>.
+# flag.  Two forms: crop_bwd_tma_kernel<NV, EXACT, FULL, STG_S, NST> (bulk-async) and crop_bwd_nhwc_kernel<VEC, NV, EXACT>
+# (strip form, every shape the bulk-async kernel does not take).
 class BwdCase(NamedTuple):
     C: int
     H: int
@@ -101,8 +101,8 @@ for _ph, _pw in ((33, 33), (7, 40), (255, 1), (40, 255)):     # wider than 32 pe
         132, *_STRIP_BIG_MAP, _ph, _pw, False, ("crop_bwd_nhwc_kernel", (4, 2, "E")))
     BWD_CASES[f"strip-vec4-nv1-C132-{_ph}x{_pw}-map24x20"] = BwdCase(
         132, *_STRIP_SMALL_MAP, _ph, _pw, False, ("crop_bwd_nhwc_kernel", (4, 1, "E")))
-# channels_last-dense grads 4 bytes off a 16-byte boundary: the scalar (VEC1) forms
-BWD_CASES["tile-vec1-nv2-full-misaligned-C256-8x8"] = BwdCase(256, 40, 40, 8, 8, True, ("crop_bwd_tile_kernel", (1, 2, "E", 1)))
+# channels_last-dense grads 4 bytes off a 16-byte boundary: the scalar (VEC1) strip form
+BWD_CASES["strip-vec1-nv1-misaligned-C256-8x8"] = BwdCase(256, 40, 40, 8, 8, True, ("crop_bwd_nhwc_kernel", (1, 1, "E")))
 BWD_CASES["strip-vec1-nv1-misaligned-C256-14x14"] = BwdCase(256, 40, 40, 14, 14, True, ("crop_bwd_nhwc_kernel", (1, 1, "E")))
 
 
@@ -173,7 +173,7 @@ def test_backward_dispatch_matrix_reaches_the_named_kernels():
                      key=lambda e: e.time_range.start)
     if not kernels:
         pytest.skip("torch.profiler recorded no CUDA kernels on this host (CUPTI unavailable)")
-    main = [e.name for e in kernels if re.search(r"crop_bwd_(tma|tile|nhwc)_kernel<", e.name)]
+    main = [e.name for e in kernels if re.search(r"crop_bwd_(tma|nhwc)_kernel<", e.name)]
     assert len(main) == len(calls), (len(main), len(calls))
     for name, (cid, exact, *_) in zip(main, calls):
         kernel, args = BWD_CASES[cid].kernel
@@ -204,7 +204,7 @@ def _pyramid_inputs(C, pool, seed):
 
 
 @gpu
-@pytest.mark.parametrize("C,pool", [(16, 7), (16, 14), (6, 7)], ids=["tma-small-stages", "tma-large-stages", "C6-tile"])
+@pytest.mark.parametrize("C,pool", [(16, 7), (16, 14), (6, 7)], ids=["tma-small-stages", "tma-large-stages", "C6-strip"])
 def test_pyramid_eight_levels_and_invalid_rows(C, pool):
     """Eight levels (maps above 256 a side, 1xW, Hx1, 1x1, one level without ROIs), level -1 / 8 and box_ind -1 / B.
     Forward: per-level values bit-exact, rows of an invalid level or image exactly zero.  Backward: per level, exact and
@@ -234,6 +234,37 @@ def test_pyramid_eight_levels_and_invalid_rows(C, pool):
             res[exact] = [host(o) for o in ops.pyramid_crop_backward(gt, tb, ti, tl, sizes, exact=exact, plan=plan)]
         for lv in range(len(maps)):
             check_backward(res[True][lv], res[False][lv], wants[lv], f"level {lv} {PYR_SIZES[lv]} planned={planned}")
+
+
+def _crop_bwd_kernels(prof):
+    """Short names (windows, group, fill, republish, tma, nhwc) of the crop_bwd kernels a profile recorded, sorted."""
+    return sorted(re.search(r"crop_bwd_(\w+?)_kernel", e.name).group(1) for e in prof.events()
+                  if e.device_type == torch.autograd.DeviceType.CUDA and "crop_bwd_" in e.name)
+
+
+@gpu
+@pytest.mark.parametrize("C,pool", [(6, 7), (16, 33)], ids=["C6-7x7", "C16-33x33"])
+def test_planned_strip_backward_skips_the_prep_kernels(C, pool):
+    """Shapes the bulk-async kernel does not take (ragged C, crops wider than 32 per side) plan ahead like the others: the
+    plan call launches the three prep kernels, and the planned backward only republishes the level table and gathers."""
+    from torch.profiler import ProfilerActivity, profile
+    from sln_amodal_b200 import ops
+    maps, boxes, ind, level, g, _ = _pyramid_inputs(C, pool, seed=C + pool)
+    tb, ti, tl = cuda(boxes), cuda(ind), cuda(level)
+    sizes = [m.shape for m in maps]
+    gt = cuda(g).contiguous(memory_format=torch.channels_last)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof_plan:
+        plan = ops.pyramid_crop_backward_plan(tb, ti, tl, sizes, C, pool, pool)
+        torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof_bwd:
+        ops.pyramid_crop_backward(gt, tb, ti, tl, sizes, plan=plan)
+        torch.cuda.synchronize()
+    plan_kernels, bwd_kernels = _crop_bwd_kernels(prof_plan), _crop_bwd_kernels(prof_bwd)
+    if not plan_kernels and not bwd_kernels:
+        pytest.skip("torch.profiler recorded no CUDA kernels on this host (CUPTI unavailable)")
+    assert plan_kernels == ["fill", "group", "windows"], plan_kernels
+    assert bwd_kernels == ["nhwc", "republish"], bwd_kernels
 
 
 # --------------------------------------------------------------------------- forward size edges

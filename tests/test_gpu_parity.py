@@ -896,26 +896,33 @@ def test_config2_contention_4000_rois_per_image_vs_reference_c():
     assert_close_rel(got, want)
 
 
-@pytest.mark.parametrize("impl", ["0", "1", "3"])
-def test_backward_kernel_forms_agree(impl, monkeypatch):
-    """The three backward forms (strip, tile owner, bulk-async; SLN_BWD_IMPL) produce the same bits in exact mode,
-    also for flipped / degenerate boxes, ragged maps and crops that need several stages per sample row."""
+@pytest.mark.parametrize("C,H,W,N,ph,pw", [(256, 40, 40, 200, 7, 7), (128, 50, 70, 150, 32, 32), (68, 21, 37, 120, 9, 20),
+                                           (512, 24, 24, 60, 14, 14)])
+@pytest.mark.parametrize("misaligned", [False, True], ids=["bulk-async", "strip-vec1"])
+def test_backward_kernel_forms_agree(misaligned, C, H, W, N, ph, pw):
+    """Both backward forms produce the oracle's bits in exact mode, also for flipped / degenerate boxes, ragged maps and
+    crops that need several stages per sample row: aligned grads take the bulk-async kernel, channels_last-dense grads
+    4 bytes off a 16-byte boundary the strip kernel with scalar loads."""
     from sln_amodal_b200 import ops
-    rng = np.random.default_rng(5)
-    for C, H, W, N, ph, pw in ((256, 40, 40, 200, 7, 7), (128, 50, 70, 150, 32, 32), (68, 21, 37, 120, 9, 20), (512, 24, 24, 60, 14, 14)):
-        B = 2
-        boxes = synth.roi_boxes(N, seed=N, outside_frac=0.2, degenerate_frac=0.1)
-        boxes[::7] = boxes[::7][:, [2, 1, 0, 3]]                   # y-flipped
-        boxes[::11] = boxes[::11][:, [0, 3, 2, 1]]                 # x-flipped
-        ind = rng.integers(0, B, N).astype(np.int32)
-        g = rng.standard_normal((N, C, ph, pw), dtype=np.float32)
-        want = oracle.crop_and_resize_bwd(g, boxes, ind, (B, C, H, W))
-        monkeypatch.setenv("SLN_BWD_IMPL", impl)
+    rng = np.random.default_rng(5 + N)
+    B = 2
+    boxes = synth.roi_boxes(N, seed=N, outside_frac=0.2, degenerate_frac=0.1)
+    boxes[::7] = boxes[::7][:, [2, 1, 0, 3]]                   # y-flipped
+    boxes[::11] = boxes[::11][:, [0, 3, 2, 1]]                 # x-flipped
+    ind = rng.integers(0, B, N).astype(np.int32)
+    g = rng.standard_normal((N, C, ph, pw), dtype=np.float32)
+    want = oracle.crop_and_resize_bwd(g, boxes, ind, (B, C, H, W))
+    if misaligned:
+        nhwc = torch.empty(g.size + 1, dtype=torch.float32, device=dev())[1:].view(N, ph, pw, C)
+        nhwc.copy_(torch.from_numpy(np.ascontiguousarray(g.transpose(0, 2, 3, 1))))
+        gt = nhwc.permute(0, 3, 1, 2)
+        assert gt.is_contiguous(memory_format=torch.channels_last) and gt.data_ptr() % 16 == 4
+    else:
         gt = cuda(g).contiguous(memory_format=torch.channels_last)
-        got = ops.crop_and_resize_backward(gt, cuda(boxes), cuda(ind), (B, C, H, W), exact=True).contiguous().cpu().numpy()
-        assert got.tobytes() == want.tobytes(), (impl, C, H, W, ph, pw)
-        got = ops.crop_and_resize_backward(gt, cuda(boxes), cuda(ind), (B, C, H, W), exact=False).contiguous().cpu().numpy()
-        assert_close_rel(got, want, rtol=2e-6)
+    got = ops.crop_and_resize_backward(gt, cuda(boxes), cuda(ind), (B, C, H, W), exact=True).contiguous().cpu().numpy()
+    assert got.tobytes() == want.tobytes()
+    got = ops.crop_and_resize_backward(gt, cuda(boxes), cuda(ind), (B, C, H, W), exact=False).contiguous().cpu().numpy()
+    assert_close_rel(got, want, rtol=2e-6)
 
 
 @pytest.mark.parametrize("pool", [7, 14])

@@ -1,7 +1,7 @@
-"""A/B of the RoIAlign backward kernels in one process (SLN_BWD_IMPL is read per call):
-   2 = strip / tile-owner forms (round 1), 3 = bulk-async form (crop_bwd_tma.cuh).
-   Checks impl 3 against impl 2 on the config-2 workload (exact mode: bit-equal; default mode: max rel error) and
-   times both with CUDA events (working set >> L2).   python tools/ab_bwd_impl.py [rois_per_img ...]"""
+"""A/B of the bulk-async backward's stage configurations (crop_bwd_tma.cuh) in one process (SLN_BWD_CFG is read per
+   call): "auto" = by crop size, c0 = 32 x 3, c1 = 16 x 6.  Checks every arm against auto on the config-2 workload (exact
+   mode: bit-equal; default mode: max rel error against auto's exact result) and times each with CUDA events
+   (working set >> L2).   python tools/ab_bwd_impl.py [rois_per_img ...]"""
 import json, os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -40,21 +40,20 @@ for per in pers:
         bb = sum(bench.bwd_bytes(int((level_np == l).sum()), side, p) for l, side in enumerate(bench.LEVEL_SIDES))
         row = {"rois_per_img": per, "pool": p}
         outs = {}
-        for impl in ("2", "3") + tuple("3c%d" % k for k in range(2)):
-            os.environ["SLN_BWD_IMPL"] = impl[0]
+        for impl in ("auto", "c0", "c1"):
             os.environ.pop("SLN_BWD_CFG", None)
-            if len(impl) > 1:
-                os.environ["SLN_BWD_CFG"] = impl[2]
+            if impl != "auto":
+                os.environ["SLN_BWD_CFG"] = impl[1]
             for exact in (False, True):
                 outs[(impl, exact)] = ops.pyramid_crop_backward(g, boxes, ind, level, maps_shape, exact=exact)
             ms = timed(lambda: ops.pyramid_crop_backward(g, boxes, ind, level, maps_shape))
             row["ms_impl%s" % impl] = round(ms, 4)
             row["frac_impl%s" % impl] = round(bb / ms / 1e6 / peak, 3)
-        row["exact_bit_equal"] = all(all(torch.equal(a, b) for a, b in zip(outs[("2", True)], outs[(k, True)]))
-                                     for k in ("3", "3c0", "3c1"))
+        row["exact_bit_equal"] = all(all(torch.equal(a, b) for a, b in zip(outs[("auto", True)], outs[(k, True)]))
+                                     for k in ("c0", "c1"))
         err = 0.0
-        for k in ("3", "3c0", "3c1"):
-            for b, e in zip(outs[(k, False)], outs[("2", True)]):
+        for k in ("auto", "c0", "c1"):
+            for b, e in zip(outs[(k, False)], outs[("auto", True)]):
                 err = max(err, float((b - e).abs().max() / e.abs().max()))
         row["default_max_rel_err"] = err
         rows.append(row)

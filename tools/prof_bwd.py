@@ -1,5 +1,5 @@
 """ncu driver: the config-2 backward (8 images, C=256, P2-P5, 8 x per ROIs), pools 7 and 14, two calls each.
-   python tools/prof_bwd.py [rois_per_img] [impl]"""
+   python tools/prof_bwd.py [rois_per_img]"""
 import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -7,8 +7,6 @@ sys.path.insert(0, ROOT)
 import bench
 from sln_amodal_b200 import ops, synth
 per = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
-if len(sys.argv) > 2:
-    os.environ["SLN_BWD_IMPL"] = sys.argv[2]
 dev = torch.device("cuda", 0)
 n = 8 * per
 boxes_np = synth.roi_boxes(n, seed=4321)
