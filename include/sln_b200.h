@@ -217,6 +217,12 @@ SLN_API int sln_refine_decode(const float *rois, const float *probs, const float
  * touched.  One launch, no host sync.                                                                      */
 SLN_API int sln_refine_topk(const float *dets, const int *class_ids, int N, int max_keep, float *result,
                     int64_t *keep, void *stream);
+/* B images of N rows each in one launch: dets f32 [B,N,5], class_ids i32 [B,N] -> result f32 [B,max_keep,6], keep i64
+ * [B,max_keep] (row indices within the image) and num_det device i32 [B] = min(max_keep, rows of the image with
+ * class_id > 0 and score > -inf).  Image b's rows [0, num_det[b]) are what sln_refine_topk writes for that image alone;
+ * later rows are not touched.  No host sync.                                                                   */
+SLN_API int sln_refine_topk_batched(const float *dets, const int *class_ids, int B, int N, int max_keep, float *result,
+                            int64_t *keep, int *num_det, void *stream);
 
 /* ---- detection targets (SURVEY 8(f)-1) -------------------------------------- *
  * sln_bbox_overlaps replaces bbox_overlaps (modal/Functions.py:184-218): IoU of boxes1 [N,4] against boxes2 [G,4]
@@ -312,6 +318,17 @@ SLN_API int sln_proposal_layer(const float *probs, const float *deltas, const fl
                        const float *std_dev_host, float img_h, float img_w,
                        float *out_boxes, int *num_out,
                        void *workspace, size_t workspace_bytes, void *stream);
+/* B images per call, one launch per stage for all of them (the dense NMS fallback aside: it is launched per image and
+ * returns at once where that image's sparse pass succeeded).  probs f32 [B,A,2], deltas f32 [B,A,4], anchors f32 [A,4]
+ * shared by all images; out_boxes f32 [B,proposal_count,4], num_out device i32 [B].  For every image b, out_boxes[b] and
+ * num_out[b] are bit-identical to sln_proposal_layer on that image alone, zero padding included.  No host sync, graph
+ * capturable; B == 0 and proposal_count == 0 are valid.  Workspace: B copies of the single-image one.          */
+SLN_API size_t sln_proposal_batched_workspace_bytes(int B, int A, int pre_nms_limit);
+SLN_API int sln_proposal_layer_batched(const float *probs, const float *deltas, const float *anchors, int B, int A,
+                               int pre_nms_limit, int proposal_count, float nms_thresh,
+                               const float *std_dev_host, float img_h, float img_w,
+                               float *out_boxes, int *num_out,
+                               void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- sem-dist target encoding ------------------------------------------- *
  * Layer codec: replaces AmodalDataset.load_layer2 (amodal_train.py:236-271) and the

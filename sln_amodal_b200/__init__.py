@@ -9,7 +9,7 @@ fails loudly if sln_amodal_b200/libsln_b200.so has not been built
 """
 from .crop_and_resize import CropAndResize, CropAndResizeFunction, RoIAlign  # noqa: F401
 from .nms import batched_nms, nms, pth_nms  # noqa: F401
-from .proposal import proposal_layer, proposal_layer_padded  # noqa: F401
+from .proposal import proposal_layer, proposal_layer_batched, proposal_layer_padded  # noqa: F401
 from .pyramid import pyramid_roi_align, pyramid_roi_align_batched, pyramid_roi_align_image  # noqa: F401
 from .semdist import decode_layers, load_layer2, sem_dist_targets  # noqa: F401
 from .detection import refine_detections  # noqa: F401

@@ -52,6 +52,7 @@ PROTOTYPES = {
     "sln_nms_ex": (_i, [_vp, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "sln_refine_decode": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(_f), _f, _f, C.POINTER(_f), _f, _vp, _vp, _vp, _vp, _vp]),
     "sln_refine_topk": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "sln_refine_topk_batched": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "sln_bbox_overlaps": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp]),
     "sln_box_refinement": (_i, [_vp, _vp, _i, C.POINTER(_f), _vp, _vp]),
     "sln_mask_targets": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
@@ -68,6 +69,8 @@ PROTOTYPES = {
     "sln_rpn_unpack_grads": (_i, [_vp, _vp, C.POINTER(_i), C.POINTER(_i), _i, _i, _i, _i, C.POINTER(_vp), C.POINTER(_vp), _vp]),
     "sln_proposal_workspace_bytes": (_sz, [_i, _i]),
     "sln_proposal_layer": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, C.POINTER(_f), _f, _f, _vp, _vp, _vp, _sz, _vp]),
+    "sln_proposal_batched_workspace_bytes": (_sz, [_i, _i, _i]),
+    "sln_proposal_layer_batched": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, C.POINTER(_f), _f, _f, _vp, _vp, _vp, _sz, _vp]),
     "sln_layer_decode": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "sln_edt_workspace_bytes": (_sz, [_i, _i, _i]),
     "sln_edt_sq": (_i, [_vp, _i, _i, _i, _vp, _vp, _sz, _vp]),

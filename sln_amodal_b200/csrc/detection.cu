@@ -101,9 +101,10 @@ namespace sln {
 
 constexpr int TOPK_THREADS = 256;
 
-__global__ void __launch_bounds__(TOPK_THREADS)
-refine_topk_kernel(const float *__restrict__ dets, const int *__restrict__ class_ids, int N, int max_keep,
-                   float *__restrict__ result, long long *__restrict__ keep)
+// num_det (nullptr in the single-image kernel): one count per written row, i.e. min(#valid rows, max_keep) in all
+__device__ __forceinline__ void refine_topk_body(const float *dets, const int *class_ids, int N,
+                                                 int max_keep, float *result, long long *keep,
+                                                 int *num_det)
 {
     __shared__ __align__(16) float s_score[TOPK_THREADS];
     const int i = blockIdx.x * TOPK_THREADS + threadIdx.x;
@@ -145,6 +146,24 @@ refine_topk_kernel(const float *__restrict__ dets, const int *__restrict__ class
     o[4] = (float)__ldg(class_ids + i);
     o[5] = si;
     keep[rank] = i;
+    if (num_det) atomicAdd(num_det, 1);
+}
+
+__global__ void __launch_bounds__(TOPK_THREADS)
+refine_topk_kernel(const float *__restrict__ dets, const int *__restrict__ class_ids, int N, int max_keep,
+                   float *__restrict__ result, long long *__restrict__ keep)
+{
+    refine_topk_body(dets, class_ids, N, max_keep, result, keep, nullptr);
+}
+
+// image b = blockIdx.y: rows [b*N, (b+1)*N), ranked among themselves; keep holds row indices within the image
+__global__ void __launch_bounds__(TOPK_THREADS)
+refine_topk_seg_kernel(const float *__restrict__ dets, const int *__restrict__ class_ids, int N, int max_keep,
+                       float *__restrict__ result, long long *__restrict__ keep, int *__restrict__ num_det)
+{
+    const size_t b = blockIdx.y;
+    refine_topk_body(dets + 5 * (size_t)N * b, class_ids + (size_t)N * b, N, max_keep, result + 6 * (size_t)max_keep * b,
+                     keep + (size_t)max_keep * b, num_det + b);
 }
 
 }  // namespace sln
@@ -158,6 +177,23 @@ extern "C" int sln_refine_topk(const float *dets, const int *class_ids, int N, i
     sln::refine_topk_kernel<<<sln::cdiv(N, sln::TOPK_THREADS), sln::TOPK_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
         dets, class_ids, N, max_keep, result, reinterpret_cast<long long *>(keep));
     SLN_LAUNCH_OK("refine_topk_kernel");
+    return SLN_OK;
+}
+
+extern "C" int sln_refine_topk_batched(const float *dets, const int *class_ids, int B, int N, int max_keep, float *result,
+                                       int64_t *keep, int *num_det, void *stream)
+{
+    SLN_REQUIRE(B >= 0 && N >= 0 && max_keep >= 0, SLN_ERR_ARG, "negative size");
+    SLN_REQUIRE(B <= 65535, SLN_ERR_ARG, "B=%d images in one call (at most 65535)", B);
+    if (B == 0) return SLN_OK;
+    SLN_REQUIRE(num_det, SLN_ERR_ARG, "null num_det");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    SLN_CUDA_OK(cudaMemsetAsync(num_det, 0, sizeof(int) * (size_t)B, st));
+    if (N == 0 || max_keep == 0) return SLN_OK;
+    SLN_REQUIRE(dets && class_ids && result && keep, SLN_ERR_ARG, "null pointer");
+    sln::refine_topk_seg_kernel<<<dim3(sln::cdiv(N, sln::TOPK_THREADS), B), sln::TOPK_THREADS, 0, st>>>(
+        dets, class_ids, N, max_keep, result, reinterpret_cast<long long *>(keep), num_det);
+    SLN_LAUNCH_OK("refine_topk_seg_kernel");
     return SLN_OK;
 }
 

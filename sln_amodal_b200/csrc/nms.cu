@@ -91,9 +91,8 @@ struct RankGather {
     int *tickets;              // [ceil(n / RANK_ROWS)]
 };
 
-__global__ void __launch_bounds__(RANK_ROWS)
-rank_kernel(const float *__restrict__ scores, int stride, const int *__restrict__ tie_ids, int n,
-            int *__restrict__ rank, RankGather ga)
+__device__ __forceinline__ void rank_body(const float *scores, int stride, const int *tie_ids, int n,
+                                          int *rank, RankGather ga)
 {
     __shared__ __align__(16) unsigned s_key[RANK_COLS];
     __shared__ __align__(16) unsigned s_tie[RANK_COLS];     // ~tie id
@@ -166,6 +165,22 @@ rank_kernel(const float *__restrict__ scores, int stride, const int *__restrict_
     if (ga.class_ids) ga.cls[r] = ga.class_ids[i];
 }
 
+__global__ void __launch_bounds__(RANK_ROWS)
+rank_kernel(const float *__restrict__ scores, int stride, const int *__restrict__ tie_ids, int n,
+            int *__restrict__ rank, RankGather ga)
+{
+    rank_body(scores, stride, tie_ids, n, rank, ga);
+}
+
+// segment z = blockIdx.z: contiguous scores (stride 1), explicit tie ids, no gather
+__global__ void __launch_bounds__(RANK_ROWS)
+rank_seg_kernel(const float *__restrict__ scores, const int *__restrict__ tie_ids, int n, int *__restrict__ rank,
+                size_t seg_stride)
+{
+    const int z = blockIdx.z;
+    rank_body(seg_at(scores, seg_stride, z), 1, seg_at(tie_ids, seg_stride, z), n, seg_at(rank, seg_stride, z), RankGather{});
+}
+
 static int rank_launch(const float *scores, int stride, const int *tie_ids, int n, int *rank, const RankGather &ga,
                        cudaStream_t st)
 {
@@ -180,6 +195,17 @@ static int rank_launch(const float *scores, int stride, const int *tie_ids, int 
 int rank_sort_launch(const float *scores, int stride, const int *tie_ids, int n, int *rank, cudaStream_t st)
 {
     return rank_launch(scores, stride, tie_ids, n, rank, RankGather{}, st);
+}
+
+int rank_sort_batched_launch(const float *scores, const int *tie_ids, int n, int B, size_t stride_bytes, int *rank,
+                             cudaStream_t st)
+{
+    if (n <= 0 || B <= 0) return SLN_OK;
+    dim3 grid(cdiv(n, RANK_ROWS), cdiv(n, RANK_COLS), B);
+    SLN_REQUIRE(grid.y <= 65535 && grid.z <= 65535, SLN_ERR_ARG, "rank sort: n=%d x %d segments too large", n, B);
+    rank_seg_kernel<<<grid, RANK_ROWS, 0, st>>>(scores, tie_ids, n, rank, stride_bytes);
+    SLN_LAUNCH_OK("rank_seg_kernel");
+    return SLN_OK;
 }
 
 // ---------------------------------------------------------------------------
@@ -828,9 +854,9 @@ __device__ __forceinline__ bool sp_sane(const float4 b)
 constexpr int SP_BIN_ITEMS = (SP_MAX_N + SP_CLUSTER * SP_BIN_THREADS - 1) / (SP_CLUSTER * SP_BIN_THREADS);   // 8
 
 template <bool CLS>
-__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_BIN_THREADS)
-nms_bin_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
-               int G, int CB, SparseBufs sb, int *__restrict__ num_keep_preset)
+__device__ __forceinline__ void nms_bin_body(const float4 *boxes, const float *areas,
+                                             const int *cls, int n, int G, int CB, SparseBufs sb,
+                                             int *num_keep_preset)
 {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
@@ -984,14 +1010,46 @@ nms_bin_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas
     }
 }
 
+template <bool CLS>
+__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_BIN_THREADS)
+nms_bin_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
+               int G, int CB, SparseBufs sb, int *__restrict__ num_keep_preset)
+{
+    nms_bin_body<CLS>(boxes, areas, cls, n, G, CB, sb, num_keep_preset);
+}
+
+// problem b of a batched call (nms_sorted_batched_launch): every buffer moved by b * stride bytes
+__device__ __forceinline__ SparseBufs sparse_at(SparseBufs sb, size_t stride, int b)
+{
+    sb.hdr = seg_at(sb.hdr, stride, b);
+    sb.cell_start = seg_at(sb.cell_start, stride, b);
+    sb.cbox = seg_at(sb.cbox, stride, b);
+    sb.carea = seg_at(sb.carea, stride, b);
+    sb.cpos = seg_at(sb.cpos, stride, b);
+    sb.ccls = seg_at(sb.ccls, stride, b);
+    sb.inl = seg_at(sb.inl, stride, b);
+    sb.seg = seg_at(sb.seg, stride, b);
+    sb.edges = seg_at(sb.edges, stride, b);
+    return sb;
+}
+
+// grid (SP_CLUSTER, B): the cluster of blockIdx.y bins problem blockIdx.y
+__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_BIN_THREADS)
+nms_bin_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, int n, int G, SparseBufs sb,
+                   size_t stride)
+{
+    const int b = blockIdx.y;
+    nms_bin_body<false>(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, n, G, 1, sparse_at(sb, stride, b), nullptr);
+}
+
 // warp per box (grid-strided): exact tests against the boxes binned in the window's cells.  The window's cell
 // rows are contiguous ranges of the cell-sorted arrays; their (start, running count) table is built once per box
 // in shared memory (one row per lane, all loads in flight together) and the lanes then walk the concatenation of
 // the ranges, so every pass tests 32 candidates whatever the row lengths are.
 template <bool CLS>
-__global__ void __launch_bounds__(32 * SP_PAIR_WARPS)
-nms_pairs_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
-                 float thresh, float ct, unsigned edge_cap, SparseBufs sb)
+__device__ __forceinline__ void nms_pairs_body(const float4 *boxes, const float *areas,
+                                               const int *cls, int n, float thresh, float ct, unsigned edge_cap,
+                                               SparseBufs sb)
 {
     __shared__ unsigned s_buf[SP_PAIR_WARPS][SP_WARP_BUF];
     __shared__ int s_rs[SP_PAIR_WARPS][64];        // first item of each window row
@@ -1095,6 +1153,23 @@ nms_pairs_kernel(const float4 *__restrict__ boxes, const float *__restrict__ are
     }
 }
 
+template <bool CLS>
+__global__ void __launch_bounds__(32 * SP_PAIR_WARPS)
+nms_pairs_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
+                 float thresh, float ct, unsigned edge_cap, SparseBufs sb)
+{
+    nms_pairs_body<CLS>(boxes, areas, cls, n, thresh, ct, edge_cap, sb);
+}
+
+__global__ void __launch_bounds__(32 * SP_PAIR_WARPS)
+nms_pairs_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, int n, float thresh, float ct,
+                     unsigned edge_cap, SparseBufs sb, size_t stride)
+{
+    const int b = blockIdx.y;
+    nms_pairs_body<false>(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, n, thresh, ct, edge_cap,
+                          sparse_at(sb, stride, b));
+}
+
 // One cluster of SP_CLUSTER CTAs: the greedy survivor set from the predecessor lists, then ordered emission.
 // Two monotone sets, full copies in every CTA's shared memory:  KF = boxes known kept, DF = boxes known dead.
 //   box b is dead   as soon as one predecessor is in KF,
@@ -1146,9 +1221,9 @@ __device__ __forceinline__ void sp_scan8(const unsigned *KF, const unsigned *DF,
     }
 }
 
-__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_RESOLVE_THREADS, 1)
-nms_sparse_resolve_kernel(const int *__restrict__ order, int n, int max_keep, unsigned edge_cap, SparseBufs sb,
-                          int64_t *__restrict__ keep64, int *__restrict__ keep32, int *__restrict__ num_keep)
+__device__ __forceinline__ void nms_sparse_resolve_body(const int *order, int n, int max_keep, unsigned edge_cap,
+                                                        SparseBufs sb, int64_t *keep64, int *keep32,
+                                                        int *num_keep)
 {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
@@ -1329,6 +1404,41 @@ nms_sparse_resolve_kernel(const int *__restrict__ order, int n, int max_keep, un
     }
 }
 
+__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_RESOLVE_THREADS, 1)
+nms_sparse_resolve_kernel(const int *__restrict__ order, int n, int max_keep, unsigned edge_cap, SparseBufs sb,
+                          int64_t *__restrict__ keep64, int *__restrict__ keep32, int *__restrict__ num_keep)
+{
+    nms_sparse_resolve_body(order, n, max_keep, edge_cap, sb, keep64, keep32, num_keep);
+}
+
+// grid (SP_CLUSTER, B): one cluster per problem; clusters beyond the GPU's cluster capacity queue
+__global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_RESOLVE_THREADS, 1)
+nms_sparse_resolve_seg_kernel(int n, int max_keep, unsigned edge_cap, SparseBufs sb, int *__restrict__ keep32,
+                              int *__restrict__ num_keep, size_t stride)
+{
+    const int b = blockIdx.y;
+    nms_sparse_resolve_body(nullptr, n, max_keep, edge_cap, sparse_at(sb, stride, b), nullptr, seg_at(keep32, stride, b),
+                            seg_at(num_keep, stride, b));
+}
+
+// grid: ~3 boxes per cell; the class-aware call spends the cells on class buckets first.  ct: the window's half-width
+// per unit of box width (see the contract above nms_bin_kernel)
+static void sparse_params(int n, bool has_cls, float thresh, int &CB, int &G, float &ct)
+{
+    CB = 1; G = 64;
+    if (has_cls) { CB = 64; G = 8; }
+    while (G > 8 && (long long)CB * G * G > (long long)n / 2) G >>= 1;
+    const float t = thresh > 1.f ? 1.f : thresh;
+    ct = (1.f - t) * (t < 0.5f ? 0.5f / t : 1.f) * 1.01f;
+}
+
+static size_t sparse_resolve_smem(int n)
+{
+    int items = cdiv(cdiv(n, 32), SP_CLUSTER * 32);
+    if (items > SP_CACHE_ITEMS) items = SP_CACHE_ITEMS;
+    return sizeof(unsigned) * (2 * SP_WORDS + 32) + 2 * SP_OV_CACHE + (size_t)items * SP_RESOLVE_THREADS * sizeof(uint4) * SP_INL_V;
+}
+
 // returns the device address of the status word the dense kernels test (nullptr: sparse path not taken)
 static int launch_sparse(const float4 *boxes, const float *areas, const int *cls, const int *order, int n, float thresh,
                          int max_keep, int64_t *keep64, int *keep32, int *num_keep, void *sparse, cudaStream_t st,
@@ -1338,12 +1448,9 @@ static int launch_sparse(const float4 *boxes, const float *areas, const int *cls
     if (sparse == nullptr || n < SP_MIN_N || n > SP_MAX_N || !(thresh >= 0.05f)) return SLN_OK;
     SparseBufs sb;
     sparse_carve(sparse, n, sb);
-    // grid: ~3 boxes per cell; the class-aware call spends the cells on class buckets first
-    int CB = 1, G = 64;
-    if (cls) { CB = 64; G = 8; }
-    while (G > 8 && (long long)CB * G * G > (long long)n / 2) G >>= 1;
-    const float t = thresh > 1.f ? 1.f : thresh;
-    const float ct = (1.f - t) * (t < 0.5f ? 0.5f / t : 1.f) * 1.01f;
+    int CB, G;
+    float ct;
+    sparse_params(n, cls != nullptr, thresh, CB, G, ct);
     const unsigned edge_cap = (unsigned)SP_EDGES_PER_BOX * (unsigned)n;
     // rank -> bin -> pairs -> resolve is a chain of short kernels: programmatic dependent launches (common.cuh)
     int *preset = sparse_only ? num_keep : nullptr;
@@ -1353,9 +1460,7 @@ static int launch_sparse(const float4 *boxes, const float *areas, const int *cls
     if (ctas > SLN_SP_PAIR_CTAS_PER_SM * sm_count()) ctas = SLN_SP_PAIR_CTAS_PER_SM * sm_count();
     SLN_CUDA_OK(launch_chain(cls ? nms_pairs_kernel<true> : nms_pairs_kernel<false>, dim3(ctas), dim3(32 * SP_PAIR_WARPS), 0, st,
                              true, boxes, areas, cls, n, thresh, ct, edge_cap, sb));
-    int items = cdiv(cdiv(n, 32), SP_CLUSTER * 32);
-    if (items > SP_CACHE_ITEMS) items = SP_CACHE_ITEMS;
-    const size_t smem = sizeof(unsigned) * (2 * SP_WORDS + 32) + 2 * SP_OV_CACHE + (size_t)items * SP_RESOLVE_THREADS * sizeof(uint4) * SP_INL_V;
+    const size_t smem = sparse_resolve_smem(n);
     SLN_CUDA_OK(cudaFuncSetAttribute(nms_sparse_resolve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     SLN_CUDA_OK(launch_chain(nms_sparse_resolve_kernel, dim3(SP_CLUSTER), dim3(SP_RESOLVE_THREADS), smem, st, true, order, n,
                              max_keep, edge_cap, sb, keep64, keep32, num_keep));
@@ -1493,6 +1598,10 @@ static int launch_scan(const unsigned long long *mask, const int *order, int n_m
     return SLN_OK;
 }
 
+static int nms_dense_launch(const float4 *boxes, const float *areas, const int *cls, const int *order, int n, float thresh,
+                            int max_keep, unsigned long long *mask, int64_t *keep64, int *keep32, int *num_keep,
+                            cudaStream_t st, void *stage, void *fix, const int *skip);
+
 // `stage`: scratch for the two-stage path (nullptr: single stage).  `order == nullptr`: kept entries
 // are visiting positions.
 int nms_sorted_launch(const float4 *boxes, const float *areas, const int *cls, const int *order, int n,
@@ -1510,6 +1619,16 @@ int nms_sorted_launch(const float4 *boxes, const float *areas, const int *cls, c
                            sparse_only);
     if (rc != SLN_OK) return rc;
     if (sparse_only && skip != nullptr) return SLN_OK;      // the caller retries with SLN_NMS_DENSE_ONLY on num_keep < 0
+    return nms_dense_launch(boxes, areas, cls, order, n, thresh, max_keep, mask, keep64, keep32, num_keep, st, stage, fix, skip);
+}
+
+// The dense pipeline (one stage, or two for n >= NMS_TWO_STAGE_MIN with `stage`); every kernel leaves at once when
+// *skip == 1 (the sparse path produced the result).  max_keep is already normalised to [1, n].
+static int nms_dense_launch(const float4 *boxes, const float *areas, const int *cls, const int *order, int n, float thresh,
+                            int max_keep, unsigned long long *mask, int64_t *keep64, int *keep32, int *num_keep,
+                            cudaStream_t st, void *stage, void *fix, const int *skip)
+{
+    int rc;
     if (!nms_two_stage(n) || stage == nullptr) {
         const int W = cdiv(n, 64);
         rc = launch_mask(boxes, areas, cls, n, nullptr, W, thresh, mask, skip, fix, st);
@@ -1548,6 +1667,51 @@ int nms_sorted_launch(const float4 *boxes, const float *areas, const int *cls, c
     if (rc != SLN_OK) return rc;
     return launch_scan(mask, order2, nm, n2, W2, max_keep, numA, keep64, keep32, num_keep,
                        static_cast<unsigned char *>(fix) + nms_fix_bytes(n), skip, st);
+}
+
+int nms_sorted_batched_launch(int B, size_t stride, const float4 *boxes, const float *areas, int n, float thresh,
+                              int max_keep, unsigned long long *mask, int *keep32, int *num_keep, cudaStream_t st,
+                              void *stage, void *fix, void *sparse)
+{
+    if (B <= 0) return SLN_OK;
+    if (max_keep <= 0 || max_keep > n) max_keep = n;
+    if (n == 0) {
+        for (int b = 0; b < B; ++b) SLN_CUDA_OK(cudaMemsetAsync(seg_at(num_keep, stride, b), 0, sizeof(int), st));
+        return SLN_OK;
+    }
+    // the same eligibility test as launch_sparse: n and thresh are common to all problems
+    const bool sparse_ok = sparse != nullptr && n >= SP_MIN_N && n <= SP_MAX_N && thresh >= 0.05f;
+    if (sparse_ok) {
+        SLN_REQUIRE(B <= 65535, SLN_ERR_ARG, "nms: %d problems in one call", B);
+        SparseBufs sb;
+        sparse_carve(sparse, n, sb);
+        int CB, G;
+        float ct;
+        sparse_params(n, false, thresh, CB, G, ct);
+        const unsigned edge_cap = (unsigned)SP_EDGES_PER_BOX * (unsigned)n;
+        SLN_CUDA_OK(launch_chain(nms_bin_seg_kernel, dim3(SP_CLUSTER, B), dim3(SP_BIN_THREADS), 0, st, true, boxes, areas, n, G,
+                                 sb, stride));
+        // about the pair grid of one single-image call in all, at least one CTA per problem
+        int ctas = cdiv(n, SP_PAIR_WARPS);
+        const int cap = cdiv(SLN_SP_PAIR_CTAS_PER_SM * sm_count(), B);
+        if (ctas > cap) ctas = cap;
+        SLN_CUDA_OK(launch_chain(nms_pairs_seg_kernel, dim3(ctas, B), dim3(32 * SP_PAIR_WARPS), 0, st, true, boxes, areas, n,
+                                 thresh, ct, edge_cap, sb, stride));
+        const size_t smem = sparse_resolve_smem(n);
+        SLN_CUDA_OK(cudaFuncSetAttribute(nms_sparse_resolve_seg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        SLN_CUDA_OK(launch_chain(nms_sparse_resolve_seg_kernel, dim3(SP_CLUSTER, B), dim3(SP_RESOLVE_THREADS), smem, st, true, n,
+                                 max_keep, edge_cap, sb, keep32, num_keep, stride));
+    }
+    // dense fallback, per problem and guarded by that problem's status word: without a host read nobody knows which
+    // problems need it, so every problem gets the launches and those whose sparse pass succeeded leave at once
+    for (int b = 0; b < B; ++b) {
+        const int *skip = sparse_ok ? &seg_at(static_cast<SparseHdr *>(sparse), stride, b)->status : nullptr;
+        const int rc = nms_dense_launch(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, nullptr, n, thresh, max_keep,
+                                        seg_at(mask, stride, b), nullptr, seg_at(keep32, stride, b), seg_at(num_keep, stride, b),
+                                        st, stage ? seg_at(stage, stride, b) : nullptr, seg_at(fix, stride, b), skip);
+        if (rc != SLN_OK) return rc;
+    }
+    return SLN_OK;
 }
 
 }  // namespace sln

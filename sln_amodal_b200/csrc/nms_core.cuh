@@ -30,6 +30,22 @@ int nms_sorted_launch(const float4 *boxes, const float *areas, const int *cls, c
                       float thresh, int max_keep, unsigned long long *mask, int64_t *keep64, int *keep32,
                       int *num_keep, cudaStream_t st, void *stage, void *fix, void *sparse, bool sparse_only = false);
 
+// Batched calls (sln_proposal_layer_batched) lay out B copies of the single-image workspace, stride_bytes apart: the
+// array of image `seg` is the image-0 pointer moved by seg * stride_bytes.
+template <typename T>
+__host__ __device__ __forceinline__ T *seg_at(T *p, size_t stride_bytes, int seg)
+{
+    return (T *)((const unsigned char *)p + stride_bytes * (size_t)seg);
+}
+
+// B independent problems of n boxes each: boxes, areas, mask, keep32, num_keep, stage, fix and sparse are those of
+// problem 0, problem b's are seg_at(.., stride_bytes, b).  One launch per sparse stage for all B (a cluster per
+// problem); the dense kernels run per problem and leave at once where that problem's sparse pass succeeded.  Each
+// problem's keep list is exactly nms_sorted_launch's (no classes, order == nullptr).
+int nms_sorted_batched_launch(int B, size_t stride_bytes, const float4 *boxes, const float *areas, int n, float thresh,
+                              int max_keep, unsigned long long *mask, int *keep32, int *num_keep, cudaStream_t st,
+                              void *stage, void *fix, void *sparse);
+
 // Total order used everywhere a "descending score, stable" sort is needed:
 // larger key first; NaN sorts as the largest value (torch.sort's convention);
 // -0.0 == +0.0.  Ties are broken by ascending index.
@@ -47,5 +63,8 @@ __device__ __forceinline__ unsigned score_key(float s)
 // O(n^2) compares spread over the whole grid: a stable, deterministic sort for the
 // n <= ~16k this path sees, with no multi-pass radix machinery.
 int rank_sort_launch(const float *scores, int stride, const int *tie_ids, int n, int *rank, cudaStream_t st);
+// B segments of n elements each, segment z = blockIdx.z: scores / tie_ids / rank of segment z are seg_at(.., stride_bytes, z)
+int rank_sort_batched_launch(const float *scores, const int *tie_ids, int n, int B, size_t stride_bytes, int *rank,
+                             cudaStream_t st);
 
 }  // namespace sln

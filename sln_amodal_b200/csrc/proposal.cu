@@ -75,9 +75,8 @@ __device__ Pick cta_pick(const unsigned *__restrict__ hist, unsigned prev_prefix
 // hist = three histograms [3][SEL_BINS], zeroed once per call.  Pass P > 0 first picks the bin of pass P-1 (from the
 // state the previous launch left + that pass's histogram); CTA 0 publishes the new state for the next launch.
 template <int PASS>
-__global__ void __launch_bounds__(SEL_THREADS)
-select_hist_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
-                   unsigned *__restrict__ hist)
+__device__ __forceinline__ void select_hist_body(const float *probs, int A, int K, SelectState *state,
+                                                 unsigned *hist)
 {
     __shared__ unsigned s_hist[SEL_BINS];
     pdl_prologue();
@@ -106,6 +105,26 @@ select_hist_kernel(const float *__restrict__ probs, int A, int K, SelectState *_
     }
 }
 
+template <int PASS>
+__global__ void __launch_bounds__(SEL_THREADS)
+select_hist_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
+                   unsigned *__restrict__ hist)
+{
+    select_hist_body<PASS>(probs, A, K, state, hist);
+}
+
+// Batched forms (sln_proposal_layer_batched): image b = blockIdx.y reads probs + b*2A and works in the b-th copy of the
+// single-image workspace, ws_stride bytes further on (seg_at).  The bodies are the single-image kernels' own.
+
+template <int PASS>
+__global__ void __launch_bounds__(SEL_THREADS)
+select_hist_seg_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
+                       unsigned *__restrict__ hist, size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    select_hist_body<PASS>(probs + 2 * (size_t)A * b, A, K, seg_at(state, ws_stride, b), seg_at(hist, ws_stride, b));
+}
+
 // Each CTA owns a contiguous slice of the anchors so that "ordered" means index order.
 __device__ __forceinline__ void slice_of(int A, int &lo, int &hi)
 {
@@ -114,9 +133,9 @@ __device__ __forceinline__ void slice_of(int A, int &lo, int &hi)
     hi = min(A, lo + per);
 }
 
-__global__ void __launch_bounds__(SEL_THREADS)
-select_count_eq_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
-                       const unsigned *__restrict__ hist, int *__restrict__ blk_eq)
+__device__ __forceinline__ void select_count_eq_body(const float *probs, int A, int K,
+                                                     SelectState *state, const unsigned *hist,
+                                                     int *blk_eq)
 {
     __shared__ int s_cnt;
     pdl_prologue();
@@ -142,9 +161,24 @@ select_count_eq_kernel(const float *__restrict__ probs, int A, int K, SelectStat
 }
 
 __global__ void __launch_bounds__(SEL_THREADS)
-select_compact_kernel(const float *__restrict__ probs, int A, SelectState *__restrict__ state,
-                      const int *__restrict__ blk_eq, float *__restrict__ cand_score,
-                      int *__restrict__ cand_idx)
+select_count_eq_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
+                       const unsigned *__restrict__ hist, int *__restrict__ blk_eq)
+{
+    select_count_eq_body(probs, A, K, state, hist, blk_eq);
+}
+
+__global__ void __launch_bounds__(SEL_THREADS)
+select_count_eq_seg_kernel(const float *__restrict__ probs, int A, int K, SelectState *__restrict__ state,
+                           const unsigned *__restrict__ hist, int *__restrict__ blk_eq, size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    select_count_eq_body(probs + 2 * (size_t)A * b, A, K, seg_at(state, ws_stride, b), seg_at(hist, ws_stride, b),
+                         seg_at(blk_eq, ws_stride, b));
+}
+
+__device__ __forceinline__ void select_compact_body(const float *probs, int A, SelectState *state,
+                                                    const int *blk_eq, float *cand_score,
+                                                    int *cand_idx)
 {
     __shared__ int s_warp[SEL_THREADS / 32];
     __shared__ int s_base;
@@ -207,13 +241,44 @@ select_compact_kernel(const float *__restrict__ probs, int A, SelectState *__res
     }
 }
 
-__global__ void select_all_kernel(const float *__restrict__ probs, int A, float *__restrict__ cand_score,
-                                  int *__restrict__ cand_idx)
+__global__ void __launch_bounds__(SEL_THREADS)
+select_compact_kernel(const float *__restrict__ probs, int A, SelectState *__restrict__ state,
+                      const int *__restrict__ blk_eq, float *__restrict__ cand_score,
+                      int *__restrict__ cand_idx)
+{
+    select_compact_body(probs, A, state, blk_eq, cand_score, cand_idx);
+}
+
+__global__ void __launch_bounds__(SEL_THREADS)
+select_compact_seg_kernel(const float *__restrict__ probs, int A, SelectState *__restrict__ state,
+                          const int *__restrict__ blk_eq, float *__restrict__ cand_score, int *__restrict__ cand_idx,
+                          size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    select_compact_body(probs + 2 * (size_t)A * b, A, seg_at(state, ws_stride, b), seg_at(blk_eq, ws_stride, b),
+                        seg_at(cand_score, ws_stride, b), seg_at(cand_idx, ws_stride, b));
+}
+
+__device__ __forceinline__ void select_all_body(const float *probs, int A, float *cand_score,
+                                                int *cand_idx)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= A) return;
     cand_score[i] = probs[2 * (size_t)i + 1];
     cand_idx[i] = i;
+}
+
+__global__ void select_all_kernel(const float *__restrict__ probs, int A, float *__restrict__ cand_score,
+                                  int *__restrict__ cand_idx)
+{
+    select_all_body(probs, A, cand_score, cand_idx);
+}
+
+__global__ void select_all_seg_kernel(const float *__restrict__ probs, int A, float *__restrict__ cand_score,
+                                      int *__restrict__ cand_idx, size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    select_all_body(probs + 2 * (size_t)A * b, A, seg_at(cand_score, ws_stride, b), seg_at(cand_idx, ws_stride, b));
 }
 
 __device__ __forceinline__ float clampf_nan(float v, float lo, float hi)
@@ -224,10 +289,10 @@ __device__ __forceinline__ float clampf_nan(float v, float lo, float hi)
 struct Float4Std { float s0, s1, s2, s3; };
 
 // Decode candidate j (anchor cand_idx[j]) and write it at its visiting position rank[j].
-__global__ void proposal_decode_kernel(const float *__restrict__ anchors, const float *__restrict__ deltas,
-                                       const int *__restrict__ cand_idx, const int *__restrict__ rank, int K,
-                                       Float4Std sd, float img_h, float img_w, float4 *__restrict__ boxes,
-                                       float *__restrict__ areas)
+__device__ __forceinline__ void proposal_decode_body(const float *anchors, const float *deltas,
+                                                     const int *cand_idx, const int *rank, int K,
+                                                     Float4Std sd, float img_h, float img_w, float4 *boxes,
+                                                     float *areas)
 {
     pdl_prologue();
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -257,9 +322,28 @@ __global__ void proposal_decode_kernel(const float *__restrict__ anchors, const 
     areas[p] = __fmul_rn(__fadd_rn(__fsub_rn(x2, x1), 1.f), __fadd_rn(__fsub_rn(y2, y1), 1.f));   // pth_nms.py:16
 }
 
-__global__ void proposal_finalize_kernel(const float4 *__restrict__ boxes, const int *__restrict__ keep,
-                                         const int *__restrict__ num_keep, int proposal_count, float img_h,
-                                         float img_w, float4 *__restrict__ out, int *__restrict__ num_out)
+__global__ void proposal_decode_kernel(const float *__restrict__ anchors, const float *__restrict__ deltas,
+                                       const int *__restrict__ cand_idx, const int *__restrict__ rank, int K,
+                                       Float4Std sd, float img_h, float img_w, float4 *__restrict__ boxes,
+                                       float *__restrict__ areas)
+{
+    proposal_decode_body(anchors, deltas, cand_idx, rank, K, sd, img_h, img_w, boxes, areas);
+}
+
+// anchors are shared by all images; deltas of image b start at b*4A
+__global__ void proposal_decode_seg_kernel(const float *__restrict__ anchors, const float *__restrict__ deltas, int A,
+                                           const int *__restrict__ cand_idx, const int *__restrict__ rank, int K,
+                                           Float4Std sd, float img_h, float img_w, float4 *__restrict__ boxes,
+                                           float *__restrict__ areas, size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    proposal_decode_body(anchors, deltas + 4 * (size_t)A * b, seg_at(cand_idx, ws_stride, b), seg_at(rank, ws_stride, b), K,
+                         sd, img_h, img_w, seg_at(boxes, ws_stride, b), seg_at(areas, ws_stride, b));
+}
+
+__device__ __forceinline__ void proposal_finalize_body(const float4 *boxes, const int *keep,
+                                                       const int *num_keep, int proposal_count, float img_h,
+                                                       float img_w, float4 *out, int *num_out)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const int nk = min(*num_keep, proposal_count);
@@ -271,6 +355,23 @@ __global__ void proposal_finalize_kernel(const float4 *__restrict__ boxes, const
         v = make_float4(__fdiv_rn(b.x, img_h), __fdiv_rn(b.y, img_w), __fdiv_rn(b.z, img_h), __fdiv_rn(b.w, img_w));
     }
     out[i] = v;
+}
+
+__global__ void proposal_finalize_kernel(const float4 *__restrict__ boxes, const int *__restrict__ keep,
+                                         const int *__restrict__ num_keep, int proposal_count, float img_h,
+                                         float img_w, float4 *__restrict__ out, int *__restrict__ num_out)
+{
+    proposal_finalize_body(boxes, keep, num_keep, proposal_count, img_h, img_w, out, num_out);
+}
+
+__global__ void proposal_finalize_seg_kernel(const float4 *__restrict__ boxes, const int *__restrict__ keep,
+                                             const int *__restrict__ num_keep, int proposal_count, float img_h,
+                                             float img_w, float4 *__restrict__ out, int *__restrict__ num_out,
+                                             size_t ws_stride)
+{
+    const int b = blockIdx.y;
+    proposal_finalize_body(seg_at(boxes, ws_stride, b), seg_at(keep, ws_stride, b), seg_at(num_keep, ws_stride, b),
+                           proposal_count, img_h, img_w, out + (size_t)proposal_count * b, num_out + b);
 }
 
 struct ProposalBuffers {
@@ -379,5 +480,83 @@ extern "C" int sln_proposal_layer(const float *probs, const float *deltas, const
     proposal_finalize_kernel<<<cdiv(proposal_count, 128), 128, 0, st>>>(
         nb.boxes, b.keep, b.num_keep, proposal_count, img_h, img_w, reinterpret_cast<float4 *>(out_boxes), num_out);
     SLN_LAUNCH_OK("proposal_finalize_kernel");
+    return SLN_OK;
+}
+
+// ---------------------------------------------------------------------------
+// B images per call.  The workspace is B copies of the single-image one, ws_stride = proposal_ws_bytes(K) apart (a
+// multiple of 256, so every array keeps its alignment); every stage is one launch over all images, the image on a grid
+// dimension, except the dense NMS fallback, which runs per image behind that image's sparse status word
+// (nms_sorted_batched_launch).  Each image goes through the single-image kernels' bodies with the single-image
+// parameters (K, thresholds, grid shapes per image aside), so its result is sln_proposal_layer's bit for bit.
+// ---------------------------------------------------------------------------
+extern "C" size_t sln_proposal_batched_workspace_bytes(int B, int A, int pre_nms_limit)
+{
+    if (B < 0 || A < 0 || pre_nms_limit < 0) return 0;
+    return (size_t)B * proposal_ws_bytes(A < pre_nms_limit ? A : pre_nms_limit);
+}
+
+extern "C" int sln_proposal_layer_batched(const float *probs, const float *deltas, const float *anchors, int B, int A,
+                                          int pre_nms_limit, int proposal_count, float nms_thresh,
+                                          const float *std_dev_host, float img_h, float img_w, float *out_boxes,
+                                          int *num_out, void *workspace, size_t workspace_bytes, void *stream)
+{
+    SLN_REQUIRE(B >= 0 && A >= 0 && pre_nms_limit >= 0 && proposal_count >= 0, SLN_ERR_ARG, "negative size");
+    SLN_REQUIRE(B <= 65535, SLN_ERR_ARG, "B=%d images in one call (at most 65535)", B);
+    if (B == 0) return SLN_OK;
+    SLN_REQUIRE(num_out && std_dev_host, SLN_ERR_ARG, "null pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int K = A < pre_nms_limit ? A : pre_nms_limit;
+    if (proposal_count > 0) SLN_REQUIRE(out_boxes, SLN_ERR_ARG, "null out_boxes");
+    if (K == 0 || proposal_count == 0) {
+        SLN_CUDA_OK(cudaMemsetAsync(num_out, 0, sizeof(int) * (size_t)B, st));
+        if (proposal_count > 0)
+            SLN_CUDA_OK(cudaMemsetAsync(out_boxes, 0, sizeof(float) * 4 * (size_t)proposal_count * B, st));
+        return SLN_OK;
+    }
+    SLN_REQUIRE(probs && deltas && anchors, SLN_ERR_ARG, "null pointer");
+    SLN_REQUIRE((reinterpret_cast<uintptr_t>(deltas) & 15u) == 0 && (reinterpret_cast<uintptr_t>(anchors) & 15u) == 0 &&
+                    (reinterpret_cast<uintptr_t>(out_boxes) & 15u) == 0,
+                SLN_ERR_LAYOUT, "deltas / anchors / out_boxes must be 16-byte aligned");
+    const size_t S = proposal_ws_bytes(K);
+    SLN_REQUIRE(workspace && workspace_bytes >= S * B, SLN_ERR_WORKSPACE,
+                "batched proposal workspace: need %zu bytes, got %zu", S * B, workspace_bytes);
+    ProposalBuffers b;
+    proposal_carve(workspace, K, b);
+    NmsBuffers nb;
+    nms_carve(b.nms, K, nb);
+
+    if (K == A) {
+        select_all_seg_kernel<<<dim3(cdiv(A, 256), B), 256, 0, st>>>(probs, A, b.cand_score, b.cand_idx, S);
+        SLN_LAUNCH_OK("select_all_seg_kernel");
+    } else {
+        // about the grid of one single-image call in all: fewer CTAs per image as B grows
+        int nblk = cdiv(4 * sm_count(), B);
+        if (nblk > SEL_MAX_BLOCKS) nblk = SEL_MAX_BLOCKS;
+        if (nblk > cdiv(A, SEL_THREADS)) nblk = cdiv(A, SEL_THREADS);
+        // every image's three histograms: one strided memset
+        SLN_CUDA_OK(cudaMemset2DAsync(b.hist, S, 0, sizeof(unsigned) * 3 * SEL_BINS, B, st));
+        const dim3 grid(nblk, B);
+        select_hist_seg_kernel<0><<<grid, SEL_THREADS, 0, st>>>(probs, A, K, b.state, b.hist, S);
+        SLN_LAUNCH_OK("select_hist_seg_kernel");
+        SLN_CUDA_OK(launch_chain(select_hist_seg_kernel<1>, grid, dim3(SEL_THREADS), 0, st, true, probs, A, K, b.state, b.hist, S));
+        SLN_CUDA_OK(launch_chain(select_hist_seg_kernel<2>, grid, dim3(SEL_THREADS), 0, st, true, probs, A, K, b.state, b.hist, S));
+        SLN_CUDA_OK(launch_chain(select_count_eq_seg_kernel, grid, dim3(SEL_THREADS), 0, st, true, probs, A, K, b.state,
+                                 (const unsigned *)b.hist, b.blk_eq, S));
+        SLN_CUDA_OK(launch_chain(select_compact_seg_kernel, grid, dim3(SEL_THREADS), 0, st, true, probs, A, b.state,
+                                 (const int *)b.blk_eq, b.cand_score, b.cand_idx, S));
+    }
+    SLN_CUDA_OK(cudaMemset2DAsync(nb.rank, S, 0, sizeof(int) * (size_t)K, B, st));
+    int rc = rank_sort_batched_launch(b.cand_score, b.cand_idx, K, B, S, nb.rank, st);
+    if (rc != SLN_OK) return rc;
+    Float4Std sd{std_dev_host[0], std_dev_host[1], std_dev_host[2], std_dev_host[3]};
+    SLN_CUDA_OK(launch_chain(proposal_decode_seg_kernel, dim3(cdiv(K, 128), B), dim3(128), 0, st, true, anchors, deltas, A,
+                             (const int *)b.cand_idx, (const int *)nb.rank, K, sd, img_h, img_w, nb.boxes, nb.areas, S));
+    rc = nms_sorted_batched_launch(B, S, nb.boxes, nb.areas, K, nms_thresh, proposal_count, nb.mask, b.keep, b.num_keep, st,
+                                   nb.stage, nb.fix, nb.sparse);
+    if (rc != SLN_OK) return rc;
+    proposal_finalize_seg_kernel<<<dim3(cdiv(proposal_count, 128), B), 128, 0, st>>>(
+        nb.boxes, b.keep, b.num_keep, proposal_count, img_h, img_w, reinterpret_cast<float4 *>(out_boxes), num_out, S);
+    SLN_LAUNCH_OK("proposal_finalize_seg_kernel");
     return SLN_OK;
 }

@@ -555,6 +555,32 @@ def refine_topk_device(dets, class_ids, max_keep=100):
     return result, keep
 
 
+def refine_topk_batched_device(dets, class_ids, max_keep=100):
+    """refine_topk_device for B images in one launch (sln_refine_topk_batched).  dets [B,N,5], class_ids int32 [B,N]
+    (sln_refine_decode's outputs of the flattened [B*N] rows, viewed per image).  Returns (result f32 [B,max_keep,6],
+    keep int64 [B,max_keep] row indices within the image, num_det int32 [B] = min(max_keep, kept rows of the image));
+    only the first num_det[b] rows of image b are written."""
+    _require_cuda(dets, "dets")
+    _require_cuda(class_ids, "class_ids")
+    if dets.dim() != 3 or dets.shape[2] != 5:
+        raise _lib.SlnError(f"dets must be [B,N,5], got {tuple(dets.shape)}")
+    B, N = int(dets.shape[0]), int(dets.shape[1])
+    if tuple(class_ids.shape) != (B, N):
+        raise _lib.SlnError(f"class_ids {tuple(class_ids.shape)} disagrees with dets {tuple(dets.shape)}")
+    if int(max_keep) < 0:
+        raise _lib.SlnError(f"max_keep must be >= 0, got {max_keep}")
+    dets, class_ids = _f32c(dets), _i32c(class_ids)
+    result = torch.empty((B, int(max_keep), 6), dtype=torch.float32, device=dets.device)
+    keep = torch.empty((B, int(max_keep)), dtype=torch.int64, device=dets.device)
+    num_det = torch.empty(B, dtype=torch.int32, device=dets.device)
+    if B:
+        with torch.cuda.device(dets.device):
+            check(lib().sln_refine_topk_batched(ptr(dets), ptr(class_ids), B, N, int(max_keep), ptr(result), ptr(keep),
+                                                ptr(num_det), stream_ptr()), "sln_refine_topk_batched")
+        _lib.count_launches(2 if N and max_keep else 1)
+    return result, keep, num_det
+
+
 def bbox_overlaps_device(boxes1, boxes2, matrix=True, reduce=False):
     """IoU of boxes1 [N,4] against boxes2 [G,4] (include/sln_b200.h, sln_bbox_overlaps).
     Returns the [N,G] matrix, or (matrix | None, iou_max [N], argmax int32 [N]) with reduce=True."""
@@ -698,6 +724,51 @@ def proposal_device(probs, deltas, anchors, proposal_count, nms_threshold, std_d
     if A and proposal_count:
         _lib.count_launches(14 if A > pre_nms_limit else 6)
     return out[:proposal_count], num
+
+
+def _proposal_batched_launches(B, A, K, nms_threshold):
+    """Launches of one sln_proposal_layer_batched call with K = min(A, pre_nms_limit) > 0: the shared stages once, the
+    dense NMS fallback (nms.cu: mask + scan, the fixed-point resolve from 160 words, two stages from 16384 boxes) once
+    per image."""
+    shared = (6 if K < A else 1) + 3                     # histogram memset + 5 select kernels | select_all; rank memset, rank, decode
+    shared += 3 if 65 <= K <= 65535 and nms_threshold >= 0.05 else 0     # bin, pairs, resolve
+    shared += 1                                          # finalize
+    if K < 16384:
+        dense = 2 + (((K + 63) // 64) >= 160)
+    else:
+        dense = 2 + 3 + 2 + (((K - 1024 + 63) // 64) >= 160)
+    return shared + B * dense
+
+
+def proposal_batched_device(probs, deltas, anchors, proposal_count, nms_threshold, std_dev, image_hw, pre_nms_limit=6000):
+    """B images in one call (sln_proposal_layer_batched).  probs [B,A,2], deltas [B,A,4], anchors [A,4] (pixels, shared).
+    Returns (boxes f32 [B,proposal_count,4] normalised, zero padded; num int32 [B]) on the device; image b's rows are
+    exactly proposal_device's for that image alone."""
+    for t, nm in ((probs, "probs"), (deltas, "deltas"), (anchors, "anchors")):
+        _require_cuda(t, nm)
+    if probs.dim() != 3 or probs.shape[2] != 2:
+        raise _lib.SlnError(f"probs must be [B,A,2], got {tuple(probs.shape)}")
+    B, A = int(probs.shape[0]), int(probs.shape[1])
+    if tuple(deltas.shape) != (B, A, 4):
+        raise _lib.SlnError(f"deltas {tuple(deltas.shape)} disagrees with probs {tuple(probs.shape)}")
+    if tuple(anchors.shape) != (A, 4):
+        raise _lib.SlnError(f"anchors {tuple(anchors.shape)} disagree with A = {A}")
+    if int(proposal_count) < 0 or int(pre_nms_limit) < 0:
+        raise _lib.SlnError(f"proposal_count ({proposal_count}) and pre_nms_limit ({pre_nms_limit}) must be >= 0")
+    probs, deltas, anchors = _f32c(probs), _f32c(deltas), _f32c(anchors)
+    R = int(proposal_count)
+    out = torch.empty((B, max(R, 1), 4), dtype=torch.float32, device=probs.device)
+    num = torch.empty(B, dtype=torch.int32, device=probs.device)
+    sd = (C.c_float * 4)(*[float(v) for v in std_dev])
+    with torch.cuda.device(probs.device):
+        ws = _workspace(lib().sln_proposal_batched_workspace_bytes(B, A, int(pre_nms_limit)), probs.device)
+        check(lib().sln_proposal_layer_batched(ptr(probs), ptr(deltas), ptr(anchors), B, A, int(pre_nms_limit), R,
+                                               float(nms_threshold), sd, float(image_hw[0]), float(image_hw[1]), ptr(out),
+                                               ptr(num), ptr(ws), ws.numel(), stream_ptr()), "sln_proposal_layer_batched")
+    K = min(A, int(pre_nms_limit))
+    if B:
+        _lib.count_launches(_proposal_batched_launches(B, A, K, float(nms_threshold)) if K and R else 1 + (R > 0))
+    return out[:, :R], num
 
 
 # ---------------------------------------------------------------------------

@@ -137,3 +137,60 @@ class MultiHeadGraph:
     def replay(self):
         self.graph.replay()
         return self.out
+
+
+class BatchedHeadGraph(HeadGraph):
+    """HeadGraph's steps for B images at once, one launch per stage for all of them (the per-image dense NMS fallback of
+    sln_proposal_layer_batched aside), captured into one graph.
+
+    feature_maps: per level [B,C,H_l,W_l]; rpn_probs [B,A,2]; rpn_bbox [B,A,4]; anchors [A,4] shared.  classifier(pooled
+    [B*R,C,p,p], rois [B*R,4]) -> (probs [B*R,K], deltas [B*R,K,4]), or a pair of static tensors of those shapes (or
+    [B,R,K] / [B,R,K,4]).  Outputs are [B, ...]: rois [B,R,4] and detections [B,D,6] zero beyond num_rois[b] /
+    num_detections[b] (keep too), pooled [B,R,C,p,p], mask_pooled [B,D,C,mp,mp].  Below the counts every image's outputs
+    are bit-identical to its own HeadGraph's: the crops, the level rule and the refine front are per row, and the
+    proposals and the top-k are ranked within the image."""
+
+    def __init__(self, anchors, config, feature_maps, rpn_probs, rpn_bbox, classifier, proposal_count=1000,
+                 max_detections=100, window=None, capture=True):
+        self.B = int(rpn_probs.shape[0])
+        super().__init__(anchors, config, feature_maps, rpn_probs, rpn_bbox, classifier, proposal_count=proposal_count,
+                         max_detections=max_detections, window=window, capture=capture)
+
+    def _steps(self):
+        cfg, B, R, D = self.cfg, self.B, self.R, self.D
+        rois, num = ops.proposal_batched_device(self.rpn_probs, self.rpn_bbox, self.anchors, R, float(cfg.RPN_NMS_THRESHOLD),
+                                                self.std_rpn, self.image_hw, pre_nms_limit=PRE_NMS_LIMIT)
+        if self._bg is None:                       # constants: made in the eager warm-up pass (host -> device copies cannot be captured)
+            h, w = self.image_hw
+            self._norm = torch.tensor([h, w, h, w], dtype=torch.float32, device=self.dev)
+            self._ar_r = torch.arange(R, device=self.dev, dtype=torch.int32)
+            self._ar_d = torch.arange(D, device=self.dev, dtype=torch.int32)
+            img = torch.arange(B, device=self.dev, dtype=torch.int32)
+            self._box_ind_r = img.repeat_interleave(R)
+            self._box_ind_d = img.repeat_interleave(D)
+        flat = rois.reshape(B * R, 4)
+        level = ops.roi_levels_device(flat, self.image_hw)
+        pooled = ops.pyramid_crop_forward(self.maps, flat, self._box_ind_r, level, int(cfg.POOL_SIZE), int(cfg.POOL_SIZE), 0.0)
+        if callable(self.classifier):
+            probs, deltas = self.classifier(pooled, flat)
+        else:
+            probs, deltas = self.classifier
+        probs = probs.reshape(B * R, probs.shape[-1])
+        deltas = deltas.reshape(B * R, deltas.shape[-2], 4)
+        if self._bg is None:
+            self._bg = torch.zeros_like(probs[:1])
+            self._bg[0, 0] = 1.0
+        # rows beyond each image's proposal count get the background class, as in HeadGraph
+        valid = (self._ar_r[None, :] < num[:, None]).reshape(B * R)
+        probs = torch.where(valid[:, None], probs, self._bg)
+        dets, _, class_ids, _ = ops.refine_decode_device(flat, probs, deltas, self.std_rpn, self.image_hw, self.window, 0.0)
+        det, keep, num_det = ops.refine_topk_batched_device(dets.view(B, R, 5), class_ids.view(B, R), D)
+        rows = self._ar_d[None, :] < num_det[:, None]
+        det = torch.where(rows[..., None], det, torch.zeros_like(det))       # rows beyond num_det were never written
+        keep = torch.where(rows, keep, torch.zeros_like(keep))
+        boxes = (det[..., :4] / self._norm).reshape(B * D, 4)
+        lvl_d = ops.roi_levels_device(boxes, self.image_hw)
+        mp = int(cfg.MASK_POOL_SIZE)
+        mask_in = ops.pyramid_crop_forward(self.maps, boxes, self._box_ind_d, lvl_d, mp, mp, 0.0)
+        return {"rois": rois, "num_rois": num, "pooled": pooled.unflatten(0, (B, R)), "detections": det, "keep": keep,
+                "num_detections": num_det, "mask_pooled": mask_in.unflatten(0, (B, D))}

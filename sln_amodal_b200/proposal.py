@@ -30,6 +30,16 @@ def proposal_layer(inputs, proposal_count, nms_threshold, anchors, config=None):
     return boxes[:k].unsqueeze(0)
 
 
+def proposal_layer_batched(inputs, proposal_count, nms_threshold, anchors, config=None):
+    """proposal_layer for B images in one call: inputs = [rpn_probs [B,A,2], rpn_bbox [B,A,4]] (not modified), anchors
+    [A,4] pixels shared by the images.  Returns (rois [B,proposal_count,4] normalised, zero padded beyond num[b]; num
+    int32 [B]) as device tensors, no host sync; rois[b, :num[b]] is proposal_layer's result for image b alone."""
+    std_dev = np.reshape(config.RPN_BBOX_STD_DEV, [4]) if config is not None else (0.1, 0.1, 0.2, 0.2)
+    height, width = (config.IMAGE_SHAPE[:2] if config is not None else (1024, 1024))
+    return ops.proposal_batched_device(inputs[0], inputs[1], anchors, proposal_count, nms_threshold, std_dev,
+                                       (height, width), pre_nms_limit=PRE_NMS_LIMIT)
+
+
 def proposal_layer_padded(rpn_probs, rpn_bbox, anchors, proposal_count, nms_threshold,
                           std_dev=(0.1, 0.1, 0.2, 0.2), image_hw=(1024, 1024)):
     """Sync-free variant for batched / graph-captured use: returns (boxes [proposal_count,4]
