@@ -193,6 +193,17 @@ SLN_API int sln_nms(const float *dets, const int *class_ids, int n, float thresh
 SLN_API int sln_nms_ex(const float *dets, const int *class_ids, int n, float thresh, int max_keep, int flags,
                int64_t *keep, int *num_keep, int *path_out, void *workspace, size_t workspace_bytes,
                void *stream);
+/* B independent problems of n boxes each in one call: dets f32 [B,n,5], class_ids i32 [B,n] (or NULL: class-agnostic).
+ * keep i64 [B,mk] with mk = max_keep when 0 < max_keep <= n, else n; num_keep device i32 [B]; path_out device i32 [B]
+ * (may be NULL).  For every b, keep[b, :num_keep[b]], num_keep[b] and path_out[b] are bit-identical to sln_nms_ex on
+ * problem b alone with the same class_ids, thresh, max_keep and flags.  Each sparse stage is one launch for all B
+ * problems (one cluster per problem); the dense pipeline is launched per problem and returns at once where that
+ * problem's sparse pass succeeded.  No host sync, graph capturable.  SLN_NMS_DENSE_ONLY is honoured;
+ * SLN_NMS_SPARSE_ONLY is rejected with SLN_ERR_ARG (it needs a host retry).  B == 0 and n == 0 are valid.        */
+SLN_API size_t sln_nms_batched_workspace_bytes(int B, int n);
+SLN_API int sln_nms_batched(const float *dets, const int *class_ids, int B, int n, float thresh, int max_keep, int flags,
+                    int64_t *keep, int *num_keep, int *path_out, void *workspace, size_t workspace_bytes,
+                    void *stream);
 
 /* ---- refine_detections, elementwise front --------------------------------- *
  * Replaces the ~25 small torch kernels at the top of refine_detections (modal/Functions.py:453-493): per ROI the
@@ -223,6 +234,18 @@ SLN_API int sln_refine_topk(const float *dets, const int *class_ids, int N, int 
  * later rows are not touched.  No host sync.                                                                   */
 SLN_API int sln_refine_topk_batched(const float *dets, const int *class_ids, int B, int N, int max_keep, float *result,
                             int64_t *keep, int *num_det, void *stream);
+
+/* ---- refine_detections, per-class NMS branch, B images ------------------------- *
+ * The step after sln_nms_batched (run on sln_refine_decode's dets f32 [B,N,5] and cls_nms i32 [B,N] with
+ * DETECTION_NMS_THRESHOLD and max_keep = D): nms_keep i64 [B,nms_max_keep], nms_num_keep device i32 [B] are its outputs.
+ * Writes result f32 [B,D,6] = (y1,x1,y2,x2,class_id,score) with class_id from class_ids i32 [B,N], keep i64 [B,D] (row
+ * indices within the image) and num_det device i32 [B] = min(D, survivors with a finite score); rows at and beyond
+ * num_det[b] are zero.  Rows below num_det[b] are the first D rows of the single-image branch (sln_nms_ex on that image
+ * without max_keep, filtered rows dropped): greedy NMS's first D survivors do not depend on where it stops.  One launch,
+ * no host sync.                                                                                                     */
+SLN_API int sln_refine_nms_emit_batched(const float *dets, const int *class_ids, int B, int N, const int64_t *nms_keep,
+                                const int *nms_num_keep, int nms_max_keep, int D, float *result, int64_t *keep,
+                                int *num_det, void *stream);
 
 /* ---- detection targets (SURVEY 8(f)-1) -------------------------------------- *
  * sln_bbox_overlaps replaces bbox_overlaps (modal/Functions.py:184-218): IoU of boxes1 [N,4] against boxes2 [G,4]

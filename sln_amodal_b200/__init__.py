@@ -12,7 +12,8 @@ from .nms import batched_nms, nms, pth_nms  # noqa: F401
 from .proposal import proposal_layer, proposal_layer_batched, proposal_layer_padded  # noqa: F401
 from .pyramid import pyramid_roi_align, pyramid_roi_align_batched, pyramid_roi_align_image  # noqa: F401
 from .semdist import decode_layers, load_layer2, sem_dist_targets  # noqa: F401
-from .detection import refine_detections  # noqa: F401
+from .detection import refine_detections, refine_detections_batched  # noqa: F401
+from .ops import nms_batched_device as nms_batched  # noqa: F401
 from .targets import (bbox_overlaps, box_refinement, build_rpn_targets, detection_target_layer, extract_bboxes,  # noqa: F401
                       resize_image, resize_image_device, resize_layer, resize_layer_device, zoom_index_map)
 from .rle import encode as rle_encode  # noqa: F401

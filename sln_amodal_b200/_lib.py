@@ -50,9 +50,12 @@ PROTOTYPES = {
     "sln_nms_workspace_bytes": (_sz, [_i]),
     "sln_nms": (_i, [_vp, _vp, _i, _f, _i, _vp, _vp, _vp, _sz, _vp]),
     "sln_nms_ex": (_i, [_vp, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "sln_nms_batched_workspace_bytes": (_sz, [_i, _i]),
+    "sln_nms_batched": (_i, [_vp, _vp, _i, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "sln_refine_decode": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(_f), _f, _f, C.POINTER(_f), _f, _vp, _vp, _vp, _vp, _vp]),
     "sln_refine_topk": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
     "sln_refine_topk_batched": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "sln_refine_nms_emit_batched": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "sln_bbox_overlaps": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp]),
     "sln_box_refinement": (_i, [_vp, _vp, _i, C.POINTER(_f), _vp, _vp]),
     "sln_mask_targets": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),

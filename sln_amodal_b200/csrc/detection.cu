@@ -198,6 +198,70 @@ extern "C" int sln_refine_topk_batched(const float *dets, const int *class_ids, 
 }
 
 // ---------------------------------------------------------------------------
+// refine_detections with per-class NMS (USE_NMS = True), B images: the step after sln_nms_batched, which ran on
+// sln_refine_decode's dets / cls_nms with max_keep = D.  Filtered rows carry score -inf and a class of their own, so the
+// NMS never suppresses them and visits them last: the rows with a finite score are a prefix of every image's keep list,
+// and its length is min(D, survivors).  Stopping the greedy NMS after D survivors does not change the first D, so this
+// equals the first D rows of the single-image path (_refine_detections_fused), which runs the NMS to the end.
+// One CTA per image (blockIdx.y), rows strided over its threads; rows at and beyond the count are zero.
+namespace sln {
+
+constexpr int EMIT_THREADS = 256;
+
+__global__ void __launch_bounds__(EMIT_THREADS)
+refine_nms_emit_seg_kernel(const float *__restrict__ dets, const int *__restrict__ class_ids, int N,
+                           const long long *__restrict__ nms_keep, const int *__restrict__ nms_num, int nms_stride, int D,
+                           float *__restrict__ result, long long *__restrict__ keep, int *__restrict__ num_det)
+{
+    const size_t b = blockIdx.y;
+    const int nk = min(__ldg(nms_num + b), nms_stride);
+    int count = 0;
+    for (int r0 = 0; r0 < D; r0 += EMIT_THREADS) {
+        const int r = r0 + threadIdx.x;
+        long long idx = 0;
+        float s = -INFINITY;
+        if (r < D && r < nk) {
+            idx = __ldg(nms_keep + b * (size_t)nms_stride + r);
+            s = __ldg(dets + 5 * ((size_t)N * b + (size_t)idx) + 4);
+        }
+        const bool valid = s > -INFINITY;
+        if (r < D) {
+            float *o = result + 6 * ((size_t)D * b + r);
+            if (valid) {
+                const float *d = dets + 5 * ((size_t)N * b + (size_t)idx);
+                o[0] = d[0]; o[1] = d[1]; o[2] = d[2]; o[3] = d[3];
+                o[4] = (float)__ldg(class_ids + (size_t)N * b + (size_t)idx);
+                o[5] = s;
+            } else {
+                o[0] = o[1] = o[2] = o[3] = o[4] = o[5] = 0.f;
+            }
+            keep[(size_t)D * b + r] = valid ? idx : 0;
+        }
+        count += __syncthreads_count(valid);
+    }
+    if (threadIdx.x == 0) num_det[b] = count;
+}
+
+}  // namespace sln
+
+extern "C" int sln_refine_nms_emit_batched(const float *dets, const int *class_ids, int B, int N, const int64_t *nms_keep,
+                                           const int *nms_num_keep, int nms_max_keep, int D, float *result, int64_t *keep,
+                                           int *num_det, void *stream)
+{
+    SLN_REQUIRE(B >= 0 && N >= 0 && nms_max_keep >= 0 && D >= 0, SLN_ERR_ARG, "negative size");
+    SLN_REQUIRE(B <= 65535, SLN_ERR_ARG, "B=%d images in one call (at most 65535)", B);
+    if (B == 0) return SLN_OK;
+    SLN_REQUIRE(num_det && nms_num_keep, SLN_ERR_ARG, "null pointer");
+    SLN_REQUIRE(D == 0 || (result && keep), SLN_ERR_ARG, "null pointer");
+    SLN_REQUIRE(N == 0 || nms_max_keep == 0 || (dets && class_ids && nms_keep), SLN_ERR_ARG, "null pointer");
+    sln::refine_nms_emit_seg_kernel<<<dim3(1, B), sln::EMIT_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
+        dets, class_ids, N, reinterpret_cast<const long long *>(nms_keep), nms_num_keep, nms_max_keep, D, result,
+        reinterpret_cast<long long *>(keep), num_det);
+    SLN_LAUNCH_OK("refine_nms_emit_seg_kernel");
+    return SLN_OK;
+}
+
+// ---------------------------------------------------------------------------
 // SURVEY 8(f)-1: detection targets -- IoU matching and box refinement
 // ---------------------------------------------------------------------------
 // bbox_overlaps (modal/Functions.py:184-218): IoU of every box of set 1 against every box of set 2, no "+1"

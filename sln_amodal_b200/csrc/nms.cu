@@ -172,13 +172,29 @@ rank_kernel(const float *__restrict__ scores, int stride, const int *__restrict_
     rank_body(scores, stride, tie_ids, n, rank, ga);
 }
 
-// segment z = blockIdx.z: contiguous scores (stride 1), explicit tie ids, no gather
+// segment z = blockIdx.z.  Inputs move by in_stride bytes per segment (scores, tie ids, the gather's dets) and by
+// cls_stride (the gather's class ids); rank and the gather's outputs and tickets by ws_stride.  Null pointers stay null.
+__device__ __forceinline__ RankGather rank_gather_at(RankGather ga, size_t in_stride, size_t cls_stride, size_t ws_stride,
+                                                     int z)
+{
+    if (ga.dets == nullptr) return ga;
+    ga.dets = seg_at(ga.dets, in_stride, z);
+    if (ga.class_ids) ga.class_ids = seg_at(ga.class_ids, cls_stride, z);
+    ga.boxes = seg_at(ga.boxes, ws_stride, z);
+    ga.areas = seg_at(ga.areas, ws_stride, z);
+    ga.cls = seg_at(ga.cls, ws_stride, z);
+    ga.order = seg_at(ga.order, ws_stride, z);
+    ga.tickets = seg_at(ga.tickets, ws_stride, z);
+    return ga;
+}
+
 __global__ void __launch_bounds__(RANK_ROWS)
-rank_seg_kernel(const float *__restrict__ scores, const int *__restrict__ tie_ids, int n, int *__restrict__ rank,
-                size_t seg_stride)
+rank_seg_kernel(const float *__restrict__ scores, int stride, const int *__restrict__ tie_ids, int n,
+                int *__restrict__ rank, RankGather ga, size_t in_stride, size_t cls_stride, size_t ws_stride)
 {
     const int z = blockIdx.z;
-    rank_body(seg_at(scores, seg_stride, z), 1, seg_at(tie_ids, seg_stride, z), n, seg_at(rank, seg_stride, z), RankGather{});
+    rank_body(seg_at(scores, in_stride, z), stride, tie_ids ? seg_at(tie_ids, in_stride, z) : nullptr, n,
+              seg_at(rank, ws_stride, z), rank_gather_at(ga, in_stride, cls_stride, ws_stride, z));
 }
 
 static int rank_launch(const float *scores, int stride, const int *tie_ids, int n, int *rank, const RankGather &ga,
@@ -197,15 +213,21 @@ int rank_sort_launch(const float *scores, int stride, const int *tie_ids, int n,
     return rank_launch(scores, stride, tie_ids, n, rank, RankGather{}, st);
 }
 
-int rank_sort_batched_launch(const float *scores, const int *tie_ids, int n, int B, size_t stride_bytes, int *rank,
-                             cudaStream_t st)
+static int rank_seg_launch(const float *scores, int stride, const int *tie_ids, int n, int B, int *rank,
+                           const RankGather &ga, size_t in_stride, size_t cls_stride, size_t ws_stride, cudaStream_t st)
 {
     if (n <= 0 || B <= 0) return SLN_OK;
     dim3 grid(cdiv(n, RANK_ROWS), cdiv(n, RANK_COLS), B);
     SLN_REQUIRE(grid.y <= 65535 && grid.z <= 65535, SLN_ERR_ARG, "rank sort: n=%d x %d segments too large", n, B);
-    rank_seg_kernel<<<grid, RANK_ROWS, 0, st>>>(scores, tie_ids, n, rank, stride_bytes);
+    rank_seg_kernel<<<grid, RANK_ROWS, 0, st>>>(scores, stride, tie_ids, n, rank, ga, in_stride, cls_stride, ws_stride);
     SLN_LAUNCH_OK("rank_seg_kernel");
     return SLN_OK;
+}
+
+int rank_sort_batched_launch(const float *scores, const int *tie_ids, int n, int B, size_t stride_bytes, int *rank,
+                             cudaStream_t st)
+{
+    return rank_seg_launch(scores, 1, tie_ids, n, B, rank, RankGather{}, stride_bytes, 0, stride_bytes, st);
 }
 
 // ---------------------------------------------------------------------------
@@ -1034,12 +1056,14 @@ __device__ __forceinline__ SparseBufs sparse_at(SparseBufs sb, size_t stride, in
 }
 
 // grid (SP_CLUSTER, B): the cluster of blockIdx.y bins problem blockIdx.y
+template <bool CLS>
 __global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_BIN_THREADS)
-nms_bin_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, int n, int G, SparseBufs sb,
-                   size_t stride)
+nms_bin_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
+                   int G, int CB, SparseBufs sb, size_t stride)
 {
     const int b = blockIdx.y;
-    nms_bin_body<false>(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, n, G, 1, sparse_at(sb, stride, b), nullptr);
+    nms_bin_body<CLS>(seg_at(boxes, stride, b), seg_at(areas, stride, b), CLS ? seg_at(cls, stride, b) : nullptr, n, G, CB,
+                      sparse_at(sb, stride, b), nullptr);
 }
 
 // warp per box (grid-strided): exact tests against the boxes binned in the window's cells.  The window's cell
@@ -1161,13 +1185,14 @@ nms_pairs_kernel(const float4 *__restrict__ boxes, const float *__restrict__ are
     nms_pairs_body<CLS>(boxes, areas, cls, n, thresh, ct, edge_cap, sb);
 }
 
+template <bool CLS>
 __global__ void __launch_bounds__(32 * SP_PAIR_WARPS)
-nms_pairs_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, int n, float thresh, float ct,
-                     unsigned edge_cap, SparseBufs sb, size_t stride)
+nms_pairs_seg_kernel(const float4 *__restrict__ boxes, const float *__restrict__ areas, const int *__restrict__ cls, int n,
+                     float thresh, float ct, unsigned edge_cap, SparseBufs sb, size_t stride)
 {
     const int b = blockIdx.y;
-    nms_pairs_body<false>(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, n, thresh, ct, edge_cap,
-                          sparse_at(sb, stride, b));
+    nms_pairs_body<CLS>(seg_at(boxes, stride, b), seg_at(areas, stride, b), CLS ? seg_at(cls, stride, b) : nullptr, n, thresh,
+                        ct, edge_cap, sparse_at(sb, stride, b));
 }
 
 // One cluster of SP_CLUSTER CTAs: the greedy survivor set from the predecessor lists, then ordered emission.
@@ -1411,14 +1436,18 @@ nms_sparse_resolve_kernel(const int *__restrict__ order, int n, int max_keep, un
     nms_sparse_resolve_body(order, n, max_keep, edge_cap, sb, keep64, keep32, num_keep);
 }
 
-// grid (SP_CLUSTER, B): one cluster per problem; clusters beyond the GPU's cluster capacity queue
+// grid (SP_CLUSTER, B): one cluster per problem; clusters beyond the GPU's cluster capacity queue.  order and the
+// workspace move by `stride`; the outputs (keep64 or keep32, and num_keep) by their own strides, in bytes, so that
+// they can live in the workspace or in a caller's [B, max_keep] / [B] arrays.  Null pointers stay null.
 __global__ void __cluster_dims__(SP_CLUSTER, 1, 1) __launch_bounds__(SP_RESOLVE_THREADS, 1)
-nms_sparse_resolve_seg_kernel(int n, int max_keep, unsigned edge_cap, SparseBufs sb, int *__restrict__ keep32,
-                              int *__restrict__ num_keep, size_t stride)
+nms_sparse_resolve_seg_kernel(const int *__restrict__ order, int n, int max_keep, unsigned edge_cap, SparseBufs sb,
+                              int64_t *__restrict__ keep64, int *__restrict__ keep32, size_t keep_stride,
+                              int *__restrict__ num_keep, size_t num_stride, size_t stride)
 {
     const int b = blockIdx.y;
-    nms_sparse_resolve_body(nullptr, n, max_keep, edge_cap, sparse_at(sb, stride, b), nullptr, seg_at(keep32, stride, b),
-                            seg_at(num_keep, stride, b));
+    nms_sparse_resolve_body(order ? seg_at(order, stride, b) : nullptr, n, max_keep, edge_cap, sparse_at(sb, stride, b),
+                            keep64 ? seg_at(keep64, keep_stride, b) : nullptr, keep32 ? seg_at(keep32, keep_stride, b) : nullptr,
+                            seg_at(num_keep, num_stride, b));
 }
 
 // grid: ~3 boxes per cell; the class-aware call spends the cells on class buckets first.  ct: the window's half-width
@@ -1669,14 +1698,15 @@ static int nms_dense_launch(const float4 *boxes, const float *areas, const int *
                        static_cast<unsigned char *>(fix) + nms_fix_bytes(n), skip, st);
 }
 
-int nms_sorted_batched_launch(int B, size_t stride, const float4 *boxes, const float *areas, int n, float thresh,
-                              int max_keep, unsigned long long *mask, int *keep32, int *num_keep, cudaStream_t st,
-                              void *stage, void *fix, void *sparse)
+int nms_sorted_batched_launch(int B, size_t stride, const float4 *boxes, const float *areas, const int *cls,
+                              const int *order, int n, float thresh, int max_keep, unsigned long long *mask,
+                              int64_t *keep64, int *keep32, size_t keep_stride, int *num_keep, size_t num_stride,
+                              cudaStream_t st, void *stage, void *fix, void *sparse)
 {
     if (B <= 0) return SLN_OK;
     if (max_keep <= 0 || max_keep > n) max_keep = n;
     if (n == 0) {
-        for (int b = 0; b < B; ++b) SLN_CUDA_OK(cudaMemsetAsync(seg_at(num_keep, stride, b), 0, sizeof(int), st));
+        for (int b = 0; b < B; ++b) SLN_CUDA_OK(cudaMemsetAsync(seg_at(num_keep, num_stride, b), 0, sizeof(int), st));
         return SLN_OK;
     }
     // the same eligibility test as launch_sparse: n and thresh are common to all problems
@@ -1687,27 +1717,29 @@ int nms_sorted_batched_launch(int B, size_t stride, const float4 *boxes, const f
         sparse_carve(sparse, n, sb);
         int CB, G;
         float ct;
-        sparse_params(n, false, thresh, CB, G, ct);
+        sparse_params(n, cls != nullptr, thresh, CB, G, ct);
         const unsigned edge_cap = (unsigned)SP_EDGES_PER_BOX * (unsigned)n;
-        SLN_CUDA_OK(launch_chain(nms_bin_seg_kernel, dim3(SP_CLUSTER, B), dim3(SP_BIN_THREADS), 0, st, true, boxes, areas, n, G,
-                                 sb, stride));
+        SLN_CUDA_OK(launch_chain(cls ? nms_bin_seg_kernel<true> : nms_bin_seg_kernel<false>, dim3(SP_CLUSTER, B),
+                                 dim3(SP_BIN_THREADS), 0, st, true, boxes, areas, cls, n, G, CB, sb, stride));
         // about the pair grid of one single-image call in all, at least one CTA per problem
         int ctas = cdiv(n, SP_PAIR_WARPS);
         const int cap = cdiv(SLN_SP_PAIR_CTAS_PER_SM * sm_count(), B);
         if (ctas > cap) ctas = cap;
-        SLN_CUDA_OK(launch_chain(nms_pairs_seg_kernel, dim3(ctas, B), dim3(32 * SP_PAIR_WARPS), 0, st, true, boxes, areas, n,
-                                 thresh, ct, edge_cap, sb, stride));
+        SLN_CUDA_OK(launch_chain(cls ? nms_pairs_seg_kernel<true> : nms_pairs_seg_kernel<false>, dim3(ctas, B),
+                                 dim3(32 * SP_PAIR_WARPS), 0, st, true, boxes, areas, cls, n, thresh, ct, edge_cap, sb, stride));
         const size_t smem = sparse_resolve_smem(n);
         SLN_CUDA_OK(cudaFuncSetAttribute(nms_sparse_resolve_seg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        SLN_CUDA_OK(launch_chain(nms_sparse_resolve_seg_kernel, dim3(SP_CLUSTER, B), dim3(SP_RESOLVE_THREADS), smem, st, true, n,
-                                 max_keep, edge_cap, sb, keep32, num_keep, stride));
+        SLN_CUDA_OK(launch_chain(nms_sparse_resolve_seg_kernel, dim3(SP_CLUSTER, B), dim3(SP_RESOLVE_THREADS), smem, st, true,
+                                 order, n, max_keep, edge_cap, sb, keep64, keep32, keep_stride, num_keep, num_stride, stride));
     }
     // dense fallback, per problem and guarded by that problem's status word: without a host read nobody knows which
     // problems need it, so every problem gets the launches and those whose sparse pass succeeded leave at once
     for (int b = 0; b < B; ++b) {
         const int *skip = sparse_ok ? &seg_at(static_cast<SparseHdr *>(sparse), stride, b)->status : nullptr;
-        const int rc = nms_dense_launch(seg_at(boxes, stride, b), seg_at(areas, stride, b), nullptr, nullptr, n, thresh, max_keep,
-                                        seg_at(mask, stride, b), nullptr, seg_at(keep32, stride, b), seg_at(num_keep, stride, b),
+        const int rc = nms_dense_launch(seg_at(boxes, stride, b), seg_at(areas, stride, b), cls ? seg_at(cls, stride, b) : nullptr,
+                                        order ? seg_at(order, stride, b) : nullptr, n, thresh, max_keep, seg_at(mask, stride, b),
+                                        keep64 ? seg_at(keep64, keep_stride, b) : nullptr,
+                                        keep32 ? seg_at(keep32, keep_stride, b) : nullptr, seg_at(num_keep, num_stride, b),
                                         st, stage ? seg_at(stage, stride, b) : nullptr, seg_at(fix, stride, b), skip);
         if (rc != SLN_OK) return rc;
     }
@@ -1761,4 +1793,52 @@ extern "C" int sln_nms(const float *dets, const int *class_ids, int n, float thr
                        int64_t *keep, int *num_keep, void *workspace, size_t workspace_bytes, void *stream)
 {
     return sln_nms_ex(dets, class_ids, n, thresh, max_keep, 0, keep, num_keep, nullptr, workspace, workspace_bytes, stream);
+}
+
+// B independent problems of n boxes.  The workspace is B copies of sln_nms_ex's, nms_buffers_bytes(n) apart (a multiple
+// of 256); problem b runs sln_nms_ex's stages with sln_nms_ex's parameters in its copy, so its survivors are the same.
+extern "C" size_t sln_nms_batched_workspace_bytes(int B, int n)
+{
+    if (B < 0 || n < 0) return 0;
+    return (size_t)B * nms_buffers_bytes(n);
+}
+
+extern "C" int sln_nms_batched(const float *dets, const int *class_ids, int B, int n, float thresh, int max_keep, int flags,
+                               int64_t *keep, int *num_keep, int *path_out, void *workspace, size_t workspace_bytes,
+                               void *stream)
+{
+    SLN_REQUIRE(B >= 0 && n >= 0, SLN_ERR_ARG, "negative size (B=%d, n=%d)", B, n);
+    SLN_REQUIRE(B <= 65535, SLN_ERR_ARG, "B=%d problems in one call (at most 65535)", B);
+    SLN_REQUIRE(!(flags & SLN_NMS_SPARSE_ONLY), SLN_ERR_ARG, "SLN_NMS_SPARSE_ONLY needs a host retry: not for the batched call");
+    if (B == 0) return SLN_OK;
+    SLN_REQUIRE(num_keep != nullptr, SLN_ERR_ARG, "null num_keep");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (path_out) SLN_CUDA_OK(cudaMemsetAsync(path_out, 0, sizeof(int) * (size_t)B, st));
+    if (n == 0) {
+        SLN_CUDA_OK(cudaMemsetAsync(num_keep, 0, sizeof(int) * (size_t)B, st));
+        return SLN_OK;
+    }
+    SLN_REQUIRE(dets && keep, SLN_ERR_ARG, "null pointer");
+    const size_t S = nms_buffers_bytes(n);
+    SLN_REQUIRE(workspace && workspace_bytes >= S * B, SLN_ERR_WORKSPACE, "batched nms workspace: need %zu bytes, got %zu",
+                S * B, workspace_bytes);
+    const int mk = (max_keep <= 0 || max_keep > n) ? n : max_keep;      // row length of keep
+    NmsBuffers b;
+    nms_carve(workspace, n, b);
+    const bool try_sparse = !(flags & SLN_NMS_DENSE_ONLY) && n >= SP_MIN_N && n <= SP_MAX_N && thresh >= 0.05f;
+    // every problem's rank[] and row-tile tickets (adjacent): one strided memset
+    const size_t clear = (size_t)(reinterpret_cast<unsigned char *>(b.tickets) - reinterpret_cast<unsigned char *>(b.rank)) +
+                         sizeof(int) * (size_t)cdiv(n, RANK_ROWS);
+    SLN_CUDA_OK(cudaMemset2DAsync(b.rank, S, 0, clear, B, st));
+    RankGather ga{dets, class_ids, b.boxes, b.areas, b.cls, b.order, b.tickets};
+    int rc = rank_seg_launch(dets + 4, 5, nullptr, n, B, b.rank, ga, sizeof(float) * 5 * (size_t)n, sizeof(int) * (size_t)n,
+                             S, st);
+    if (rc != SLN_OK) return rc;
+    rc = nms_sorted_batched_launch(B, S, b.boxes, b.areas, class_ids ? b.cls : nullptr, b.order, n, thresh, max_keep, b.mask,
+                                   keep, nullptr, sizeof(int64_t) * (size_t)mk, num_keep, sizeof(int), st, b.stage, b.fix,
+                                   try_sparse ? b.sparse : nullptr);
+    if (rc != SLN_OK) return rc;
+    if (path_out && try_sparse)      // SparseHdr.status of every problem: 1 when the sparse path produced its result
+        SLN_CUDA_OK(cudaMemcpy2DAsync(path_out, sizeof(int), b.sparse, S, sizeof(int), B, cudaMemcpyDeviceToDevice, st));
+    return SLN_OK;
 }

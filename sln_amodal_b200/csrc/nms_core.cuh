@@ -38,13 +38,15 @@ __host__ __device__ __forceinline__ T *seg_at(T *p, size_t stride_bytes, int seg
     return (T *)((const unsigned char *)p + stride_bytes * (size_t)seg);
 }
 
-// B independent problems of n boxes each: boxes, areas, mask, keep32, num_keep, stage, fix and sparse are those of
-// problem 0, problem b's are seg_at(.., stride_bytes, b).  One launch per sparse stage for all B (a cluster per
-// problem); the dense kernels run per problem and leave at once where that problem's sparse pass succeeded.  Each
-// problem's keep list is exactly nms_sorted_launch's (no classes, order == nullptr).
-int nms_sorted_batched_launch(int B, size_t stride_bytes, const float4 *boxes, const float *areas, int n, float thresh,
-                              int max_keep, unsigned long long *mask, int *keep32, int *num_keep, cudaStream_t st,
-                              void *stage, void *fix, void *sparse);
+// B independent problems of n boxes each: boxes, areas, cls, order, mask, stage, fix and sparse are those of problem 0,
+// problem b's are seg_at(.., stride_bytes, b); the outputs move by their own strides (keep64 / keep32 by keep_stride,
+// num_keep by num_stride, in bytes).  cls, order, keep64 and keep32 may be nullptr.  One launch per sparse stage for all
+// B (a cluster per problem); the dense kernels run per problem and leave at once where that problem's sparse pass
+// succeeded.  Each problem's keep list is exactly nms_sorted_launch's.
+int nms_sorted_batched_launch(int B, size_t stride_bytes, const float4 *boxes, const float *areas, const int *cls,
+                              const int *order, int n, float thresh, int max_keep, unsigned long long *mask,
+                              int64_t *keep64, int *keep32, size_t keep_stride, int *num_keep, size_t num_stride,
+                              cudaStream_t st, void *stage, void *fix, void *sparse);
 
 // Total order used everywhere a "descending score, stable" sort is needed:
 // larger key first; NaN sorts as the largest value (torch.sort's convention);

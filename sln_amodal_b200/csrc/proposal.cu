@@ -552,8 +552,8 @@ extern "C" int sln_proposal_layer_batched(const float *probs, const float *delta
     Float4Std sd{std_dev_host[0], std_dev_host[1], std_dev_host[2], std_dev_host[3]};
     SLN_CUDA_OK(launch_chain(proposal_decode_seg_kernel, dim3(cdiv(K, 128), B), dim3(128), 0, st, true, anchors, deltas, A,
                              (const int *)b.cand_idx, (const int *)nb.rank, K, sd, img_h, img_w, nb.boxes, nb.areas, S));
-    rc = nms_sorted_batched_launch(B, S, nb.boxes, nb.areas, K, nms_thresh, proposal_count, nb.mask, b.keep, b.num_keep, st,
-                                   nb.stage, nb.fix, nb.sparse);
+    rc = nms_sorted_batched_launch(B, S, nb.boxes, nb.areas, nullptr, nullptr, K, nms_thresh, proposal_count, nb.mask, nullptr,
+                                   b.keep, S, b.num_keep, S, st, nb.stage, nb.fix, nb.sparse);
     if (rc != SLN_OK) return rc;
     proposal_finalize_seg_kernel<<<dim3(cdiv(proposal_count, 128), B), 128, 0, st>>>(
         nb.boxes, b.keep, b.num_keep, proposal_count, img_h, img_w, reinterpret_cast<float4 *>(out_boxes), num_out, S);

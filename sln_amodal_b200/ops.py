@@ -514,6 +514,56 @@ def nms_device(dets, thresh, class_ids=None, max_keep=0, dense_only=False, retur
     return keep, num
 
 
+def _dense_nms_launches(n):
+    """Kernels of nms.cu's dense pipeline for n > 0 boxes: mask + scan, the fixed-point resolve from 160 words, and from
+    16384 boxes two stages (stage A's mask + scan, suppress, compact, emit, then stage B)."""
+    if n < 16384:
+        return 2 + (((n + 63) // 64) >= 160)
+    return 2 + 3 + 2 + (((n - 1024 + 63) // 64) >= 160)
+
+
+def nms_batched_device(dets, thresh, class_ids=None, max_keep=0, dense_only=False, return_path=False):
+    """B independent greedy NMS problems in one call (sln_nms_batched).  dets [B,n,5], class_ids integer [B,n] or None.
+    Returns (keep int64 [B,mk], num_keep int32 [B]) on the device, mk = max_keep if 0 < max_keep <= n else n, plus a
+    device int32 [B] path report with return_path.  keep[b, :num_keep[b]] and num_keep[b] are nms_device's for problem b
+    alone; entries beyond num_keep[b] are undefined.  No host sync; graph capturable."""
+    _require_cuda(dets, "dets")
+    if dets.dim() != 3 or dets.shape[2] != 5:
+        raise _lib.SlnError(f"dets must be [B,n,5] (y1,x1,y2,x2,score), got {tuple(dets.shape)}")
+    if not dets.dtype.is_floating_point:
+        raise _lib.SlnError(f"dets must be floating point, got {dets.dtype}")
+    B, n = int(dets.shape[0]), int(dets.shape[1])
+    if B > 65535:
+        raise _lib.SlnError(f"B={B} problems in one call (at most 65535)")
+    if int(max_keep) < 0:
+        raise _lib.SlnError(f"max_keep must be >= 0 (0: all), got {max_keep}")
+    if class_ids is not None:
+        _require_cuda(class_ids, "class_ids")
+        if tuple(class_ids.shape) != (B, n):
+            raise _lib.SlnError(f"class_ids {tuple(class_ids.shape)} disagrees with dets {tuple(dets.shape)}")
+        if class_ids.dtype.is_floating_point or class_ids.dtype == torch.bool:
+            raise _lib.SlnError(f"class_ids must be an integer tensor, got {class_ids.dtype}")
+    dets = _f32c(dets)
+    cls = _i32c(class_ids) if class_ids is not None else None
+    mk = n if int(max_keep) == 0 or int(max_keep) > n else int(max_keep)
+    keep = torch.empty((B, mk), dtype=torch.int64, device=dets.device)
+    num = torch.empty(B, dtype=torch.int32, device=dets.device)
+    path = torch.empty(B, dtype=torch.int32, device=dets.device) if return_path else None
+    with torch.cuda.device(dets.device):
+        ws = _workspace(lib().sln_nms_batched_workspace_bytes(B, n), dets.device)
+        check(lib().sln_nms_batched(ptr(dets), ptr(cls), B, n, float(thresh), int(max_keep), 1 if dense_only else 0,
+                                    ptr(keep), ptr(num), ptr(path), ptr(ws), ws.numel(), stream_ptr()), "sln_nms_batched")
+    if B:
+        sparse = n > 0 and not dense_only and 65 <= n <= 65535 and float(thresh) >= 0.05
+        launches = 2 + 3 * sparse + B * _dense_nms_launches(n) if n else 1      # rank memset + rank; bin, pairs, resolve
+        if return_path:
+            launches += 1 + sparse                                              # path memset (+ the status copy)
+        _lib.count_launches(launches)
+    if return_path:
+        return keep, num, path
+    return keep, num
+
+
 def refine_decode_device(rois, probs, deltas, std_dev, image_hw, window, min_confidence=0.0):
     """Elementwise front of refine_detections in one launch (include/sln_b200.h, sln_refine_decode).
     Returns (dets [N,5], cls_nms int32[N], class_ids int32[N], n_excluded int32[1]) on the device."""
@@ -578,6 +628,37 @@ def refine_topk_batched_device(dets, class_ids, max_keep=100):
             check(lib().sln_refine_topk_batched(ptr(dets), ptr(class_ids), B, N, int(max_keep), ptr(result), ptr(keep),
                                                 ptr(num_det), stream_ptr()), "sln_refine_topk_batched")
         _lib.count_launches(2 if N and max_keep else 1)
+    return result, keep, num_det
+
+
+def refine_nms_emit_batched_device(dets, class_ids, nms_keep, nms_num, max_detections):
+    """The per-class NMS branch's last step for B images (sln_refine_nms_emit_batched).  dets [B,N,5] and class_ids int32
+    [B,N] are sln_refine_decode's outputs viewed per image; nms_keep [B,mk] / nms_num [B] are nms_batched_device's on
+    (dets, cls_nms) with max_keep = max_detections.  Returns (result f32 [B,D,6], keep int64 [B,D], num_det int32 [B]),
+    zero beyond num_det[b] = min(D, survivors with a finite score)."""
+    _require_cuda(dets, "dets")
+    if dets.dim() != 3 or dets.shape[2] != 5:
+        raise _lib.SlnError(f"dets must be [B,N,5], got {tuple(dets.shape)}")
+    B, N, D = int(dets.shape[0]), int(dets.shape[1]), int(max_detections)
+    if D < 0:
+        raise _lib.SlnError(f"max_detections must be >= 0, got {max_detections}")
+    if tuple(class_ids.shape) != (B, N):
+        raise _lib.SlnError(f"class_ids {tuple(class_ids.shape)} disagrees with dets {tuple(dets.shape)}")
+    if nms_keep.dim() != 2 or int(nms_keep.shape[0]) != B or int(nms_keep.shape[1]) > N or tuple(nms_num.shape) != (B,):
+        raise _lib.SlnError(f"nms keep {tuple(nms_keep.shape)} / num {tuple(nms_num.shape)} disagree with dets {tuple(dets.shape)}")
+    if nms_keep.dtype != torch.int64 or nms_num.dtype != torch.int32:
+        raise _lib.SlnError("nms keep must be int64 and num int32 (nms_batched_device's outputs)")
+    dets, class_ids = _f32c(dets), _i32c(class_ids)
+    nms_keep, nms_num = nms_keep.contiguous(), nms_num.contiguous()
+    result = torch.empty((B, D, 6), dtype=torch.float32, device=dets.device)
+    keep = torch.empty((B, D), dtype=torch.int64, device=dets.device)
+    num_det = torch.empty(B, dtype=torch.int32, device=dets.device)
+    if B:
+        with torch.cuda.device(dets.device):
+            check(lib().sln_refine_nms_emit_batched(ptr(dets), ptr(class_ids), B, N, ptr(nms_keep), ptr(nms_num),
+                                                    int(nms_keep.shape[1]), D, ptr(result), ptr(keep), ptr(num_det),
+                                                    stream_ptr()), "sln_refine_nms_emit_batched")
+        _lib.count_launches(1)
     return result, keep, num_det
 
 

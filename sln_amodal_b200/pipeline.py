@@ -9,8 +9,13 @@ replayed with a single launch per image -- no Python between the kernels, no hos
     proposal_layer (top-6000 select, decode, clip, NMS, top-k; `num` stays on the device)
       -> FPN level of every ROI + one crop launch for all levels            (pyramid_roi_align, pool 7)
       -> [classifier callback: the model's own head, out of scope here]
-      -> refine_detections, USE_NMS = False branch: decode + top-100 in two launches (rows beyond `num` masked out)
+      -> refine_detections, the branch config.USE_NMS names (rows beyond `num` masked out):
+           USE_NMS = False: decode + top-100 in two launches
+           USE_NMS = True:  decode + batched class-aware NMS + one emit launch (refine_detections_batched)
       -> FPN level + crop of the detections                                 (pyramid_roi_align, pool 14 / 16)
+
+With USE_NMS = True the graph keeps the first `max_detections` survivors; the reference keeps all of them.  Pass
+max_detections = proposal_count for its untruncated output.
 
 Padding contract: `rois` has `proposal_count` rows, zeros beyond `num`; `detections` has 100 rows, zeros beyond `num_det`;
 the crops of padded rows are crops of the zero box (harmless, never read by a caller that honours the counts).  Rows
@@ -22,6 +27,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .detection import refine_detections_batched
 from .proposal import PRE_NMS_LIMIT
 
 
@@ -32,7 +38,11 @@ class HeadGraph:
     reference's config.py names).  feature_maps / rpn_probs [A,2] / rpn_bbox [A,4] are the STATIC input tensors: the graph
     reads these addresses on every replay, so the caller refreshes their contents in place (copy_) between replays.
     classifier(pooled [R,C,p,p], rois [R,4]) -> (probs [R,K], deltas [R,K,4]) runs inside the capture (any capturable
-    torch code: the model's classifier head); it may also be a pair of static tensors (probs, deltas)."""
+    torch code: the model's classifier head); it may also be a pair of static tensors (probs, deltas).
+    With config.USE_NMS true (also reading DETECTION_MIN_CONFIDENCE and DETECTION_NMS_THRESHOLD) refine_detections takes
+    its per-class NMS branch and keeps the first max_detections survivors; the reference keeps all of them, so pass
+    max_detections = proposal_count for its untruncated output.  Without the attribute, or with it false, the top-k
+    branch runs."""
 
     def __init__(self, anchors, config, feature_maps, rpn_probs, rpn_bbox, classifier, proposal_count=1000,
                  max_detections=100, window=None, capture=True):
@@ -79,11 +89,16 @@ class HeadGraph:
             self._box_ind = torch.zeros(R, dtype=torch.int32, device=self.dev)
         valid = self._ar_r < num
         probs = torch.where(valid[:, None], probs[:R], self._bg)
-        dets, _, class_ids, n_excl = ops.refine_decode_device(rois, probs, deltas[:R], self.std_rpn, self.image_hw, self.window, 0.0)
-        det, keep = ops.refine_topk_device(dets, class_ids, D)
-        num_det = torch.clamp(R - n_excl, max=D)
-        rows = self._ar_d < num_det
-        det = torch.where(rows[:, None], det, torch.zeros_like(det))         # rows beyond num_det were never written
+        if getattr(cfg, "USE_NMS", False):
+            # per-class NMS branch, the B = 1 case of the batched form: rows zero beyond num_det, keep too
+            det, keep, num_det = refine_detections_batched(rois[None], probs[None], deltas[:R][None], self.window, cfg, D)
+            det, keep = det[0], keep[0]
+        else:
+            dets, _, class_ids, n_excl = ops.refine_decode_device(rois, probs, deltas[:R], self.std_rpn, self.image_hw, self.window, 0.0)
+            det, keep = ops.refine_topk_device(dets, class_ids, D)
+            num_det = torch.clamp(R - n_excl, max=D)
+            rows = self._ar_d < num_det
+            det = torch.where(rows[:, None], det, torch.zeros_like(det))     # rows beyond num_det were never written
         boxes = det[:, :4] / self._norm
         lvl_d = ops.roi_levels_device(boxes, self.image_hw)
         mp = int(cfg.MASK_POOL_SIZE)
@@ -148,7 +163,8 @@ class BatchedHeadGraph(HeadGraph):
     [B,R,K] / [B,R,K,4]).  Outputs are [B, ...]: rois [B,R,4] and detections [B,D,6] zero beyond num_rois[b] /
     num_detections[b] (keep too), pooled [B,R,C,p,p], mask_pooled [B,D,C,mp,mp].  Below the counts every image's outputs
     are bit-identical to its own HeadGraph's: the crops, the level rule and the refine front are per row, and the
-    proposals and the top-k are ranked within the image."""
+    proposals, the top-k and the per-class NMS (config.USE_NMS, as in HeadGraph, with the same max_detections cap) run
+    within the image."""
 
     def __init__(self, anchors, config, feature_maps, rpn_probs, rpn_bbox, classifier, proposal_count=1000,
                  max_detections=100, window=None, capture=True):
@@ -183,11 +199,15 @@ class BatchedHeadGraph(HeadGraph):
         # rows beyond each image's proposal count get the background class, as in HeadGraph
         valid = (self._ar_r[None, :] < num[:, None]).reshape(B * R)
         probs = torch.where(valid[:, None], probs, self._bg)
-        dets, _, class_ids, _ = ops.refine_decode_device(flat, probs, deltas, self.std_rpn, self.image_hw, self.window, 0.0)
-        det, keep, num_det = ops.refine_topk_batched_device(dets.view(B, R, 5), class_ids.view(B, R), D)
-        rows = self._ar_d[None, :] < num_det[:, None]
-        det = torch.where(rows[..., None], det, torch.zeros_like(det))       # rows beyond num_det were never written
-        keep = torch.where(rows, keep, torch.zeros_like(keep))
+        if getattr(cfg, "USE_NMS", False):
+            det, keep, num_det = refine_detections_batched(rois, probs.view(B, R, -1), deltas.view(B, R, -1, 4), self.window,
+                                                           cfg, D)
+        else:
+            dets, _, class_ids, _ = ops.refine_decode_device(flat, probs, deltas, self.std_rpn, self.image_hw, self.window, 0.0)
+            det, keep, num_det = ops.refine_topk_batched_device(dets.view(B, R, 5), class_ids.view(B, R), D)
+            rows = self._ar_d[None, :] < num_det[:, None]
+            det = torch.where(rows[..., None], det, torch.zeros_like(det))   # rows beyond num_det were never written
+            keep = torch.where(rows, keep, torch.zeros_like(keep))
         boxes = (det[..., :4] / self._norm).reshape(B * D, 4)
         lvl_d = ops.roi_levels_device(boxes, self.image_hw)
         mp = int(cfg.MASK_POOL_SIZE)
