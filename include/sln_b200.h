@@ -287,6 +287,11 @@ SLN_API int sln_plane_bboxes(const uint8_t *planes, int M, int H, int W, int *bo
  * the string length, or -(needed capacity) when cap is too small.                                          */
 SLN_API int sln_rle_encode(const uint8_t *masks, int n, long long a, uint32_t *counts, int cap, int *m_out, void *stream);
 SLN_API long long sln_rle_to_string(const uint32_t *counts, long long m, char *out, long long cap);
+/* sln_rle_to_string on the device for n count lists counts u32 [n][cap] of m[i] runs each (a list with m[i] <= 0 or
+ * > cap gets an empty string): the strings packed in list order into `strings` (no terminators), str_off / str_len
+ * i32 [n], *str_total = total bytes.  strings_cap >= 7 * cap * n and < 2^31.  Three launches, no host sync.       */
+SLN_API int sln_rle_strings(const uint32_t *counts, int n, int cap, const int *m, int *str_off, int *str_len,
+                    int *str_total, char *strings, long long strings_cap, void *stream);
 
 /* Mask paste after the path (SURVEY 8(f)-3): utils.unmold_mask (utils.py:447-465) for N detections in one launch.
  * masks f32 [N,mh,mw] (the head's small masks), boxes i32 [N,4] = (y1,x1,y2,x2) in image pixels, y2 / x2 exclusive,
@@ -296,6 +301,26 @@ SLN_API long long sln_rle_to_string(const uint32_t *counts, long long m, char *o
  * detections first, model.py:786-795, and its paste raises on a box outside the image).  mh, mw <= 256.          */
 SLN_API int sln_unmold_masks(const float *masks, int N, int mh, int mw, const int *boxes, int H, int W,
                      uint8_t *out, void *stream);
+
+/* Batched evaluation tail: MaskRCNN.unmold_detections (model.py:747-806) + COCO RLE (amodal_train.py:371-400) for B
+ * images of D detection rows, from box-sized masks: no H x W plane is written.  detections f32 [B,D,6] contiguous,
+ * (y1,x1,y2,x2,class_id,score); mrcnn_mask f32 [B,D,mh,mw,K] read through mask_strides_host (5 element strides, any
+ * layout); H_host / W_host: B image sizes; scale_shift_host f64 [B,4] = (h_scale, w_scale, window[0], window[1]) as
+ * the reference computes them.  Per image: the padding cut (first row with class 0), class collapse to 1, astype(int32)
+ * of (box - shift) * scale in float64, the keep rule of unmold_detections, compaction in order.  Outputs, rows at and
+ * beyond num_kept[b] zero: boxes i32 [B,D,4], class_ids i32 [B,D], scores f32 [B,D], src_row i32 [B,D] (detection row
+ * of each kept box), num_kept i32 [B] (-1: a row before the cut names a class outside the K mask channels, where the
+ * reference raises).  Per kept mask, m_out [B,D] = number of runs of the column-major H x W plane, or -m when m > cap
+ * (nothing written; 0 for rows past num_kept), and its rleToString string at strings[str_off : str_off + str_len]
+ * (packed in row order, no terminator; *str_total bytes in all).  strings_cap >= 7 * cap * B * D.  Five launches for
+ * any B and D, no host sync, graph capturable.  B <= 512.  B == 0 and D == 0 are valid.                        */
+SLN_API size_t sln_unmold_rle_batched_workspace_bytes(int B, int D, const int *H_host, const int *W_host, int cap);
+SLN_API int sln_unmold_rle_batched(const float *detections, int B, int D, const float *mrcnn_mask, int mh, int mw,
+                           int K, const long long *mask_strides_host, const int *H_host, const int *W_host,
+                           const double *scale_shift_host, int cap, int *boxes, int *class_ids, float *scores,
+                           int *src_row, int *num_kept, int *m_out, int *str_off, int *str_len, int *str_total,
+                           char *strings, long long strings_cap, void *workspace, size_t workspace_bytes,
+                           void *stream);
 
 /* Image resize in front of the path (SURVEY 8(f)-2): utils.resize_image (utils.py:301-356) squashes the uint8 image to
  * (max_dim, max_dim) with scipy.misc.imresize = Pillow's 8-bit bilinear resample per band (triangle filter of support

@@ -18,7 +18,7 @@ from .targets import (bbox_overlaps, box_refinement, build_rpn_targets, detectio
                       resize_image, resize_image_device, resize_layer, resize_layer_device, zoom_index_map)
 from .rle import encode as rle_encode  # noqa: F401
 from .rpn import rpn_forward_levels, rpn_pack  # noqa: F401
-from .unmold import unmold_detections, unmold_mask, unmold_masks  # noqa: F401
+from .unmold import unmold_detections, unmold_detections_batched, unmold_mask, unmold_masks  # noqa: F401
 from .install import install  # noqa: F401
 
 __version__ = "0.1.0"

@@ -64,7 +64,12 @@ PROTOTYPES = {
     "sln_plane_bboxes": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "sln_rle_encode": (_i, [_vp, _i, C.c_longlong, _vp, _i, _vp, _vp]),
     "sln_rle_to_string": (C.c_longlong, [_vp, C.c_longlong, C.c_char_p, C.c_longlong]),
+    "sln_rle_strings": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, C.c_longlong, _vp]),
     "sln_unmold_masks": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _vp, _vp]),
+    "sln_unmold_rle_batched_workspace_bytes": (_sz, [_i, _i, C.POINTER(_i), C.POINTER(_i), _i]),
+    "sln_unmold_rle_batched": (_i, [_vp, _i, _i, _vp, _i, _i, _i, C.POINTER(C.c_longlong), C.POINTER(_i), C.POINTER(_i),
+                                    C.POINTER(C.c_double), _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                    C.c_longlong, _vp, _sz, _vp]),
     "sln_resize_image_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "sln_resize_image_u8": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
     "sln_gather_planes": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp]),

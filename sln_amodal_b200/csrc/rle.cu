@@ -9,9 +9,12 @@
 //   pass 2  every thread walks its chunk again and writes, for its k-th change at j, counts[k] = j - previous change
 // The masks are read in the memory order given (pycocotools encodes column-major planes: pass them transposed).
 // Bytes per mask: a (read twice, the second pass from L2) + 4 m written.
+// For sln_unmold_rle_batched the runs come from box-sized masks instead (rle_box_kernel: the plane is never built), and
+// the strings are made on the device too (rle_str_*_kernel: maskApi.c's rleToString, packed for all masks).
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "eval_tail.cuh"
 
 #include <cooperative_groups.h>
 
@@ -276,6 +279,212 @@ rle_encode_coalesced_kernel(const unsigned char *__restrict__ masks, long long a
     }
 }
 
+// ---------------------------------------------------------------------------
+// Runs from a box-sized mask (sln_unmold_rle_batched).  The column-major H x W plane that pycocotools encodes is zero
+// outside the box, so its value changes lie in the box's column segments [x*H + y1, x*H + y2) or right after them.  A
+// segment's first pixel is compared with 0, except in a full-height box (y1 == 0, y2 == H) past its first column:
+// there the plane runs straight on from the previous column's last box pixel (the box is one contiguous stretch of the
+// plane).  After a segment the plane is 0 again, so a set last pixel makes a change one past it, unless the next
+// column's segment follows at once (full height) or the plane ends there.  The final run closes at a = H*W.
+// One CTA per detection; each thread takes a contiguous chunk of the bh*bw box bytes, in two passes like
+// rle_encode_kernel (count, block scan, write).  The string length of maskApi.c's rleToString is added up at the end.
+// ---------------------------------------------------------------------------
+constexpr int RLEB_THREADS = 256;
+
+// characters rleToString spends on one delta x (maskApi.c:204-216): 5 bits per char until the rest is the sign
+__device__ __forceinline__ int rle_chars(long long x)
+{
+    int n = 0;
+    bool more = true;
+    while (more) {
+        const int c = (int)(x & 0x1f);
+        x >>= 5;
+        more = (c & 0x10) ? x != -1 : x != 0;
+        ++n;
+    }
+    return n;
+}
+
+__device__ __forceinline__ void rle_put(long long x, char *o)
+{
+    bool more = true;
+    while (more) {
+        char c = (char)(x & 0x1f);
+        x >>= 5;
+        more = (c & 0x10) ? x != -1 : x != 0;
+        if (more) c |= 0x20;
+        *o++ = (char)(c + 48);
+    }
+}
+
+// maskApi.c's delta: counts[k] against counts[k-2], from k = 3 on (sic: `if (i > 2)`)
+__device__ __forceinline__ long long rle_delta(const uint32_t *c, int k)
+{
+    long long x = (long long)c[k];
+    if (k > 2) x -= (long long)c[k - 2];
+    return x;
+}
+
+template <int THREADS>
+__device__ __forceinline__ int block_string_length(const uint32_t *c, int m, int *warp_tot)
+{
+    int n = 0;
+    for (int k = threadIdx.x; k < m; k += THREADS) n += rle_chars(rle_delta(c, k));
+    int total;
+    block_excl_sum<THREADS>(n, warp_tot, &total);
+    return total;
+}
+
+__global__ void __launch_bounds__(RLEB_THREADS)
+rle_box_kernel(const BoxRow *__restrict__ rows, const int *__restrict__ nk, int D, const uint8_t *__restrict__ maskbuf,
+               uint32_t *__restrict__ counts, int cap, int *__restrict__ m_out, int *__restrict__ str_len)
+{
+    __shared__ int s_cnt[RLEB_THREADS / 32];
+    __shared__ long long s_last[RLEB_THREADS / 32];
+    const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = row / D;
+    if (row - b * D >= nk[b]) {
+        if (tid == 0) { m_out[row] = 0; str_len[row] = 0; }
+        return;
+    }
+    const BoxRow R = rows[row];
+    const long long H = R.H, a = H * R.W, area = (long long)R.bh * R.bw;
+    const uint8_t *T = maskbuf + R.off;
+    uint32_t *out = counts + (size_t)row * cap;
+    const bool merge = R.y1 == 0 && R.bh == R.H;
+    const long long len = (area + RLEB_THREADS - 1) / RLEB_THREADS;
+    const long long i0 = min(area, tid * len), i1 = min(area, i0 + len);
+
+    auto walk = [&](auto &&on_change) {
+        if (i0 >= i1) return;
+        int c = (int)(i0 / R.bh), r = (int)(i0 - (long long)c * R.bh);
+        long long col = (long long)(R.x1 + c) * H + R.y1;      // plane position of box row 0 of column c
+        unsigned prev = (r > 0 || (merge && i0 > 0)) ? T[i0 - 1] : 0u;
+        for (long long i = i0; i < i1; ++i) {
+            const unsigned v = T[i];
+            if (v != prev) on_change(col + r);
+            if (r == R.bh - 1) {
+                if (v && (!merge || c == R.bw - 1) && col + r + 1 < a) on_change(col + r + 1);
+                ++c;
+                r = 0;
+                col += H;
+                prev = merge ? v : 0u;
+            } else {
+                ++r;
+                prev = v;
+            }
+        }
+    };
+
+    // ---- pass 1: count, remember the last change; then the exclusive count and the last change before each thread
+    int cnt = 0;
+    long long last = -1;
+    walk([&](long long j) { ++cnt; last = j; });
+    long long lmax = last;
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long l = __shfl_up_sync(0xffffffffu, lmax, o);
+        if (lane >= o) lmax = max(lmax, l);
+    }
+    if (lane == 31) s_last[warp] = lmax;
+    int total;
+    const int off = block_excl_sum<RLEB_THREADS>(cnt, s_cnt, &total);   // its barriers publish s_last too
+    long long before = -1, last_all = -1;
+    for (int w = 0; w < RLEB_THREADS / 32; ++w) {
+        if (w < warp) before = max(before, s_last[w]);
+        last_all = max(last_all, s_last[w]);
+    }
+    long long prev_change = __shfl_up_sync(0xffffffffu, lmax, 1);
+    if (lane == 0) prev_change = -1;
+    prev_change = max(prev_change, before);
+    // ---- pass 2: counts[k] = change k - change k-1 (the first from 0); counts[total] closes the plane
+    const int m = total + 1;
+    if (m <= cap) {
+        int k = off;
+        long long pc = prev_change < 0 ? 0 : prev_change;
+        walk([&](long long j) { out[k++] = (uint32_t)(j - pc); pc = j; });
+        if (tid == 0) out[total] = (uint32_t)(a - (last_all < 0 ? 0 : last_all));
+    }
+    __syncthreads();                                   // the counts are read back below by other threads
+    const int slen = m <= cap ? block_string_length<RLEB_THREADS>(out, m, s_cnt) : 0;
+    if (tid == 0) {
+        m_out[row] = m <= cap ? m : -m;
+        str_len[row] = slen;
+    }
+}
+
+// ---------------------------------------------------------------------------
+// Device string coder: rleToString (maskApi.c:204-216) for n count lists, packed into one buffer.  The characters of
+// counts[k] depend only on counts[k] and counts[k-2], so a mask's string is per-count lengths, a scan and the writes;
+// the masks' strings follow one another in mask order (a scan over the n lengths).  Byte for byte what the host
+// helper sln_rle_to_string writes, without its terminating 0.
+// ---------------------------------------------------------------------------
+constexpr int STR_THREADS = 256;
+constexpr int STR_SCAN_THREADS = 1024;
+
+__global__ void __launch_bounds__(STR_THREADS)
+rle_str_len_kernel(const uint32_t *__restrict__ counts, int cap, const int *__restrict__ m, int *__restrict__ str_len)
+{
+    __shared__ int s_w[STR_THREADS / 32];
+    const int i = blockIdx.x, mi = m[i];
+    const int len = (mi > 0 && mi <= cap) ? block_string_length<STR_THREADS>(counts + (size_t)i * cap, mi, s_w) : 0;
+    if (threadIdx.x == 0) str_len[i] = len;
+}
+
+__global__ void __launch_bounds__(STR_SCAN_THREADS)
+rle_str_scan_kernel(const int *__restrict__ str_len, int n, int *__restrict__ str_off, int *__restrict__ str_total)
+{
+    __shared__ int s_w[STR_SCAN_THREADS / 32];
+    int run = 0;
+    for (int c0 = 0; c0 < n; c0 += STR_SCAN_THREADS) {
+        const int i = c0 + threadIdx.x;
+        const int v = i < n ? str_len[i] : 0;
+        int t;
+        const int e = block_excl_sum<STR_SCAN_THREADS>(v, s_w, &t);
+        if (i < n) str_off[i] = run + e;
+        run += t;
+    }
+    if (threadIdx.x == 0) *str_total = run;
+}
+
+__global__ void __launch_bounds__(STR_THREADS)
+rle_str_write_kernel(const uint32_t *__restrict__ counts, int cap, const int *__restrict__ m,
+                     const int *__restrict__ str_off, const int *__restrict__ str_len, char *__restrict__ strings)
+{
+    __shared__ int s_w[STR_THREADS / 32];
+    const int i = blockIdx.x;
+    if (str_len[i] == 0) return;
+    const int mi = m[i];
+    const uint32_t *c = counts + (size_t)i * cap;
+    char *o = strings + str_off[i];
+    int run = 0;
+    for (int k0 = 0; k0 < mi; k0 += STR_THREADS) {
+        const int k = k0 + threadIdx.x;
+        const long long x = k < mi ? rle_delta(c, k) : 0;
+        int t;
+        const int e = block_excl_sum<STR_THREADS>(k < mi ? rle_chars(x) : 0, s_w, &t);
+        if (k < mi) rle_put(x, o + run + e);
+        run += t;
+    }
+}
+
+int launch_rle_boxes(const BoxRow *rows, const int *nk, int B, int D, const uint8_t *maskbuf, uint32_t *counts, int cap,
+                     int *m_out, int *str_len, cudaStream_t st)
+{
+    rle_box_kernel<<<B * D, RLEB_THREADS, 0, st>>>(rows, nk, D, maskbuf, counts, cap, m_out, str_len);
+    SLN_LAUNCH_OK("rle_box_kernel");
+    return SLN_OK;
+}
+
+int launch_rle_strings(const uint32_t *counts, int n, int cap, const int *m, const int *str_len, int *str_off,
+                       int *str_total, char *strings, cudaStream_t st)
+{
+    rle_str_scan_kernel<<<1, STR_SCAN_THREADS, 0, st>>>(str_len, n, str_off, str_total);
+    SLN_LAUNCH_OK("rle_str_scan_kernel");
+    rle_str_write_kernel<<<n, STR_THREADS, 0, st>>>(counts, cap, m, str_off, str_len, strings);
+    SLN_LAUNCH_OK("rle_str_write_kernel");
+    return SLN_OK;
+}
+
 }  // namespace sln
 
 extern "C" int sln_rle_encode(const uint8_t *masks, int n, long long a, uint32_t *counts, int cap, int *m_out, void *stream)
@@ -317,4 +526,22 @@ extern "C" long long sln_rle_to_string(const uint32_t *counts, long long m, char
     }
     if (p < cap) out[p] = 0;
     return p < cap ? p : -(p + 1);
+}
+
+extern "C" int sln_rle_strings(const uint32_t *counts, int n, int cap, const int *m, int *str_off, int *str_len,
+                               int *str_total, char *strings, long long strings_cap, void *stream)
+{
+    SLN_REQUIRE(n >= 0 && cap >= 1, SLN_ERR_ARG, "rle_strings: bad n / cap");
+    SLN_REQUIRE(strings_cap >= 7ll * cap * n && strings_cap < (1ll << 31), SLN_ERR_ARG,
+                "rle_strings: strings_cap must be >= 7 * cap * n and < 2^31 (got %lld)", strings_cap);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    SLN_REQUIRE(str_total, SLN_ERR_ARG, "rle_strings: null pointer");
+    if (n == 0) {
+        SLN_CUDA_OK(cudaMemsetAsync(str_total, 0, sizeof(int), st));
+        return SLN_OK;
+    }
+    SLN_REQUIRE(counts && m && str_off && str_len && strings, SLN_ERR_ARG, "rle_strings: null pointer");
+    sln::rle_str_len_kernel<<<n, sln::STR_THREADS, 0, st>>>(counts, cap, m, str_len);
+    SLN_LAUNCH_OK("rle_str_len_kernel");
+    return sln::launch_rle_strings(counts, n, cap, m, str_len, str_off, str_total, strings, st);
 }

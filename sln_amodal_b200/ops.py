@@ -7,6 +7,7 @@ the caller side, as the ABI requires) and the stream.
 """
 from __future__ import annotations
 
+import collections
 import ctypes as C
 
 import numpy as np
@@ -660,6 +661,127 @@ def refine_nms_emit_batched_device(dets, class_ids, nms_keep, nms_num, max_detec
                                                     stream_ptr()), "sln_refine_nms_emit_batched")
         _lib.count_launches(1)
     return result, keep, num_det
+
+
+UNMOLD_BATCH_MAX = 512          # images per sln_unmold_rle_batched call (their sizes and windows travel as kernel parameters)
+
+
+def unmold_scale_shift(image_shape, window):
+    """model.py:774-779 for one image: (h_scale, w_scale, window[0], window[1]) as Python floats, computed with the
+    reference's own expressions.  The device runs the box arithmetic in float64, which is what numpy does for integer
+    and float64 windows; a float32 / float16 window would make numpy round in that type, and is refused."""
+    if isinstance(window, torch.Tensor):
+        window = window.detach().cpu().numpy()
+    h_scale = image_shape[0] / (window[2] - window[0])
+    w_scale = image_shape[1] / (window[3] - window[1])
+    shift = window[:2]
+    scales = np.array([h_scale, w_scale, h_scale, w_scale])
+    shifts = np.array([shift[0], shift[1], shift[0], shift[1]])
+    if np.result_type(np.float32, shifts.dtype, scales.dtype) != np.float64:
+        raise _lib.SlnError(f"window {window!r}: the box arithmetic would run in "
+                            f"{np.result_type(np.float32, shifts.dtype, scales.dtype)}, not float64 (pass integer or float64 windows)")
+    return float(scales[0]), float(scales[1]), float(shifts[0]), float(shifts[1])
+
+
+# Outputs of unmold_rle_batched_device, all on the device.  boxes int32 [B,D,4], class_ids int32 [B,D], scores f32 [B,D],
+# src_row int32 [B,D], m int32 [B,D], str_off int32 [B,D], str_len int32 [B,D], num_kept int32 [B] and str_total int32
+# [1] are views of one int32 buffer `meta` (one copy brings them all to the host); strings u8 holds the packed strings.
+UnmoldRle = collections.namedtuple("UnmoldRle", "boxes class_ids scores src_row m str_off str_len num_kept str_total "
+                                                "strings meta")
+
+
+def unmold_meta_views(meta, B, D):
+    """Split the int32 metadata buffer of unmold_rle_batched_device (device tensor or its host copy) into its fields:
+    boxes [B,D,4], class_ids, scores (f32), src_row, m, str_off, str_len [B,D], num_kept [B], str_total [1]."""
+    n, o, out = B * D, 0, []
+    for size, shape in ((4 * n, (B, D, 4)), (n, (B, D)), (n, (B, D)), (n, (B, D)), (n, (B, D)), (n, (B, D)), (n, (B, D)),
+                        (B, (B,)), (1, (1,))):
+        out.append(meta[o:o + size].reshape(shape))
+        o += size
+    out[2] = out[2].view(torch.float32) if isinstance(out[2], torch.Tensor) else out[2].view(np.float32)
+    return out
+
+
+def unmold_rle_batched_device(detections, mrcnn_mask, image_shapes, windows, cap=None, workspace=None):
+    """unmold_detections + COCO RLE for B images in one sync-free device pass (sln_unmold_rle_batched, five launches).
+    detections f32 [B,D,6] and mrcnn_mask f32 [B,D,h,w,K] (any strides) on the device; image_shapes and windows: B host
+    values each.  cap: most runs per mask (default 2 * max W + 1: a mask whose every column holds one stretch of ones has
+    at most two changes per column); a mask with more gets m = -runs and no string.  workspace: a u8 CUDA tensor of at
+    least sln_unmold_rle_batched_workspace_bytes (allocated when None).  Returns an UnmoldRle of device tensors."""
+    _require_cuda(detections, "detections")
+    _require_cuda(mrcnn_mask, "mrcnn_mask")
+    if detections.dim() != 3 or detections.shape[2] != 6 or detections.dtype != torch.float32:
+        raise _lib.SlnError(f"detections must be f32 [B,D,6], got {detections.dtype} {tuple(detections.shape)}")
+    if mrcnn_mask.dim() != 5 or mrcnn_mask.dtype != torch.float32:
+        raise _lib.SlnError(f"mrcnn_mask must be f32 [B,D,h,w,K], got {mrcnn_mask.dtype} {tuple(mrcnn_mask.shape)}")
+    B, D = int(detections.shape[0]), int(detections.shape[1])
+    if tuple(mrcnn_mask.shape[:2]) != (B, D):
+        raise _lib.SlnError(f"mrcnn_mask {tuple(mrcnn_mask.shape)} disagrees with detections {tuple(detections.shape)}")
+    if len(image_shapes) != B or len(windows) != B:
+        raise _lib.SlnError(f"{len(image_shapes)} image shapes and {len(windows)} windows for B = {B} images")
+    if B > UNMOLD_BATCH_MAX:
+        raise _lib.SlnError(f"B = {B} images in one call (at most {UNMOLD_BATCH_MAX})")
+    mh, mw, K = (int(v) for v in mrcnn_mask.shape[2:])
+    if not (1 <= mh <= 256 and 1 <= mw <= 256 and K >= 1):
+        raise _lib.SlnError(f"mask [h, w, K] = {(mh, mw, K)}: h, w in [1, 256] and K >= 1")
+    Hs = [int(s[0]) for s in image_shapes]
+    Ws = [int(s[1]) for s in image_shapes]
+    if any(not (1 <= v <= 65535) for v in Hs + Ws):
+        raise _lib.SlnError(f"image sides must be in [1, 65535], got {list(zip(Hs, Ws))}")
+    ss = [unmold_scale_shift(image_shapes[b], windows[b]) for b in range(B)]
+    cap = 2 * max(Ws, default=1) + 1 if cap is None else int(cap)
+    n = B * D
+    if cap < 1 or 7 * cap * n >= 1 << 31:
+        raise _lib.SlnError(f"cap = {cap} for {n} masks: need cap >= 1 and 7 * cap * B * D < 2^31")
+    dev = detections.device
+    det = detections.detach().contiguous()
+    mask = mrcnn_mask.detach()
+    meta = torch.empty(10 * n + B + 1, dtype=torch.int32, device=dev)
+    strings = torch.empty(max(7 * cap * n, 1), dtype=torch.uint8, device=dev)
+    views = unmold_meta_views(meta, B, D)
+    boxes, cls, scores, src, m, off, slen, num_kept, total = views
+    Ha, Wa = (C.c_int * max(B, 1))(*Hs), (C.c_int * max(B, 1))(*Ws)
+    sa = (C.c_double * max(4 * B, 1))(*[v for t in ss for v in t])
+    st = (C.c_longlong * 5)(*[int(v) for v in mask.stride()])
+    with torch.cuda.device(dev):
+        need = lib().sln_unmold_rle_batched_workspace_bytes(B, D, Ha, Wa, cap)
+        if workspace is None:
+            workspace = _workspace(need, dev)
+        elif workspace.numel() < need or not workspace.is_cuda:
+            raise _lib.SlnError(f"workspace: need {need} bytes on the device, got {workspace.numel()}")
+        check(lib().sln_unmold_rle_batched(ptr(det), B, D, ptr(mask), mh, mw, K, st, Ha, Wa, sa, cap, ptr(boxes), ptr(cls),
+                                           ptr(scores), ptr(src), ptr(num_kept), ptr(m), ptr(off), ptr(slen), ptr(total),
+                                           ptr(strings), strings.numel(), ptr(workspace), workspace.numel(), stream_ptr()),
+              "sln_unmold_rle_batched")
+    if B and D:
+        _lib.count_launches(5)      # box prep, box-local paste, runs, string scan, string write
+    return UnmoldRle(*views, strings, meta)
+
+
+def rle_strings_device(counts, m):
+    """The device string coder (sln_rle_strings): counts u32-as-int32 [n, cap] and m int32 [n] (the outputs of
+    rle.rle_counts_device) -> (strings u8, str_off int32 [n], str_len int32 [n], str_total int32 [1]).  List i's
+    rleToString string is strings[str_off[i] : str_off[i] + str_len[i]]; lists with m[i] <= 0 or > cap get none."""
+    _require_cuda(counts, "counts")
+    _require_cuda(m, "m")
+    if counts.dim() != 2 or counts.dtype not in (torch.int32, torch.uint32) or m.dtype != torch.int32 or \
+            tuple(m.shape) != (counts.shape[0],):
+        raise _lib.SlnError(f"counts must be 32-bit [n, cap] and m int32 [n], got {tuple(counts.shape)} / {tuple(m.shape)}")
+    n, cap = int(counts.shape[0]), int(counts.shape[1])
+    if cap < 1 or 7 * cap * n >= 1 << 31:
+        raise _lib.SlnError(f"counts [{n}, {cap}]: need cap >= 1 and 7 * cap * n < 2^31")
+    counts, m = counts.contiguous(), m.contiguous()
+    dev = counts.device
+    strings = torch.empty(max(7 * cap * n, 1), dtype=torch.uint8, device=dev)
+    off = torch.empty(n, dtype=torch.int32, device=dev)
+    slen = torch.empty(n, dtype=torch.int32, device=dev)
+    total = torch.empty(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().sln_rle_strings(ptr(counts), n, cap, ptr(m), ptr(off), ptr(slen), ptr(total), ptr(strings),
+                                    strings.numel(), stream_ptr()), "sln_rle_strings")
+    if n:
+        _lib.count_launches(3)
+    return strings, off, slen, total
 
 
 def bbox_overlaps_device(boxes1, boxes2, matrix=True, reduce=False):

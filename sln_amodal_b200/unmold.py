@@ -4,17 +4,21 @@
     unmold_mask(mask, bbox, image_shape)                               -> u8 [H, W]   (the reference's signature)
     unmold_masks(masks [N,h,w], boxes [N,4], image_shape)              -> u8 [N, H, W] on the device
     unmold_detections(detections, mrcnn_mask, image_shape, window)     -> boxes, class_ids, scores, masks [H, W, N]
+    unmold_detections_batched(detections [B,D,6], mrcnn_mask [B,D,h,w,K], image_shapes, windows)
+                                                                       -> per image: boxes, class_ids, scores, COCO RLEs
 
 The reference resizes with scipy.misc.imresize(interp='bilinear') = scipy's bytescale + Pillow's 8-bit resampler;
 sln_unmold_masks reproduces both bit for bit (csrc/unmold.cu).  The planes stay on the device so that
 rle.encode() -- the next step of the reference's evaluation (amodal_train.py:371-400) -- takes them without a copy.
+The batched form goes from B images' detections to COCO RLE strings on the device without any H x W plane
+(ops.unmold_rle_batched_device); its results are those of unmold_detections followed by rle.encode, image by image.
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, ops, rle
 from ._lib import check, lib, ptr, stream_ptr
 
 
@@ -94,3 +98,40 @@ def unmold_detections(detections, mrcnn_mask, image_shape, window, return_device
     if return_device_planes:
         return boxes, class_ids, scores, planes
     return boxes, class_ids, scores, np.ascontiguousarray(planes.permute(1, 2, 0).cpu().numpy())
+
+
+def unmold_detections_batched(detections, mrcnn_mask, image_shapes, windows, cap=None):
+    """unmold_detections + rle.encode for B images at once.  detections f32 [B,D,6] (BatchedHeadGraph's output, or a
+    stack of per-image [D,6]) and mrcnn_mask f32 [B,D,h,w,K] (any strides: a permuted view of [B,D,K,h,w] works) on
+    the device; image_shapes and windows: B host values each (images may differ in size).  Returns, per image,
+    (boxes int32 [n,4], class_ids int32 [n], scores f32 [n], rles) with rles a list of {"size": [H, W], "counts": bytes}:
+    what unmold_detections(..., return_device_planes=True) followed by rle.encode(planes) returns for that image (for an
+    image with no kept detection, rles is [] where the single-image path returns the reference's placeholder array).
+    The device work runs sync-free (ops.unmold_rle_batched_device); the host waits once, then copies the metadata and
+    the packed strings.  Masks with more than `cap` runs (see the ops function) are re-encoded through unmold_masks +
+    rle.encode."""
+    B = int(detections.shape[0]) if isinstance(detections, torch.Tensor) else len(detections)
+    out = ops.unmold_rle_batched_device(detections, mrcnn_mask, image_shapes, windows, cap=cap)
+    if B == 0:
+        return []
+    D = int(detections.shape[1])
+    meta = out.meta.cpu().numpy()                                       # the one wait for the device
+    boxes, cls, scores, src, m, off, slen, num_kept, total = ops.unmold_meta_views(meta, B, D)
+    strings = out.strings[: int(total[0])].cpu().numpy().tobytes() if int(total[0]) else b""
+    results = []
+    for b in range(B):
+        n = int(num_kept[b])
+        if n < 0:
+            raise IndexError(f"image {b}: a detection's class indexes outside the {int(mrcnn_mask.shape[4])} mask channels")
+        H, W = int(image_shapes[b][0]), int(image_shapes[b][1])
+        rles = [{"size": [H, W], "counts": strings[int(off[b, k]): int(off[b, k]) + int(slen[b, k])]} if m[b, k] > 0
+                else None for k in range(n)]
+        retry = [k for k in range(n) if m[b, k] <= 0]
+        if retry:                                                       # more runs than cap: the full-plane path
+            dev = mrcnn_mask.device
+            masks = mrcnn_mask[b][torch.as_tensor(src[b, retry].astype(np.int64), device=dev), :, :,
+                                  torch.as_tensor(cls[b, retry].astype(np.int64), device=dev)]
+            for k, r in zip(retry, rle.encode(unmold_masks(masks, boxes[b, retry], image_shapes[b]))):
+                rles[k] = r
+        results.append((boxes[b, :n].copy(), cls[b, :n].copy(), scores[b, :n].copy(), rles))
+    return results
