@@ -266,6 +266,29 @@ SLN_API int sln_box_refinement(const float *box, const float *gt_box, int M, con
 SLN_API int sln_mask_targets(const uint8_t *gt_masks, int L, int G, int H, int W, const int *assignment,
                      const float *boxes, int P, int mh, int mw, float *out, void *stream);
 
+/* detection_target_layer for B images, the two device halves around the host's sampling.
+ * sln_target_match_batched: proposals f32 [B,R,4], num_proposals device i32 [B] (NULL: all R rows) -> per row codes u8
+ * [B,R] (bit 0 = positive, iou_max >= 0.5; bit 1 = negative-eligible, iou_max < 0.5 and, in an image with a crowd GT row
+ * (class < 0), crowd_iou_max < 0.001; a NaN iou_max is neither, as in the reference; 0 past num_proposals[b]) and argmax
+ * i32 [B,R] = the first maximum's row in gt_boxes[b].  Candidates: the first num_gt_host[b] rows of gt_boxes f32 [B,G,4]
+ * / gt_class_ids i32 [B,G], only those with class > 0 in a crowd image.  num_gt_host is passed by value in the kernel's
+ * parameters (B <= 512).  Same IoU arithmetic as sln_bbox_overlaps.  One launch.
+ * sln_detection_targets_emit_batched: after sampling, sel i32 [B,T] (proposal rows, positives first), num_positive /
+ * num_rois i32 [B] and, per image, mask_planes[b] = device address of its u8 masks [L, mask_g[b], H, W] (device
+ * arrays).  Writes the whole padded output: rois f32 [B,T,4], class_ids i32 [B,T], deltas f32 [B,T,4] (divided by
+ * std_dev_host when not NULL), masks f32 [B,T,L,mh,mw]; positive rows as sln_box_refinement / sln_mask_targets compute
+ * them (the mask box in the GT box's frame when use_mini_mask), negative rows the proposal with class 0 and zeros, rows
+ * past num_rois[b] zeros.  One launch.                                                                          */
+SLN_API int sln_target_match_batched(const float *proposals, int B, int R, const int *num_proposals,
+                             const float *gt_boxes, const int *gt_class_ids, int G, const int *num_gt_host,
+                             uint8_t *codes, int *argmax, void *stream);
+SLN_API int sln_detection_targets_emit_batched(const float *proposals, int B, int R, const int *argmax,
+                                       const float *gt_boxes, const int *gt_class_ids, int G, const int *sel,
+                                       const int *num_positive, const int *num_rois,
+                                       const uint8_t *const *mask_planes, const int *mask_g, int T, int L, int H,
+                                       int W, int mh, int mw, const float *std_dev_host, int use_mini_mask,
+                                       float *rois, int *class_ids, float *deltas, float *masks, void *stream);
+
 /* Overlap reductions of build_rpn_targets (modal/Functions.py:773-792; SURVEY 8(f)-2) in float64, without the
  * [A,G] matrix: anchor_iou_max f64 [A] and anchor_argmax i32 [A] = max / first argmax over the GT boxes of every anchor,
  * gt_argmax i32 [G] = first argmax over the anchors of every GT box (numpy rules: NaN is the maximum).  Any output may

@@ -14,8 +14,9 @@ from .pyramid import pyramid_roi_align, pyramid_roi_align_batched, pyramid_roi_a
 from .semdist import decode_layers, load_layer2, sem_dist_targets  # noqa: F401
 from .detection import refine_detections, refine_detections_batched  # noqa: F401
 from .ops import nms_batched_device as nms_batched  # noqa: F401
-from .targets import (bbox_overlaps, box_refinement, build_rpn_targets, detection_target_layer, extract_bboxes,  # noqa: F401
-                      resize_image, resize_image_device, resize_layer, resize_layer_device, zoom_index_map)
+from .targets import (bbox_overlaps, box_refinement, build_rpn_targets, detection_target_layer,  # noqa: F401
+                      detection_target_layer_batched, extract_bboxes, resize_image, resize_image_device, resize_layer,
+                      resize_layer_device, zoom_index_map)
 from .rle import encode as rle_encode  # noqa: F401
 from .rpn import rpn_forward_levels, rpn_pack  # noqa: F401
 from .unmold import unmold_detections, unmold_detections_batched, unmold_mask, unmold_masks  # noqa: F401

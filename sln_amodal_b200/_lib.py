@@ -59,6 +59,9 @@ PROTOTYPES = {
     "sln_bbox_overlaps": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp]),
     "sln_box_refinement": (_i, [_vp, _vp, _i, C.POINTER(_f), _vp, _vp]),
     "sln_mask_targets": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "sln_target_match_batched": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, C.POINTER(_i), _vp, _vp, _vp]),
+    "sln_detection_targets_emit_batched": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i,
+                                                _i, _i, C.POINTER(_f), _i, _vp, _vp, _vp, _vp, _vp]),
     "sln_rpn_overlap_workspace_bytes": (_sz, [_i]),
     "sln_rpn_overlap_reductions": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "sln_plane_bboxes": (_i, [_vp, _i, _i, _i, _vp, _vp]),

@@ -271,6 +271,28 @@ extern "C" int sln_refine_nms_emit_batched(const float *dets, const int *class_i
 // (torch.max semantics: a NaN in the row is the maximum).
 namespace sln {
 
+// IoU of box a (area1 = its area) against box g, bbox_overlaps' operation sequence.  Shared by bbox_overlaps_kernel and
+// the batched match kernel, so that both round the same way.
+__device__ __forceinline__ float iou_f32(const float4 a, float area1, const float4 g)
+{
+    const float y1 = fmaxf(a.x, g.x), x1 = fmaxf(a.y, g.y), y2 = fminf(a.z, g.z), x2 = fminf(a.w, g.w);
+    // torch.max(x2 - x1, zeros): NaN-propagating in torch, fmaxf is not -- handled through `inter != inter` below
+    const float dx = __fsub_rn(x2, x1), dy = __fsub_rn(y2, y1);
+    float inter = __fmul_rn(dx > 0.f ? dx : (dx != dx ? dx : 0.f), dy > 0.f ? dy : (dy != dy ? dy : 0.f));
+    const float area2 = __fmul_rn(__fsub_rn(g.z, g.x), __fsub_rn(g.w, g.y));
+    const float uni = __fsub_rn(__fadd_rn(area1, area2), inter);
+    return __fdiv_rn(inter, uni);
+}
+
+__device__ __forceinline__ float box_area_f32(const float4 a) { return __fmul_rn(__fsub_rn(a.z, a.x), __fsub_rn(a.w, a.y)); }
+
+// torch.max(dim) over a row visited in index order: the first NaN is the maximum and stays, else the first strict maximum
+__device__ __forceinline__ void row_max_update(float v, int j, float &best, int &arg, bool &best_nan)
+{
+    const bool vnan = v != v;
+    if (!best_nan && (vnan || v > best)) { best = v; arg = j; best_nan = vnan; }
+}
+
 __global__ void __launch_bounds__(128)
 bbox_overlaps_kernel(const float *__restrict__ b1, int N, const float *__restrict__ b2, int G,
                      float *__restrict__ overlaps, float *__restrict__ iou_max, int *__restrict__ argmax)
@@ -278,19 +300,13 @@ bbox_overlaps_kernel(const float *__restrict__ b1, int N, const float *__restric
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
     const float4 a = *reinterpret_cast<const float4 *>(b1 + 4 * (size_t)i);          // (y1, x1, y2, x2)
-    const float area1 = __fmul_rn(__fsub_rn(a.z, a.x), __fsub_rn(a.w, a.y));
+    const float area1 = box_area_f32(a);
     float best = -INFINITY;
     int arg = 0;
     bool best_nan = false;
     for (int j = 0; j < G; ++j) {
         const float4 g = __ldg(reinterpret_cast<const float4 *>(b2) + j);
-        const float y1 = fmaxf(a.x, g.x), x1 = fmaxf(a.y, g.y), y2 = fminf(a.z, g.z), x2 = fminf(a.w, g.w);
-        // torch.max(x2 - x1, zeros): NaN-propagating in torch, fmaxf is not -- handled through `inter != inter` below
-        const float dx = __fsub_rn(x2, x1), dy = __fsub_rn(y2, y1);
-        float inter = __fmul_rn(dx > 0.f ? dx : (dx != dx ? dx : 0.f), dy > 0.f ? dy : (dy != dy ? dy : 0.f));
-        const float area2 = __fmul_rn(__fsub_rn(g.z, g.x), __fsub_rn(g.w, g.y));
-        const float uni = __fsub_rn(__fadd_rn(area1, area2), inter);
-        const float v = __fdiv_rn(inter, uni);
+        const float v = iou_f32(a, area1, g);
         if (overlaps) overlaps[(size_t)i * G + j] = v;
         const bool vnan = v != v;
         if (!best_nan && (vnan || v > best)) { best = v; arg = j; best_nan = vnan; }
@@ -299,7 +315,20 @@ bbox_overlaps_kernel(const float *__restrict__ b1, int N, const float *__restric
     if (argmax) argmax[i] = arg;
 }
 
-// utils.box_refinement (utils.py:96-117), optionally divided by BBOX_STD_DEV (Functions.py:309-313)
+// utils.box_refinement (utils.py:96-117) of box b onto gt box g, optionally divided by BBOX_STD_DEV (Functions.py:309-313)
+__device__ __forceinline__ float4 box_refinement_f32(const float4 b, const float4 g, int use_std, float s0, float s1,
+                                                     float s2, float s3)
+{
+    const float h = __fsub_rn(b.z, b.x), w = __fsub_rn(b.w, b.y);
+    const float cy = __fadd_rn(b.x, __fmul_rn(0.5f, h)), cx = __fadd_rn(b.y, __fmul_rn(0.5f, w));
+    const float gh = __fsub_rn(g.z, g.x), gw = __fsub_rn(g.w, g.y);
+    const float gcy = __fadd_rn(g.x, __fmul_rn(0.5f, gh)), gcx = __fadd_rn(g.y, __fmul_rn(0.5f, gw));
+    float dy = __fdiv_rn(__fsub_rn(gcy, cy), h), dx = __fdiv_rn(__fsub_rn(gcx, cx), w);
+    float dh = (float)log((double)__fdiv_rn(gh, h)), dw = (float)log((double)__fdiv_rn(gw, w));   // within 1 ulp of torch's CPU log
+    if (use_std) { dy = __fdiv_rn(dy, s0); dx = __fdiv_rn(dx, s1); dh = __fdiv_rn(dh, s2); dw = __fdiv_rn(dw, s3); }
+    return make_float4(dy, dx, dh, dw);
+}
+
 __global__ void __launch_bounds__(128)
 box_refinement_kernel(const float *__restrict__ box, const float *__restrict__ gt, int M, int use_std, float s0,
                       float s1, float s2, float s3, float *__restrict__ out)
@@ -308,14 +337,7 @@ box_refinement_kernel(const float *__restrict__ box, const float *__restrict__ g
     if (i >= M) return;
     const float4 b = *reinterpret_cast<const float4 *>(box + 4 * (size_t)i);
     const float4 g = *reinterpret_cast<const float4 *>(gt + 4 * (size_t)i);
-    const float h = __fsub_rn(b.z, b.x), w = __fsub_rn(b.w, b.y);
-    const float cy = __fadd_rn(b.x, __fmul_rn(0.5f, h)), cx = __fadd_rn(b.y, __fmul_rn(0.5f, w));
-    const float gh = __fsub_rn(g.z, g.x), gw = __fsub_rn(g.w, g.y);
-    const float gcy = __fadd_rn(g.x, __fmul_rn(0.5f, gh)), gcx = __fadd_rn(g.y, __fmul_rn(0.5f, gw));
-    float dy = __fdiv_rn(__fsub_rn(gcy, cy), h), dx = __fdiv_rn(__fsub_rn(gcx, cx), w);
-    float dh = (float)log((double)__fdiv_rn(gh, h)), dw = (float)log((double)__fdiv_rn(gw, w));   // within 1 ulp of torch's CPU log
-    if (use_std) { dy = __fdiv_rn(dy, s0); dx = __fdiv_rn(dx, s1); dh = __fdiv_rn(dh, s2); dw = __fdiv_rn(dw, s3); }
-    *reinterpret_cast<float4 *>(out + 4 * (size_t)i) = make_float4(dy, dx, dh, dw);
+    *reinterpret_cast<float4 *>(out + 4 * (size_t)i) = box_refinement_f32(b, g, use_std, s0, s1, s2, s3);
 }
 
 }  // namespace sln
@@ -358,6 +380,24 @@ extern "C" int sln_box_refinement(const float *box, const float *gt_box, int M, 
 // u8 -> f32 is exact) and rounds half-to-even.  out f32 [P, L, mh, mw].
 namespace sln {
 
+// Sample (y, x) of the mh x mw crop over box (y1,x1,y2,x2) of plane (l, g) of the u8 masks [L,G,H,W], before the
+// rounding; 0 outside the plane (extrapolation value, :339).  Shared by mask_targets_kernel and the batched emit kernel.
+__device__ __forceinline__ float mask_target_sample(const unsigned char *masks, int l, int G, int g, int H, int W,
+                                                    float y1, float x1, float y2, float x2, int mh, int mw, int y, int x)
+{
+    float v = 0.f;
+    const Tap ty = axis_tap(y1, y2, axis_scale(y1, y2, H, mh), H, mh, y);
+    const Tap tx = axis_tap(x1, x2, axis_scale(x1, x2, W, mw), W, mw, x);
+    if (ty.lo != INVALID_TAP && tx.lo != INVALID_TAP) {
+        const unsigned char *pl = masks + ((size_t)l * G + g) * H * W;
+        const int yh = ty.lo + (ty.lerp != 0.f), xh = tx.lo + (tx.lerp != 0.f);
+        const float tl = (float)pl[(size_t)ty.lo * W + tx.lo], tr = (float)pl[(size_t)ty.lo * W + xh];
+        const float bl = (float)pl[(size_t)yh * W + tx.lo], br = (float)pl[(size_t)yh * W + xh];
+        v = lerp2(tl, tr, bl, br, tx.lerp, ty.lerp);
+    }
+    return v;
+}
+
 __global__ void __launch_bounds__(256)
 mask_targets_kernel(const unsigned char *__restrict__ masks, int L, int G, int H, int W, const int *__restrict__ assignment,
                     const float *__restrict__ boxes, int P, int mh, int mw, float *__restrict__ out)
@@ -371,18 +411,9 @@ mask_targets_kernel(const unsigned char *__restrict__ masks, int L, int G, int H
     const int p = (int)(idx / ((long long)mw * mh * L));
     const int gidx = assignment[p];
     float v = 0.f;                                                        // extrapolation value 0 (:339)
-    if (gidx >= 0 && gidx < G) {
-        const float y1 = boxes[4 * p + 0], x1 = boxes[4 * p + 1], y2 = boxes[4 * p + 2], x2 = boxes[4 * p + 3];
-        const Tap ty = axis_tap(y1, y2, axis_scale(y1, y2, H, mh), H, mh, y);
-        const Tap tx = axis_tap(x1, x2, axis_scale(x1, x2, W, mw), W, mw, x);
-        if (ty.lo != INVALID_TAP && tx.lo != INVALID_TAP) {
-            const unsigned char *pl = masks + ((size_t)l * G + gidx) * H * W;
-            const int yh = ty.lo + (ty.lerp != 0.f), xh = tx.lo + (tx.lerp != 0.f);
-            const float tl = (float)pl[(size_t)ty.lo * W + tx.lo], tr = (float)pl[(size_t)ty.lo * W + xh];
-            const float bl = (float)pl[(size_t)yh * W + tx.lo], br = (float)pl[(size_t)yh * W + xh];
-            v = lerp2(tl, tr, bl, br, tx.lerp, ty.lerp);
-        }
-    }
+    if (gidx >= 0 && gidx < G)
+        v = mask_target_sample(masks, l, G, gidx, H, W, boxes[4 * p + 0], boxes[4 * p + 1], boxes[4 * p + 2],
+                               boxes[4 * p + 3], mh, mw, y, x);
     out[idx] = rintf(v);                                                  // torch.round (:346)
 }
 
@@ -400,6 +431,183 @@ extern "C" int sln_mask_targets(const uint8_t *gt_masks, int L, int G, int H, in
     sln::mask_targets_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         gt_masks, L, G, H, W, assignment, boxes, P, mh, mw, out);
     SLN_LAUNCH_OK("mask_targets_kernel");
+    return SLN_OK;
+}
+
+// ---------------------------------------------------------------------------
+// detection_target_layer for B images: a match launch, one host round trip (sampling), an emit launch
+// ---------------------------------------------------------------------------
+// Match: one thread per proposal row of image b = blockIdx.y.  The candidates are the image's first num_gt[b] GT rows,
+// or, when one of them has a class < 0 (a COCO crowd), its rows with class > 0 (Functions.py:253-267); the argmax is the
+// candidate's index in gt_boxes[b] (the single-image path compacts the candidates in order, so its first maximum is the
+// same box).  codes[b, i] bit 0 = positive (iou_max >= 0.5, :279), bit 1 = negative-eligible (iou_max < 0.5, and in a
+// crowd image crowd_iou_max < 0.001, :351-352).  A row whose iou_max is NaN is neither, as in the reference (NaN
+// compares false); rows at and beyond num_proposals[b] get 0.  The GT counts travel by value: no copy before the launch.
+namespace sln {
+
+template <int NB> struct TargetGtCounts { int v[NB]; };
+
+constexpr int TARGET_BATCH_MAX = 512;
+
+template <int NB>
+__global__ void __launch_bounds__(128)
+target_match_kernel(const float *__restrict__ proposals, int R, const int *__restrict__ num_proposals,
+                    const float *__restrict__ gt_boxes, const int *__restrict__ gt_class_ids, int G, const __grid_constant__ TargetGtCounts<NB> ng,
+                    unsigned char *__restrict__ codes, int *__restrict__ argmax)
+{
+    const int b = blockIdx.y;
+    const int n_gt = ng.v[b];
+    const int *cls = gt_class_ids + (size_t)b * G;
+    const float4 *gt = reinterpret_cast<const float4 *>(gt_boxes) + (size_t)b * G;
+    int crowd = 0;
+    for (int j = threadIdx.x; j < n_gt; j += blockDim.x) crowd |= __ldg(cls + j) < 0;
+    crowd = __syncthreads_or(crowd);
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R) return;
+    const size_t o = (size_t)b * R + i;
+    const int n_prop = num_proposals ? min(max(__ldg(num_proposals + b), 0), R) : R;
+    if (i >= n_prop) { codes[o] = 0; argmax[o] = 0; return; }
+    const float4 a = *reinterpret_cast<const float4 *>(proposals + 4 * o);
+    const float area1 = box_area_f32(a);
+    float best = -INFINITY, cbest = -INFINITY;
+    int arg = 0, carg = 0;
+    bool best_nan = false, cbest_nan = false;
+    for (int j = 0; j < n_gt; ++j) {
+        const int c = crowd ? __ldg(cls + j) : 1;
+        if (c == 0) continue;                                   // only reached in a crowd image
+        const float v = iou_f32(a, area1, __ldg(gt + j));
+        if (c > 0) row_max_update(v, j, best, arg, best_nan);
+        else row_max_update(v, j, cbest, carg, cbest_nan);
+    }
+    codes[o] = (unsigned char)((best >= 0.5f ? 1 : 0) | (best < 0.5f && (!crowd || cbest < 0.001f) ? 2 : 0));
+    argmax[o] = arg;
+}
+
+template <int NB>
+static int launch_target_match(const float *proposals, int B, int R, const int *num_proposals, const float *gt_boxes,
+                               const int *gt_class_ids, int G, const int *num_gt_host, uint8_t *codes, int *argmax,
+                               cudaStream_t st)
+{
+    TargetGtCounts<NB> ng;
+    for (int b = 0; b < NB; ++b) ng.v[b] = b < B ? num_gt_host[b] : 0;
+    target_match_kernel<NB><<<dim3(cdiv(R, 128), B), 128, 0, st>>>(proposals, R, num_proposals, gt_boxes, gt_class_ids, G,
+                                                                     ng, codes, argmax);
+    SLN_LAUNCH_OK("target_match_kernel");
+    return SLN_OK;
+}
+
+// Emit: one CTA per output row (b, t) of the padded [B,T] result, after the host has sampled the rows.  sel[b, t] is a
+// proposal row of image b for t < num_rois[b]; the first num_positive[b] rows are the positives: their GT box and class
+// come through the match kernel's argmax, the deltas through box_refinement_kernel's arithmetic, the L mask targets
+// through mask_targets_kernel's sampling of image b's u8 planes (mask_planes[b] = [L, mask_g[b], H, W]) over the
+// proposal, or over it in the GT box's frame under USE_MINI_MASK (:316-325).  Negative rows: the proposal, class 0, zero
+// deltas and masks (:370-384).  Rows at and beyond num_rois[b]: zeros.  Every output element is written.
+constexpr int TARGET_EMIT_THREADS = 256;
+
+__global__ void __launch_bounds__(TARGET_EMIT_THREADS)
+detection_targets_emit_kernel(const float *__restrict__ proposals, int R, const int *__restrict__ argmax,
+                              const float *__restrict__ gt_boxes, const int *__restrict__ gt_class_ids, int G,
+                              const int *__restrict__ sel, const int *__restrict__ num_positive,
+                              const int *__restrict__ num_rois, const uint8_t *const *__restrict__ mask_planes,
+                              const int *__restrict__ mask_g, int T, int L, int H, int W, int mh, int mw, int use_std,
+                              float s0, float s1, float s2, float s3, int mini_mask, float *__restrict__ rois,
+                              int *__restrict__ class_ids, float *__restrict__ deltas, float *__restrict__ masks)
+{
+    const int row = blockIdx.x;
+    const int b = row / T, t = row - b * T;
+    const bool live = t < __ldg(num_rois + b);
+    const bool pos = live && t < __ldg(num_positive + b);
+    const int n = L * mh * mw;
+    float *mo = masks + (size_t)row * n;
+    float4 roi = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (live) roi = *reinterpret_cast<const float4 *>(proposals + 4 * ((size_t)b * R + __ldg(sel + row)));
+    if (!pos) {
+        if (threadIdx.x == 0) {
+            *reinterpret_cast<float4 *>(rois + 4 * (size_t)row) = roi;
+            class_ids[row] = 0;
+            *reinterpret_cast<float4 *>(deltas + 4 * (size_t)row) = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+        for (int k = threadIdx.x; k < n; k += TARGET_EMIT_THREADS) mo[k] = 0.f;
+        return;
+    }
+    const int g = __ldg(argmax + (size_t)b * R + __ldg(sel + row));
+    const float4 gt = *reinterpret_cast<const float4 *>(gt_boxes + 4 * ((size_t)b * G + g));
+    if (threadIdx.x == 0) {
+        *reinterpret_cast<float4 *>(rois + 4 * (size_t)row) = roi;
+        class_ids[row] = __ldg(gt_class_ids + (size_t)b * G + g);
+        *reinterpret_cast<float4 *>(deltas + 4 * (size_t)row) = box_refinement_f32(roi, gt, use_std, s0, s1, s2, s3);
+    }
+    float4 box = roi;
+    if (mini_mask) {
+        const float gh = __fsub_rn(gt.z, gt.x), gw = __fsub_rn(gt.w, gt.y);
+        box = make_float4(__fdiv_rn(__fsub_rn(roi.x, gt.x), gh), __fdiv_rn(__fsub_rn(roi.y, gt.y), gw),
+                          __fdiv_rn(__fsub_rn(roi.z, gt.x), gh), __fdiv_rn(__fsub_rn(roi.w, gt.y), gw));
+    }
+    const uint8_t *planes = mask_planes[b];
+    const int gs = __ldg(mask_g + b);
+    for (int k = threadIdx.x; k < n; k += TARGET_EMIT_THREADS) {
+        const int x = k % mw, y = (k / mw) % mh, l = k / (mw * mh);
+        mo[k] = rintf(mask_target_sample(planes, l, gs, g, H, W, box.x, box.y, box.z, box.w, mh, mw, y, x));
+    }
+}
+
+}  // namespace sln
+
+extern "C" int sln_target_match_batched(const float *proposals, int B, int R, const int *num_proposals,
+                                        const float *gt_boxes, const int *gt_class_ids, int G, const int *num_gt_host,
+                                        uint8_t *codes, int *argmax, void *stream)
+{
+    SLN_REQUIRE(B >= 0 && R >= 0 && G >= 0, SLN_ERR_ARG, "target_match_batched: negative size");
+    SLN_REQUIRE(B <= sln::TARGET_BATCH_MAX, SLN_ERR_ARG, "target_match_batched: B=%d images in one call (at most %d)", B,
+                sln::TARGET_BATCH_MAX);
+    if (B == 0 || R == 0) return SLN_OK;
+    SLN_REQUIRE(proposals && codes && argmax && num_gt_host, SLN_ERR_ARG, "target_match_batched: null pointer");
+    for (int b = 0; b < B; ++b)
+        SLN_REQUIRE(num_gt_host[b] >= 0 && num_gt_host[b] <= G, SLN_ERR_ARG,
+                    "target_match_batched: num_gt[%d] = %d outside [0, G=%d]", b, num_gt_host[b], G);
+    SLN_REQUIRE(G == 0 || (gt_boxes && gt_class_ids), SLN_ERR_ARG, "target_match_batched: null pointer");
+    SLN_REQUIRE(((reinterpret_cast<uintptr_t>(proposals) | reinterpret_cast<uintptr_t>(gt_boxes)) & 15u) == 0,
+                SLN_ERR_LAYOUT, "target_match_batched: proposals / gt_boxes must be 16-byte aligned");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (B <= 16)
+        return sln::launch_target_match<16>(proposals, B, R, num_proposals, gt_boxes, gt_class_ids, G, num_gt_host, codes, argmax, st);
+    if (B <= 128)
+        return sln::launch_target_match<128>(proposals, B, R, num_proposals, gt_boxes, gt_class_ids, G, num_gt_host, codes, argmax, st);
+    return sln::launch_target_match<sln::TARGET_BATCH_MAX>(proposals, B, R, num_proposals, gt_boxes, gt_class_ids, G,
+                                                           num_gt_host, codes, argmax, st);
+}
+
+extern "C" int sln_detection_targets_emit_batched(const float *proposals, int B, int R, const int *argmax,
+                                                  const float *gt_boxes, const int *gt_class_ids, int G, const int *sel,
+                                                  const int *num_positive, const int *num_rois,
+                                                  const uint8_t *const *mask_planes, const int *mask_g, int T, int L,
+                                                  int H, int W, int mh, int mw, const float *std_dev_host,
+                                                  int use_mini_mask, float *rois, int *class_ids, float *deltas,
+                                                  float *masks, void *stream)
+{
+    SLN_REQUIRE(B >= 0 && R >= 0 && G >= 0 && T >= 0 && L >= 0 && H >= 0 && W >= 0 && mh >= 1 && mw >= 1, SLN_ERR_ARG,
+                "detection_targets_emit_batched: bad size");
+    SLN_REQUIRE(B <= sln::TARGET_BATCH_MAX, SLN_ERR_ARG, "detection_targets_emit_batched: B=%d images in one call (at most %d)",
+                B, sln::TARGET_BATCH_MAX);
+    if ((long long)B * T == 0) return SLN_OK;
+    SLN_REQUIRE(sel && num_positive && num_rois && rois && class_ids && deltas && masks, SLN_ERR_ARG,
+                "detection_targets_emit_batched: null pointer");
+    SLN_REQUIRE(R == 0 || (proposals && argmax), SLN_ERR_ARG, "detection_targets_emit_batched: null pointer");
+    SLN_REQUIRE(G == 0 || (gt_boxes && gt_class_ids), SLN_ERR_ARG, "detection_targets_emit_batched: null pointer");
+    SLN_REQUIRE(L == 0 || (mask_planes && mask_g), SLN_ERR_ARG, "detection_targets_emit_batched: null pointer");
+    SLN_REQUIRE(H <= 32767 && W <= 32767, SLN_ERR_ARG, "detection_targets_emit_batched: mask side above 32767");
+    SLN_REQUIRE((long long)L * mh * mw < (1ll << 31) && (long long)B * T < (1ll << 31), SLN_ERR_ARG,
+                "detection_targets_emit_batched: too many targets");
+    SLN_REQUIRE(((reinterpret_cast<uintptr_t>(proposals) | reinterpret_cast<uintptr_t>(gt_boxes) |
+                  reinterpret_cast<uintptr_t>(rois) | reinterpret_cast<uintptr_t>(deltas)) & 15u) == 0, SLN_ERR_LAYOUT,
+                "detection_targets_emit_batched: proposals / gt_boxes / rois / deltas must be 16-byte aligned");
+    const float *s = std_dev_host;
+    sln::detection_targets_emit_kernel<<<(unsigned)((long long)B * T), sln::TARGET_EMIT_THREADS, 0,
+                                         static_cast<cudaStream_t>(stream)>>>(
+        proposals, R, argmax, gt_boxes, gt_class_ids, G, sel, num_positive, num_rois, mask_planes, mask_g, T, L, H, W, mh,
+        mw, s != nullptr, s ? s[0] : 1.f, s ? s[1] : 1.f, s ? s[2] : 1.f, s ? s[3] : 1.f, use_mini_mask != 0, rois, class_ids,
+        deltas, masks);
+    SLN_LAUNCH_OK("detection_targets_emit_kernel");
     return SLN_OK;
 }
 

@@ -841,6 +841,147 @@ def mask_targets_device(gt_masks, assignment, boxes, mh, mw):
     return out
 
 
+TARGET_BATCH_MAX = 512          # images per batched detection-target call (their GT counts travel as kernel parameters)
+
+
+def target_num_gt(num_gt, B, G):
+    """num_gt of the batched detection targets as B host ints in [0, G] (None: G for every image)."""
+    if num_gt is None:
+        return [G] * B
+    if isinstance(num_gt, torch.Tensor):
+        if num_gt.is_cuda:
+            raise _lib.SlnError("num_gt must be host ints (a device tensor would need a sync to read)")
+        num_gt = num_gt.tolist()
+    num_gt = [int(v) for v in num_gt]
+    if len(num_gt) != B:
+        raise _lib.SlnError(f"num_gt has {len(num_gt)} entries for B = {B} images")
+    if any(not (0 <= v <= G) for v in num_gt):
+        raise _lib.SlnError(f"num_gt {num_gt} outside [0, G = {G}]")
+    return num_gt
+
+
+def target_mask_planes(gt_masks, B, G, num_gt, device):
+    """The GT masks of the batched detection targets: one u8 / bool tensor [B,L,G,H,W] or a list of B tensors
+    [L,G_b,H,W] with G_b == num_gt[b], on `device`.  Returns (planes: B contiguous u8 tensors [L,G_b,H,W], their G_b,
+    (L, H, W)).  Nothing is stacked or copied, except an entry that is not contiguous."""
+    if isinstance(gt_masks, torch.Tensor):
+        _require_cuda(gt_masks, "gt_masks")
+        if gt_masks.dim() != 5 or int(gt_masks.shape[0]) != B or int(gt_masks.shape[2]) != G:
+            raise _lib.SlnError(f"gt_masks must be [B={B},L,G={G},H,W] or a list of B tensors [L,G_b,H,W], "
+                                f"got {tuple(gt_masks.shape)}")
+        entries = [gt_masks[b] for b in range(B)]
+        gs = [int(gt_masks.shape[2])] * B
+    else:
+        entries = list(gt_masks)
+        if len(entries) != B:
+            raise _lib.SlnError(f"gt_masks has {len(entries)} entries for B = {B} images")
+        for b, m in enumerate(entries):
+            if not isinstance(m, torch.Tensor) or m.dim() != 4:
+                raise _lib.SlnError(f"gt_masks[{b}] must be a tensor [L,G_b,H,W]")
+        gs = [int(m.shape[1]) for m in entries]
+        if gs != list(num_gt):
+            raise _lib.SlnError(f"gt_masks entries have G_b = {gs}, num_gt is {list(num_gt)}")
+    planes = []
+    for b, m in enumerate(entries):
+        _require_cuda(m, f"gt_masks[{b}]")
+        if m.dtype not in (torch.uint8, torch.bool):
+            raise _lib.SlnError(f"gt_masks must be uint8 / bool, got {m.dtype}")
+        if m.device != device:
+            raise _lib.SlnError(f"gt_masks[{b}] is on {m.device}, the proposals on {device}")
+        planes.append((m.view(torch.uint8) if m.dtype == torch.bool else m).contiguous())
+    lhw = {(int(m.shape[0]), int(m.shape[2]), int(m.shape[3])) for m in planes}
+    if len(lhw) > 1:
+        raise _lib.SlnError(f"every image needs the same L, H, W of its masks, got {sorted(lhw)}")
+    L, H, W = lhw.pop() if lhw else (0, 1, 1)
+    if not (1 <= H <= 32767 and 1 <= W <= 32767):
+        raise _lib.SlnError(f"mask side outside [1, 32767]: {H} x {W}")
+    return planes, gs, (L, H, W)
+
+
+def target_match_batched_device(proposals, gt_class_ids, gt_boxes, num_gt=None, num_proposals=None):
+    """Match half of the batched detection targets (sln_target_match_batched, one launch): proposals f32 [B,R,4],
+    gt_class_ids int [B,G], gt_boxes f32 [B,G,4] on the device, num_gt B host ints (None: all G rows), num_proposals
+    int32 device [B] (None: all R rows).  Returns (codes u8 [B,R]: bit 0 positive, bit 1 negative-eligible; argmax
+    int32 [B,R]: the matched row of gt_boxes[b])."""
+    B, R, G, num_gt, cls, num_proposals = target_inputs(proposals, gt_class_ids, gt_boxes, num_gt, num_proposals)
+    dev = proposals.device
+    codes = torch.empty((B, R), dtype=torch.uint8, device=dev)
+    argmax = torch.empty((B, R), dtype=torch.int32, device=dev)
+    if B and R:
+        ng = (C.c_int * B)(*num_gt)
+        with torch.cuda.device(dev):
+            check(lib().sln_target_match_batched(ptr(proposals.contiguous()), B, R, ptr(num_proposals), ptr(gt_boxes.contiguous()),
+                                                 ptr(cls), G, ng, ptr(codes), ptr(argmax), stream_ptr()),
+                  "sln_target_match_batched")
+        _lib.count_launches(1)
+    return codes, argmax
+
+
+def target_inputs(proposals, gt_class_ids, gt_boxes, num_gt, num_proposals):
+    """Checks the batched detection targets' inputs (SlnError on any mismatch, before anything is launched).  Returns
+    (B, R, G, num_gt as B host ints, gt_class_ids as int32, num_proposals contiguous or None)."""
+    for t, name in ((proposals, "proposals"), (gt_class_ids, "gt_class_ids"), (gt_boxes, "gt_boxes")):
+        _require_cuda(t, name)
+    if proposals.dim() != 3 or proposals.shape[2] != 4 or proposals.dtype != torch.float32:
+        raise _lib.SlnError(f"proposals must be f32 [B,R,4], got {proposals.dtype} {tuple(proposals.shape)}")
+    B, R = int(proposals.shape[0]), int(proposals.shape[1])
+    if B > TARGET_BATCH_MAX:
+        raise _lib.SlnError(f"B = {B} images in one call (at most {TARGET_BATCH_MAX})")
+    if gt_boxes.dim() != 3 or int(gt_boxes.shape[0]) != B or gt_boxes.shape[2] != 4 or gt_boxes.dtype != torch.float32:
+        raise _lib.SlnError(f"gt_boxes must be f32 [B={B},G,4], got {gt_boxes.dtype} {tuple(gt_boxes.shape)}")
+    G = int(gt_boxes.shape[1])
+    if tuple(gt_class_ids.shape) != (B, G) or gt_class_ids.dtype.is_floating_point or gt_class_ids.dtype == torch.bool:
+        raise _lib.SlnError(f"gt_class_ids must be integer [B,G] = [{B},{G}], got {gt_class_ids.dtype} {tuple(gt_class_ids.shape)}")
+    for t, name in ((gt_class_ids, "gt_class_ids"), (gt_boxes, "gt_boxes")):
+        if t.device != proposals.device:
+            raise _lib.SlnError(f"{name} is on {t.device}, the proposals on {proposals.device}")
+    num_gt = target_num_gt(num_gt, B, G)
+    if num_proposals is not None:
+        _require_cuda(num_proposals, "num_proposals")
+        if tuple(num_proposals.shape) != (B,) or num_proposals.dtype != torch.int32 or num_proposals.device != proposals.device:
+            raise _lib.SlnError(f"num_proposals must be int32 [B={B}] beside the proposals, got {num_proposals.dtype} "
+                                f"{tuple(num_proposals.shape)} on {num_proposals.device}")
+        num_proposals = num_proposals.contiguous()
+    return B, R, G, num_gt, _i32c(gt_class_ids), num_proposals
+
+
+# Staging buffer of the batched detection targets (int32 slots): what the host's sampling sends to the emit kernel in
+# one copy.  planes: B device addresses of the images' u8 masks (two slots each, int64); then mask_g, num_positive,
+# num_rois [B] and sel [B,T].
+def target_stage_layout(B, T):
+    return {"planes": 0, "mask_g": 2 * B, "num_positive": 3 * B, "num_rois": 4 * B, "sel": 5 * B, "total": 5 * B + B * T}
+
+
+def detection_targets_emit_batched_device(proposals, argmax, gt_boxes, gt_class_ids, stage, T, LHW, mask_shape,
+                                          std_dev=None, use_mini_mask=False):
+    """Emit half of the batched detection targets (sln_detection_targets_emit_batched, one launch).  proposals f32
+    [B,R,4], argmax int32 [B,R] (target_match_batched_device's), gt_boxes f32 [B,G,4], gt_class_ids int32 [B,G]; stage:
+    the int32 device buffer of target_stage_layout(B, T), filled by the host's sampling; LHW = (L, H, W) of the masks it
+    points at.  Returns (rois f32 [B,T,4], class_ids int32 [B,T], deltas f32 [B,T,4], masks f32 [B,T,L,mh,mw]), every
+    element written."""
+    B, R, G = int(proposals.shape[0]), int(proposals.shape[1]), int(gt_boxes.shape[1])
+    L, H, W = (int(v) for v in LHW)
+    mh, mw = int(mask_shape[0]), int(mask_shape[1])
+    lay = target_stage_layout(B, T)
+    if stage.dtype != torch.int32 or stage.numel() != lay["total"]:
+        raise _lib.SlnError(f"stage must be int32 [{lay['total']}], got {stage.dtype} [{stage.numel()}]")
+    dev = proposals.device
+    rois = torch.empty((B, T, 4), dtype=torch.float32, device=dev)
+    class_ids = torch.empty((B, T), dtype=torch.int32, device=dev)
+    deltas = torch.empty((B, T, 4), dtype=torch.float32, device=dev)
+    masks = torch.empty((B, T, L, mh, mw), dtype=torch.float32, device=dev)
+    if B and T:
+        at = lambda k: C.c_void_p(stage.data_ptr() + 4 * lay[k])
+        sd = (C.c_float * 4)(*[float(v) for v in std_dev]) if std_dev is not None else None
+        with torch.cuda.device(dev):
+            check(lib().sln_detection_targets_emit_batched(
+                ptr(proposals.contiguous()), B, R, ptr(argmax), ptr(gt_boxes.contiguous()), ptr(gt_class_ids), G, at("sel"),
+                at("num_positive"), at("num_rois"), at("planes"), at("mask_g"), T, L, H, W, mh, mw, sd, int(bool(use_mini_mask)),
+                ptr(rois), ptr(class_ids), ptr(deltas), ptr(masks), stream_ptr()), "sln_detection_targets_emit_batched")
+        _lib.count_launches(1)
+    return rois, class_ids, deltas, masks
+
+
 def rpn_overlap_reductions_device(anchors, gt_boxes, want_argmax=True):
     """float64 IoU reductions of build_rpn_targets (sln_rpn_overlap_reductions).  anchors f64 [A,4], gt_boxes f64 [G,4]
     on the device -> (anchor_iou_max f64 [A], anchor_argmax i32 [A] | None, gt_argmax i32 [G] | None)."""

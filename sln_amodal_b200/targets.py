@@ -25,6 +25,34 @@ def box_refinement(box, gt_box):
     return ops.box_refinement_device(box, gt_box)
 
 
+def _sample_rois(positive_h, negative_h, config):
+    """The reference's subsampling (:281-291, :353-366) of one image on the host: bool [n] positive / negative rows ->
+    (positive rows, negative rows) as int64 index arrays, drawn with `torch.randperm` from the CPU generator under the
+    reference's conditions and in its order (the negative draw only after at least one positive).  Both
+    detection_target_layer and detection_target_layer_batched sample through here."""
+    pos_sel = neg_sel = np.zeros(0, np.int64)
+    if positive_h.any():
+        positive_indices = np.nonzero(positive_h)[0]
+        want = int(config.TRAIN_ROIS_PER_IMAGE * config.ROI_POSITIVE_RATIO)
+        rand_idx = torch.randperm(positive_indices.shape[0])[:want].numpy()   # CPU generator, like the reference
+        pos_sel = positive_indices[rand_idx]
+    if pos_sel.shape[0] > 0 and negative_h.any():
+        negative_indices = np.nonzero(negative_h)[0]
+        r = 1.0 / config.ROI_POSITIVE_RATIO
+        negative_count = int(r * pos_sel.shape[0] - pos_sel.shape[0])
+        rand_idx = torch.randperm(negative_indices.shape[0])[:negative_count].numpy()
+        neg_sel = negative_indices[rand_idx]
+    return pos_sel, neg_sel
+
+
+def rois_per_image(config):
+    """Most rows detection_target_layer can return for one image: max over p = 1..want of p + int(r*p - p), with the
+    reference's own float expressions (want positives at most, r = 1 / ROI_POSITIVE_RATIO)."""
+    want = int(config.TRAIN_ROIS_PER_IMAGE * config.ROI_POSITIVE_RATIO)
+    r = 1.0 / config.ROI_POSITIVE_RATIO
+    return max((p + int(r * p - p) for p in range(1, want + 1)), default=0)
+
+
 def detection_target_layer(proposals, gt_class_ids, gt_boxes, gt_masks, config):
     """proposals [1,N,4] normalised, gt_class_ids [1,G], gt_boxes [1,G,4] normalised, gt_masks [1,L,G,H,W]
     -> (rois [R,4], roi_gt_class_ids [R], deltas [R,4], masks [R,L,mh,mw]); empty tensors when nothing is sampled
@@ -72,21 +100,8 @@ def detection_target_layer(proposals, gt_class_ids, gt_boxes, gt_masks, config):
 
     L = gt_masks.shape[0]
     mh, mw = int(config.MASK_SHAPE[0]), int(config.MASK_SHAPE[1])
-    positive_count = negative_count = 0
-    pos_sel = neg_sel = None
-    if positive_h.any():                                                      # :281-291
-        positive_indices = np.nonzero(positive_h)[0]
-        want = int(config.TRAIN_ROIS_PER_IMAGE * config.ROI_POSITIVE_RATIO)
-        rand_idx = torch.randperm(positive_indices.shape[0])[:want].numpy()   # CPU generator, like the reference
-        pos_sel = positive_indices[rand_idx]
-        positive_count = pos_sel.shape[0]
-    if positive_count > 0 and negative_h.any():                               # :353-366
-        negative_indices = np.nonzero(negative_h)[0]
-        r = 1.0 / config.ROI_POSITIVE_RATIO
-        negative_count = int(r * positive_count - positive_count)
-        rand_idx = torch.randperm(negative_indices.shape[0])[:negative_count].numpy()
-        neg_sel = negative_indices[rand_idx]
-        negative_count = neg_sel.shape[0]
+    pos_sel, neg_sel = _sample_rois(positive_h, negative_h, config)
+    positive_count, negative_count = pos_sel.shape[0], neg_sel.shape[0]
     if positive_count > 0:
         sel = torch.from_numpy(np.concatenate([pos_sel, neg_sel]) if negative_count > 0 else pos_sel).to(dev)
         positive_indices = sel[:positive_count]
@@ -127,6 +142,54 @@ def detection_target_layer(proposals, gt_class_ids, gt_boxes, gt_masks, config):
         deltas = torch.empty(0, device=dev)
         masks = torch.empty(0, device=dev)
     return rois, roi_gt_class_ids, deltas, masks
+
+
+def detection_target_layer_batched(proposals, gt_class_ids, gt_boxes, gt_masks, config, num_proposals=None, num_gt=None):
+    """detection_target_layer for B images: one match launch, one host round trip, one emit launch.
+
+    proposals f32 [B,R,4] normalised (e.g. proposal_layer_batched's zero-padded rois), gt_class_ids int [B,G], gt_boxes
+    f32 [B,G,4] normalised, gt_masks u8 / bool on the device: one tensor [B,L,G,H,W] or a list of B tensors [L,G_b,H,W]
+    with G_b = num_gt[b] (never stacked or copied); num_proposals int32 device [B] (None: all R rows are proposals),
+    num_gt B host ints (None: all G rows are GT boxes).  Every image has the same L, H, W.
+    Returns (rois f32 [B,T,4], class_ids int32 [B,T], deltas f32 [B,T,4], masks f32 [B,T,L,mh,mw], num_positive int32
+    [B], num_rois int32 [B]) on the device, T = rois_per_image(config): image b's rows [0, num_positive[b]) are its
+    positives, then its negatives up to num_rois[b], then zeros.  Rows below num_rois[b] equal what
+    detection_target_layer returns for proposals[b, :num_proposals[b]] and gt_*[b, :num_gt[b]] alone (num_rois[b] = 0
+    where it returns empty tensors), and a seeded call draws the same `torch.randperm`s from the CPU generator in the same
+    order as the B single-image calls in image order.
+    One difference: a proposal whose IoU maximum is NaN (a zero-area proposal against a zero-area GT box) is neither
+    positive nor negative here, as in the reference (Functions.py:351, NaN < 0.5 is false); detection_target_layer counts
+    it as a negative.
+    The sampling runs on the host between the two launches (one wait, one device-to-host copy of a byte per proposal, one
+    host-to-device copy of the sampled rows), so the call cannot be captured in a CUDA graph."""
+    B, R, G, num_gt, gt_class_ids, num_proposals = ops.target_inputs(proposals, gt_class_ids, gt_boxes, num_gt, num_proposals)
+    dev = proposals.device
+    planes, mask_g, LHW = ops.target_mask_planes(gt_masks, B, G, num_gt, dev)
+    proposals, gt_boxes = proposals.contiguous(), gt_boxes.contiguous()
+    T = rois_per_image(config)
+    codes, argmax = ops.target_match_batched_device(proposals, gt_class_ids, gt_boxes, num_gt, num_proposals)
+    codes_h = codes.cpu().numpy()                                             # the one wait
+    lay = ops.target_stage_layout(B, T)
+    stage_h = torch.empty(lay["total"], dtype=torch.int32, pin_memory=True)
+    h = stage_h.numpy()
+    h[lay["planes"]:lay["mask_g"]].view(np.int64)[:] = [m.data_ptr() for m in planes]
+    h[lay["mask_g"]:lay["num_positive"]] = mask_g
+    sel = h[lay["sel"]:].reshape(B, T)
+    sel[:] = -1
+    for b in range(B):
+        pos_sel, neg_sel = _sample_rois((codes_h[b] & 1) != 0, (codes_h[b] & 2) != 0, config)
+        n_pos, n_rois = pos_sel.shape[0], pos_sel.shape[0] + neg_sel.shape[0]
+        sel[b, :n_pos] = pos_sel
+        sel[b, n_pos:n_rois] = neg_sel
+        h[lay["num_positive"] + b] = n_pos
+        h[lay["num_rois"] + b] = n_rois
+    stage = torch.empty(lay["total"], dtype=torch.int32, device=dev)
+    stage.copy_(stage_h, non_blocking=True)
+    rois, class_ids, deltas, masks = ops.detection_targets_emit_batched_device(
+        proposals, argmax, gt_boxes, gt_class_ids, stage, T, LHW, config.MASK_SHAPE, np.reshape(config.BBOX_STD_DEV, [4]),
+        config.USE_MINI_MASK)
+    return (rois, class_ids, deltas, masks, stage[lay["num_positive"]:lay["num_rois"]],
+            stage[lay["num_rois"]:lay["sel"]])
 
 
 _ANCHOR_CACHE = {}

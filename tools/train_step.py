@@ -16,6 +16,7 @@ mode='training'), losses (model.py:423-436), backward }, gradient clipping, SGD 
     accumulation under DDP.no_sync() until the rank's last image), weak scaling gives every rank 16.
 
     python tools/train_step.py                 (one GPU)
+    python tools/train_step.py --images-per-forward 16   (16 images per forward: batched proposals, targets, crops)
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/train_step.py --gpus N
 """
 from __future__ import annotations
@@ -161,7 +162,9 @@ class SLNTrainNet(nn.Module):
         self.register_buffer("anchors", anchors, persistent=False)
         self.cfg = Cfg()
 
-    def forward(self, image, rpn_match, rpn_bbox_t, gt_ids, gt_boxes, gt_masks, injected):
+    def forward(self, image, rpn_match=None, rpn_bbox_t=None, gt_ids=None, gt_boxes=None, gt_masks=None, injected=None):
+        if isinstance(image, dict):                                   # B images at once (batch_inputs)
+            return self.forward_batch(**image)
         from sln_amodal_b200 import detection_target_layer, proposal_layer, pyramid_roi_align, rpn as srpn
         cfg = self.cfg
         feats = self.fpn(image)
@@ -196,6 +199,66 @@ class SLNTrainNet(nn.Module):
                 loss = loss + F.binary_cross_entropy_with_logits(mlog[torch.arange(n_pos, device=mlog.device), cid], tm)
         return loss, n_pos
 
+    def forward_batch(self, images, rpn_match, rpn_bbox_t, gt_ids, gt_boxes, gt_masks, num_gt, injected):
+        """B images per forward: images [B,3,H,W] through the FPN as one batch (BatchNorms in eval mode, so every image
+        sees what it sees alone), rpn_pack, proposal_layer_batched, the injected proposals in front of each image's
+        proposals, detection_target_layer_batched, pyramid_roi_align_batched on the sampled rows.  gt_ids [B,G] /
+        gt_boxes [B,G,4] are padded beyond num_gt (B host ints), gt_masks a list of B [L,G_b,H,W]; rpn_match, rpn_bbox_t
+        and injected are lists of B.  Returns the sum over the images of forward()'s per-image loss, and the positives."""
+        from sln_amodal_b200 import detection_target_layer_batched, proposal_layer_batched, pyramid_roi_align_batched
+        from sln_amodal_b200 import rpn as srpn
+        cfg = self.cfg
+        B, dev = images.shape[0], images.device
+        feats = self.fpn(images)
+        cls_maps, box_maps = zip(*[self.rpn(p) for p in feats])
+        logits, probs, deltas = srpn.rpn_pack(list(cls_maps), list(box_maps))        # [B,A,2], [B,A,2], [B,A,4]
+        K = cfg.POST_NMS_ROIS_TRAINING
+        with torch.no_grad():
+            rois, num = proposal_layer_batched([probs, deltas], K, cfg.RPN_NMS_THRESHOLD, self.anchors, cfg)
+            n_inj = [int(j.shape[0]) for j in injected]
+            rois = torch.stack([torch.cat([injected[b], rois[b, : max(K - n_inj[b], 0)]])[:K] for b in range(B)])
+            num = torch.clamp(num + torch.tensor(n_inj, dtype=torch.int32, device=dev), max=K).to(torch.int32)
+            t_rois, t_ids, t_deltas, t_masks, _, t_num = detection_target_layer_batched(rois, gt_ids, gt_boxes, gt_masks, cfg,
+                                                                                     num_proposals=num, num_gt=num_gt)
+        loss = logits.new_zeros(())
+        for b in range(B):                                            # RPN losses (model.py:423-426), per image
+            m = rpn_match[b].view(-1)
+            sel = torch.nonzero(m != 0).view(-1)
+            loss = loss + F.cross_entropy(logits[b, sel], (m[sel] == 1).long())
+            pos = torch.nonzero(m == 1).view(-1)
+            if pos.numel():
+                loss = loss + F.smooth_l1_loss(deltas[b, pos], rpn_bbox_t[b][: pos.numel()])
+        T = t_rois.shape[1]
+        k = t_num.cpu().tolist()
+        rows = torch.from_numpy(np.concatenate([b * T + np.arange(k[b]) for b in range(B)]).astype(np.int64)).to(dev)
+        if rows.numel() == 0:
+            return loss, 0
+        img = torch.div(rows, T, rounding_mode="floor")
+
+        def per_image_mean(v, idx, n):                                # sum over the images of each image's mean
+            return (torch.zeros(B, device=dev).index_add_(0, idx, v) / n).sum()
+
+        ids = t_ids.view(-1)[rows].long()
+        boxes = t_rois.view(-1, 4)[rows]
+        maps = feats[:4]
+        pooled = pyramid_roi_align_batched(boxes, img.to(torch.int32), maps, cfg.POOL_SIZE, cfg.IMAGE_SHAPE)
+        cls_logits, bbox = self.classifier(pooled)
+        loss = loss + per_image_mean(F.cross_entropy(cls_logits, ids, reduction="none"), img,
+                                     torch.tensor(k, dtype=torch.float32, device=dev).clamp(min=1))
+        posr = torch.nonzero(ids > 0).view(-1)
+        n_pos = int(posr.numel())
+        if n_pos:
+            cid, pimg = ids[posr], img[posr]
+            pcnt = torch.zeros(B, device=dev).index_add_(0, pimg, torch.ones(n_pos, device=dev)).clamp(min=1)
+            dl = F.smooth_l1_loss(bbox[posr, cid], t_deltas.view(-1, 4)[rows][posr], reduction="none")
+            loss = loss + per_image_mean(dl.sum(1), pimg, 4 * pcnt)
+            pooled_m = pyramid_roi_align_batched(boxes[posr], pimg.to(torch.int32), maps, cfg.MASK_POOL_SIZE, cfg.IMAGE_SHAPE)
+            mlog = self.mask(pooled_m)
+            tm = t_masks.view(B * T, *t_masks.shape[2:])[rows][posr][:, 0]
+            bce = F.binary_cross_entropy_with_logits(mlog[torch.arange(n_pos, device=dev), cid], tm, reduction="none")
+            loss = loss + per_image_mean(bce.flatten(1).sum(1), pimg, pcnt * tm[0].numel())
+        return loss, n_pos
+
 
 # ----------------------------------------------------------------------------- synthetic D2SA-shaped data
 def make_image(seed, dev, anchors_np):
@@ -226,15 +289,32 @@ def make_image(seed, dev, anchors_np):
             "gt_ids": t(ids).unsqueeze(0), "gt_boxes": t(nb).unsqueeze(0), "gt_masks": t(masks).unsqueeze(0), "injected": t(jit)}
 
 
+def batch_inputs(items):
+    """SLNTrainNet.forward_batch's inputs for a list of make_image examples: the images as one [B,3,H,W] batch, the GT
+    ids / boxes padded to the largest instance count, the masks as a list (never stacked)."""
+    B, dev = len(items), items[0]["image"].device
+    num_gt = [int(d["gt_ids"].shape[1]) for d in items]
+    gt_ids = torch.zeros((B, max(num_gt)), dtype=torch.int32, device=dev)
+    gt_boxes = torch.zeros((B, max(num_gt), 4), dtype=torch.float32, device=dev)
+    for b, d in enumerate(items):
+        gt_ids[b, :num_gt[b]] = d["gt_ids"][0]
+        gt_boxes[b, :num_gt[b]] = d["gt_boxes"][0]
+    return {"images": torch.cat([d["image"] for d in items]).contiguous(memory_format=torch.channels_last),
+            "rpn_match": [d["rpn_match"] for d in items], "rpn_bbox_t": [d["rpn_bbox"] for d in items],
+            "gt_ids": gt_ids, "gt_boxes": gt_boxes, "gt_masks": [d["gt_masks"][0] for d in items], "num_gt": num_gt,
+            "injected": [d["injected"] for d in items]}
+
+
 class RCfg:
     RPN_TRAIN_ANCHORS_PER_IMAGE = 256
     RPN_BBOX_STD_DEV = np.array([0.1, 0.1, 0.2, 0.2])
 
 
 # ----------------------------------------------------------------------------- the measurement
-def run(dev, rank, world, steps=2, warmup=1, images_per_step=16, weak=False, log=None):
+def run(dev, rank, world, steps=2, warmup=1, images_per_step=16, weak=False, log=None, images_per_forward=1):
     """Times `steps` optimizer steps (CUDA events, barrier on both sides, max over ranks).  strong scaling: the 16 images
-    of a step are split over the ranks; weak: 16 per rank.  Returns a dict for bench.py."""
+    of a step are split over the ranks; weak: 16 per rank.  images_per_forward > 1 sends that many images through one
+    forward (SLNTrainNet.forward_batch) instead of one at a time.  Returns a dict for bench.py."""
     import torch.distributed as dist
     from sln_amodal_b200 import dist as sdist, synth
     from contextlib import nullcontext
@@ -257,7 +337,27 @@ def run(dev, rank, world, steps=2, warmup=1, images_per_step=16, weak=False, log
             dist.barrier()
         torch.cuda.synchronize()
 
+    B = max(1, min(int(images_per_forward), per_rank))
+    groups = [batch_inputs([data[(g + j) % len(data)] for j in range(min(B, per_rank - g))])
+              for g in range(0, per_rank, B)] if B > 1 else []
+
+    def step_batched(sync=True):
+        opt.zero_grad(set_to_none=True)
+        pos = 0
+        for i, grp in enumerate(groups):
+            last = i == len(groups) - 1
+            ctx = nullcontext() if (world == 1 or (last and sync)) else ddp.no_sync()
+            with ctx:
+                loss, n_pos = ddp(grp)
+                (loss / per_rank).backward()
+            pos += n_pos
+        torch.nn.utils.clip_grad_norm_(net.parameters(), 5.0)
+        opt.step()
+        return float(loss.detach()) / len(groups[-1]["num_gt"]), pos      # per image, like the per-image step's
+
     def step(sync=True):
+        if groups:
+            return step_batched(sync)
         opt.zero_grad(set_to_none=True)
         pos = 0
         for i in range(per_rank):
@@ -292,6 +392,8 @@ def run(dev, rank, world, steps=2, warmup=1, images_per_step=16, weak=False, log
            "n_gpus": world, "scaling": "weak" if weak else "strong", "images_per_step_global": per_rank * world,
            "ms_per_step": round(ms, 2), "images_per_s": round(per_rank * world / (ms * 1e-3), 2),
            "parameters": n_params, "positives_last_step": pos, "loss_last_step": round(loss, 4), "steps": steps}
+    if groups:
+        res["images_per_forward"] = B
     if world > 1:
         ms_ns, _ = timed(False)                                       # the same step without the gradient all-reduce
         res["ms_per_step_without_allreduce"] = round(ms_ns, 2)
@@ -317,6 +419,8 @@ def main():
     ap.add_argument("--steps", type=int, default=2)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--weak", action="store_true")
+    ap.add_argument("--images-per-forward", type=int, default=1,
+                    help="images per forward pass (B > 1: FPN on a [B,3,H,W] batch, batched proposals and targets)")
     args = ap.parse_args()
     from sln_amodal_b200 import dist as sdist
     real_stdout = os.dup(1)
@@ -324,7 +428,8 @@ def main():
     rank, world = sdist.init()
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
-    res = run(torch.device("cuda", local), rank, world, steps=args.steps, warmup=args.warmup, weak=args.weak)
+    res = run(torch.device("cuda", local), rank, world, steps=args.steps, warmup=args.warmup, weak=args.weak,
+              images_per_forward=args.images_per_forward)
     if rank == 0:
         os.write(real_stdout, (json.dumps(res) + "\n").encode())
     if world > 1:
